@@ -2,7 +2,7 @@
 """bench.py - nuclei/s of the radius-graph + neighbour-type composition + degree-statistics build on
 a 1M-nucleus synthetic WSI (BASELINE.json configs[1], "C2"), per GPU, weak-scaled by slide over N GPUs.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--dump-outputs DIR]
 
 One "step" = one pass of the hot path over one slide:
   pg_grid_build (histogram, look-back scan, counting-sort scatter) -> pg_radius_graph (one neighbourhood walk with
@@ -21,6 +21,8 @@ One "step" = one pass of the hot path over one slide:
              strong scaling, checksums against the single-GPU build) and `c4_cohort` (64 x 500 k nuclei slides from
              page-locked host tables, slide-parallel), plus the host-link ceiling measured with all ranks copying at once.
 `cpu_baseline` / `--impl reference`: the notebook's scipy path (oracle/graph.py) on the host cores, full 1 M slide.
+`--dump-outputs DIR`: rank 0 writes what the last timed step computed as DIR/<name>.npy (see last_step_outputs), so
+that two builds run with the same arguments - same seeded inputs - can be compared output for output.
 Prints ONE JSON line on rank 0.
 """
 from __future__ import annotations
@@ -294,6 +296,52 @@ class C2Slide:
         self.eng.grid_build(self.d_xy, self.d_ty, None, self.cell, self.bounds)
         self.out = self.eng.radius_graph(RADIUS, upper=True, n_types=N_TYPES, want_dist32=True, want_edges=True,
                                          capacity=self.cap, out=self.out)
+
+
+DUMP_ROWS = 1 << 18       # rows kept of each per-nucleus / per-edge output: ~25 MB of .npy for the 1 M slide
+DUMP_MAX_BYTES = 64 * 10**6
+
+
+def last_step_outputs(slide):
+    """Host copies of what a C2 step hands its caller: the per-nucleus outputs (degree, nbr_count, upper-CSR row_ptr),
+    the valid prefix of the pre-sized per-edge outputs (edges, col, float32 dist; row_ptr[-1] entries) and the degree
+    statistics. Indices and counts are stored as float64 (exact), dist as float32. Outputs longer than DUMP_ROWS rows
+    keep a fixed seeded sample of rows (node_rows / edge_rows, stored too); the sample depends only on N and E."""
+    import torch
+
+    from path_gene_multimodal_b200.engine import Engine
+
+    o = slide.out
+    n_edges = int(o["row_ptr"][-1])
+    rng = np.random.default_rng(0)
+
+    def rows(count):
+        return np.arange(count) if count <= DUMP_ROWS else np.sort(rng.choice(count, DUMP_ROWS, replace=False))
+
+    node_rows, edge_rows = rows(slide.n), rows(n_edges)
+    ni = torch.from_numpy(node_rows).to(o["row_ptr"].device)
+    ei = torch.from_numpy(edge_rows).to(o["row_ptr"].device)
+
+    def f64(t):
+        return t.cpu().numpy().astype(np.float64)
+
+    st = Engine.decode_stats(o["stats"], o["hist"])
+    return {
+        "node_rows": node_rows.astype(np.float64), "degree": f64(o["degree"][ni]), "nbr_count": f64(o["nbr_count"][ni]),
+        "row_ptr": f64(o["row_ptr"][ni]),
+        "edge_rows": edge_rows.astype(np.float64), "edges": f64(o["edges"][ei]), "col": f64(o["col"][ei]),
+        "dist": o["dist32"][ei].cpu().numpy(),
+        "n_edges": np.array([n_edges], dtype=np.float64),
+        "degree_stats": np.array([st["min"], st["max"], st["sum"], st["sumsq"], st["n"]], dtype=np.float64),
+        "degree_hist": st["hist"].astype(np.float64),
+    }
+
+
+def write_outputs(out_dir, arrays):
+    total = sum(a.nbytes for a in arrays.values())
+    assert total <= DUMP_MAX_BYTES, f"output dump of {total} bytes exceeds {DUMP_MAX_BYTES}"
+    for name, a in arrays.items():
+        np.save(Path(out_dir) / f"{name}.npy", a)
 
 
 def timed_steps(fn, flush, steps, warmup):
@@ -598,6 +646,7 @@ def run_ours(args, rank, world, local_rank):
     barrier()
     step_ms = timed_steps(run_step, flush, args.steps, 0)
     barrier()
+    dump = last_step_outputs(slide) if args.dump_outputs and rank == 0 else None
     launches = launches_per_step * args.steps
     eng.check_overflow()
     total_ms = float(sum(step_ms))
@@ -645,6 +694,8 @@ def run_ours(args, rank, world, local_rank):
     e2e_n = e2e("notebook")
     e2e_n["api"] = "the same call with outputs='notebook': host edge_index int64 [2,2E] / edge_attr float32 [2E,1] / degree / nbr_count"
     clocks = sampler.stop() if rank == 0 else None
+    if dump is not None:
+        write_outputs(args.dump_outputs, dump)
 
     line = {
         "metric": METRIC, "value": value, "unit": "nuclei/s", "n_gpus": world, "steps": args.steps, "warmup": warm,
@@ -873,7 +924,13 @@ def main():
     ap.add_argument("--steps", type=int, default=20)
     ap.add_argument("--warmup", type=int, default=3)
     ap.add_argument("--impl", choices=["ours", "reference"], default="ours")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the outputs of the last timed step (rank 0's slide) as DIR/<name>.npy, float32 / float64")
     args = ap.parse_args()
+    if args.dump_outputs:
+        if args.impl != "ours":
+            ap.error("--dump-outputs writes the outputs of --impl ours")
+        Path(args.dump_outputs).mkdir(parents=True, exist_ok=True)
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))

@@ -1,8 +1,7 @@
-"""CPU: the oracle against the committed golden vectors (reference-generated), the notebook's stored
-numbers (SURVEY Appendix D), brute force, networkx and - when /root/reference is mounted - the reference's
-own add_wsi_coords_to_nuclei."""
+"""CPU: the oracle against the committed golden vectors (reference-generated, including the reference's own
+add_wsi_coords_to_nuclei outputs and error message), the notebook's stored numbers (SURVEY Appendix D), brute force
+and networkx."""
 import numpy as np
-import pandas as pd
 import pytest
 
 from conftest import GOLDEN, frames_from_golden
@@ -27,19 +26,16 @@ def test_tile_to_wsi_oracle_matches_reference_golden(golden_add_wsi):
     assert got["wsi_polygon"].iloc[3] is None and got["wsi_polygon"].iloc[10] is None
 
 
-def test_tile_to_wsi_oracle_matches_live_reference_when_mounted():
-    ref = omap.load_reference_function()
-    if ref is None:
-        pytest.skip("/root/reference not mounted (GPU box): covered by the committed golden vectors")
-    tab = synth.make_table(300, seed=9, dtype=np.float64)
-    nuc, tiles = synth.to_frames(tab, closed_rings=True)
-    pd.testing.assert_frame_equal(ref(nuc, tiles), omap.add_wsi_coords_to_nuclei_oracle(nuc, tiles))
-    bad = nuc.copy()
-    bad.loc[0, "tile_path"] = "/x/y/nope.png"
-    with pytest.raises(ValueError):
-        ref(bad, tiles)
-    with pytest.raises(ValueError):
-        omap.add_wsi_coords_to_nuclei_oracle(bad, tiles)
+def test_tile_to_wsi_oracle_missing_tile_raises_like_reference(golden_add_wsi):
+    # the frame the reference raised on when tests/golden/add_wsi_ref_error.txt was written (oracle/make_golden.py)
+    nuc, tiles, _ = frames_from_golden(golden_add_wsi)
+    nuc.loc[2, "tile_path"] = "/nowhere/patches/123_456.png"
+    ref_msg = (GOLDEN / "add_wsi_ref_error.txt").read_text()
+    with pytest.raises(ValueError) as ei:
+        omap.add_wsi_coords_to_nuclei_oracle(nuc, tiles)
+    head = "Some nuclei have tile_key with no matching tile coords:"
+    assert ref_msg.startswith(head) and str(ei.value).startswith(head)
+    assert "123_456" in ref_msg and "123_456" in str(ei.value)
 
 
 def test_map_arrays_equals_frame_oracle():
