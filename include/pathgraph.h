@@ -329,6 +329,27 @@ int pg_raster_solidity(pg_handle* h, int32_t height, int32_t width, const int32_
                        const int32_t* area, const int32_t* bbox, int32_t* convex_area, double* solidity,
                        pg_stream stream);
 
+/* ---- K14: per-ring convex hull (cell 18's `solidity` and `orientation`, ipynb:2415-2456, for the polygons K1 measures).
+ *   poly_off   int32 [N+1]  CSR offsets into poly_xy (vertex units), as for pg_map_morph
+ *   n_vertices              vertices in poly_xy (M); sizes the workspace of rings that do not fit a shared-memory slab
+ *   poly_xy    T     [M,2]  ring vertices, interleaved x,y, any order or self-intersection; closing vertex optional
+ * Outputs float64 [N], each may be NULL:
+ *   convex_area  area of the convex hull of the ring's vertices (Andrew's monotone chain)
+ *   solidity     |shoelace area| / convex_area
+ *   orientation  skimage's: 0.5 atan2(-2b, c - a) with (a, b, c) = (mu_xx, -mu_xy, mu_yy) of the ring's area moments,
+ *                x = column, y = row (+-pi/4 when a == c): pi/2 in magnitude for a ring long along x, 0 along y.
+ * Rows with < 3 vertices give NaN everywhere; zero area gives NaN solidity / orientation; zero convex area gives
+ * convex_area 0 and NaN solidity. Exact (float64 terms are integers / 4) for vertices on the half-pixel lattice. */
+typedef struct {
+  double* convex_area;
+  double* solidity;
+  double* orientation;
+} pg_hull_out;
+int pg_ring_hull_f32(pg_handle* h, int32_t n, int64_t n_vertices, const int32_t* poly_off, const float* poly_xy,
+                     const pg_hull_out* out, pg_stream stream);
+int pg_ring_hull_f64(pg_handle* h, int32_t n, int64_t n_vertices, const int32_t* poly_off, const double* poly_xy,
+                     const pg_hull_out* out, pg_stream stream);
+
 /* ---- K13: instance map -> one polygon per instance (SURVEY 8f-3): aggregated_hovernet_run.py:183-198 -
  * find_contours(inst_map == id, 0.5), the longest contour, (x, y) = (col, row), approximate_polygon(tolerance).
  * area / bbox are pg_raster_props outputs for the same map. count: poly_off int32 [n_labels + 1] (device, 16-byte

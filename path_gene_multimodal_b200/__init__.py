@@ -4,7 +4,8 @@ neighbour-type composition and degree statistics.
 
 Public surface (reference-style module-level functions; see DESIGN.md / INTEGRATION.md):
     add_wsi_coords_to_nuclei, map_morph_arrays            (nuclei_wsi)
-    polygon_morphology_table, nuclei_morphology_table     (polygon_morphology)
+    polygon_morphology_table, nuclei_morphology_table,
+    hull_arrays                                           (polygon_morphology)
     build_knn_graph, build_radius_graph,
     neighbour_type_composition, degree_stats,
     filter_graph_by_type, clustering_coefficients,
@@ -25,6 +26,7 @@ _EXPORTS = {
     "polygons_to_csr": "nuclei_wsi", "csr_to_polygons": "nuclei_wsi",
     "polygon_morphology_table": "polygon_morphology", "nuclei_morphology_table": "polygon_morphology",
     "tag_polygons": "polygon_morphology", "zscore_columns": "polygon_morphology",
+    "hull_arrays": "polygon_morphology",
     "build_knn_graph": "cell_graph", "build_radius_graph": "cell_graph",
     "neighbour_type_composition": "cell_graph", "degree_stats": "cell_graph",
     "filter_graph_by_type": "cell_graph", "clustering_coefficients": "cell_graph",

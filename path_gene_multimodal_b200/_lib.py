@@ -46,6 +46,10 @@ class PgRasterOut(C.Structure):
                                         "minor_axis", "orientation")]
 
 
+class PgHullOut(C.Structure):
+    _fields_ = [(name, vp) for name in ("convex_area", "solidity", "orientation")]
+
+
 class PathGraphError(RuntimeError):
     def __init__(self, code: int, msg: str):
         super().__init__(f"libpathgraph error {code}: {msg}")
@@ -101,6 +105,8 @@ SIGNATURES = {
     "pg_type_interactions": (C.c_int, [vp, i32, vp, vp, i32, vp, vp]),
     "pg_raster_props": (C.c_int, [vp, i32, i32, vp, i32, C.POINTER(PgRasterOut), vp]),
     "pg_raster_solidity": (C.c_int, [vp, i32, i32, vp, i32, vp, vp, vp, vp, vp]),
+    "pg_ring_hull_f32": (C.c_int, [vp, i32, i64, vp, vp, C.POINTER(PgHullOut), vp]),
+    "pg_ring_hull_f64": (C.c_int, [vp, i32, i64, vp, vp, C.POINTER(PgHullOut), vp]),
     "pg_instance_contours_count": (C.c_int, [vp, i32, i32, vp, i32, vp, vp, f64, vp, vp]),
     "pg_instance_contours_total": (C.c_int, [vp, C.POINTER(i64)]),
     "pg_instance_contours_fill": (C.c_int, [vp, i32, vp, vp, vp]),

@@ -77,6 +77,8 @@ struct pg_handle {
   int64_t contour_raw = 0;
   size_t morph_smem_set[2][3] = {{0, 0, 0}, {0, 0, 0}};  // K1: dynamic shared memory opted in on this handle's device, per [T][EXTRA]
   double morph_mean_verts = 0;  // pg_map_morph_hint: expected vertices per ring (sizes K1's shared-memory slabs)
+  pg_buf hull;         // K14 (pg_hull.cu): chain buffers of the rings that do not fit a warp's slab
+  size_t hull_smem_set[2] = {0, 0};  // K14: dynamic shared memory opted in on this handle's device, per T
   // launch accounting / optional per-kernel CUDA-event timing (pg_profile_*)
   int64_t launches = 0;
   bool profiling = false;

@@ -13,7 +13,7 @@ import numpy as np
 import torch
 
 from . import _lib
-from ._lib import PathGraphError, PgMorphOut, PgRasterOut, PgUnionOut
+from ._lib import PathGraphError, PgHullOut, PgMorphOut, PgRasterOut, PgUnionOut
 
 _INF = float("inf")
 
@@ -194,6 +194,29 @@ class Engine:
                        self._p(bbox, torch.int32, "bbox"), self._p(wsi_poly, vt, "wsi_poly_xy"),
                        self._p(wsi_c, torch.float64, "wsi_centroid"), self._p(wsi_b, torch.int32, "wsi_bbox"),
                        C.byref(mo), self._stream()))
+        return res
+
+    # ---- K14 -----------------------------------------------------------------------------------
+    def ring_hull(self, poly_off, poly_xy, out=None):
+        """Convex area, solidity and orientation of every ring (pg_ring_hull_f32 / _f64).
+
+        poly_off int32 [N+1]; poly_xy float32|float64 [M,2].  Returns a dict of float64 device tensors [N]:
+        convex_area, solidity, orientation.  ``out`` may carry preallocated tensors of the same names.  Asynchronous
+        and free of host synchronisation once the workspace has grown, so it can be captured (``capture``)."""
+        n = int(poly_off.numel()) - 1
+        vt = poly_xy.dtype
+        if vt not in (torch.float32, torch.float64):
+            raise ValueError("poly_xy must be float32 or float64")
+        m = int(poly_xy.shape[0]) if poly_xy.dim() == 2 else int(poly_xy.numel() // 2)
+        res = dict(out) if out else {}
+        ho = PgHullOut()
+        for name in ("convex_area", "solidity", "orientation"):
+            if res.get(name) is None:
+                res[name] = self._empty((n,), torch.float64)
+            setattr(ho, name, self._p(res[name], torch.float64, name))
+        fn = self.lib.pg_ring_hull_f32 if vt == torch.float32 else self.lib.pg_ring_hull_f64
+        self._check(fn(self._h, n, m, self._p(poly_off, torch.int32, "poly_off"), self._p(poly_xy, vt, "poly_xy"),
+                       C.byref(ho), self._stream()))
         return res
 
     # ---- K2-K4 ---------------------------------------------------------------------------------

@@ -7,16 +7,20 @@
 * ``nuclei_morphology_table``   - the cell-18 columns of hovernet_tile_inference.ipynb:2415-2456
   (``area, perimeter, eccentricity, major_axis_length, minor_axis_length`` + derived
   ``perimeter_area, compactness, roundness, elongation``), evaluated on the ring's exact area moments
-  instead of a raster, and the cell-21 z-scores (ipynb:2903) on request.
+  instead of a raster, and the cell-21 z-scores (ipynb:2903) on request; with ``hull=True`` also cell 18's
+  ``solidity`` and ``orientation`` from the per-ring convex hull (pg_ring_hull_*).
 
-All features come from one launch of the fused kernel (pg_map_morph_*); the derived columns are
+All other features come from one launch of the fused kernel (pg_map_morph_*); the derived columns are
 the notebook's own pandas expressions on top.
 """
 from __future__ import annotations
 
 import numpy as np
 import pandas as pd
+import torch
 
+from . import _host
+from .engine import get_engine
 from .nuclei_wsi import map_morph_arrays, polygons_to_csr
 
 ISLAND_COLUMNS = ["area_px2", "perimeter_px", "centroid_x", "centroid_y",
@@ -84,20 +88,46 @@ def zscore_columns(df: pd.DataFrame, cols=CONT_COLS) -> pd.DataFrame:
     return df
 
 
-def nuclei_morphology_table(polygons, poly_off=None, inst_id=None, zscore: bool = False, device=None) -> pd.DataFrame:
+def hull_arrays(poly_off, poly_xy, device=None) -> dict:
+    """Array-level entry of the per-ring convex hull: numpy (host) in, numpy out, one kernel in between.
+
+    poly_off int32 [N+1]; poly_xy float32 or float64 [M,2] (the dtype chooses pg_ring_hull_f32 / _f64).  Returns
+    float64 [N] ``convex_area``, ``solidity`` (|area| / convex area) and ``orientation`` (skimage's convention, x =
+    column, y = row).  Rings with fewer than 3 vertices give NaN; see include/pathgraph.h for the other NaN rules."""
+    eng = get_engine(device)
+    dev = eng.device
+    vt = np.float32 if np.asarray(poly_xy).dtype == np.float32 else np.float64
+    d_off = _host.to_device(poly_off, np.int32, dev)
+    d_xy = _host.to_device(np.asarray(poly_xy).reshape(-1, 2), vt, dev)
+    with torch.cuda.device(dev):
+        res = eng.ring_hull(d_off, d_xy)
+        return {k: _host.to_host(v) for k, v in res.items()}
+
+
+def nuclei_morphology_table(polygons, poly_off=None, inst_id=None, zscore: bool = False, device=None,
+                            hull: bool = False) -> pd.DataFrame:
     """``morph_df`` of cell 18: ``inst_id, area, perimeter, eccentricity, major_axis_length,
-    minor_axis_length, perimeter_area, compactness, roundness, elongation`` (+ ``*_z``)."""
+    minor_axis_length, perimeter_area, compactness, roundness, elongation`` (+ ``*_z``).
+
+    ``hull=True`` adds ``solidity`` after ``eccentricity`` and ``orientation`` after ``minor_axis_length`` (cell 18's
+    order), from the ring's convex hull and area moments; ``zscore`` then also yields ``solidity_z``."""
     off, xy, _ = _as_csr(polygons, poly_off)
     res = map_morph_arrays(off, xy, write_polygons=False, extra=True, device=device)
     n = len(off) - 1
-    df = pd.DataFrame({
+    cols = {
         "inst_id": np.arange(1, n + 1) if inst_id is None else np.asarray(inst_id),
         "area": res["area"].astype(np.float64),
         "perimeter": res["perimeter"].astype(np.float64),
         "eccentricity": res["eccentricity"].astype(np.float64),
-        "major_axis_length": res["major_axis"].astype(np.float64),
-        "minor_axis_length": res["minor_axis"].astype(np.float64),
-    })
+    }
+    hres = hull_arrays(off, xy, device=device) if hull else None
+    if hull:
+        cols["solidity"] = hres["solidity"]
+    cols["major_axis_length"] = res["major_axis"].astype(np.float64)
+    cols["minor_axis_length"] = res["minor_axis"].astype(np.float64)
+    if hull:
+        cols["orientation"] = hres["orientation"]
+    df = pd.DataFrame(cols)
     df = derived_columns(df)
     df["circularity"] = res["circularity"].astype(np.float64)
     if zscore:
