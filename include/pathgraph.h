@@ -324,7 +324,8 @@ int pg_raster_props(pg_handle* h, int32_t height, int32_t width, const int32_t* 
 /* solidity = area / convex area (skimage regionprops: convex_hull_image of the region - the hull of the pixels' diamond
  * corners, rasterised with its border - cell 18's fourth property). area / bbox: pg_raster_props outputs of the same map.
  * convex_area int32 [n_labels], solidity float64 [n_labels] (NaN for absent labels); either may be NULL. Exact integer
- * arithmetic; one host synchronisation (workspace size). */
+ * arithmetic; one host synchronisation (workspace size). PG_ERR_INVALID when the workspace, sum 4 (2 rows + 1) over
+ * the labels' boxes, is past INT32_MAX entries. */
 int pg_raster_solidity(pg_handle* h, int32_t height, int32_t width, const int32_t* inst_map, int32_t n_labels,
                        const int32_t* area, const int32_t* bbox, int32_t* convex_area, double* solidity,
                        pg_stream stream);
@@ -357,7 +358,9 @@ int pg_ring_hull_f64(pg_handle* h, int32_t n, int64_t n_vertices, const int32_t*
  * inside count for the scratch); fill: poly_xy float64 [total][2], closed rings (first == last vertex) as skimage
  * returns them. Douglas-Peucker decisions are taken in exact integer arithmetic on the half-pixel lattice (a distance
  * equal to the tolerance is not "greater"; the first maximum splits) - skimage's float evaluation breaks such ties
- * by libm rounding. fill must follow its count on the same handle (the contours wait in the workspace). */
+ * by libm rounding. fill must follow its count on the same handle (the contours wait in the workspace). count
+ * returns PG_ERR_INVALID when its scratch (visited bits: a quarter byte per square of every label's window; raw
+ * contour vertices) is past INT32_MAX bytes / entries: many labels whose windows span a large map. */
 int pg_instance_contours_count(pg_handle* h, int32_t height, int32_t width, const int32_t* inst_map,
                                int32_t n_labels, const int32_t* area, const int32_t* bbox, double tolerance,
                                int32_t* poly_off, pg_stream stream);

@@ -115,6 +115,7 @@ struct pg_kernel_scope {
 #define PG_MISC_BADINPUT 72   // int32: build epoch of the last pg_grid_build that met a non-finite coordinate
 #define PG_MISC_TOTALS 128    // int32 x 8 totals copied to pinned memory: [0] radius [1] union [2] upper [3] contour scans; [4..5] uint64 overflow-region entries the last count pass needed
 #define PG_MISC_TMPCUR 192    // uint64 allocation cursor of tmp_ent's overflow region (zero between count passes: the row pass moves it to TOTALS[4..5])
+#define PG_MISC_SUM64 200     // int64: 64-bit total of the last pg_scan_i32_total (copied to pinned[12..13])
 #define PG_MISC_FEAT_TICKET 4608  // uint32 [PG_FEAT_MAX_COLS] CTA tickets of feature_stats_kernel, one per column (zero between launches)
 #define PG_FEAT_MAX_COLS 256
 #define PG_MISC_ACC 256       // pg_stats_acc: degree-statistics accumulators kept in their reset state
@@ -179,6 +180,11 @@ struct pg_scan_publish {
 };
 int pg_scan_i32(pg_handle* h, const int32_t* in, int32_t* out, int32_t n, cudaStream_t s, int32_t* total_copy = nullptr,
                 bool clear_in = false, const pg_scan_publish* publish = nullptr);
+// pg_scan_i32 of non-negative counts whose total the host needs: the total is also summed in 64 bits and read back
+// into *total (synchronises the stream). PG_ERR_INVALID, naming `what`, when it is past INT32_MAX: the int32
+// offsets would have wrapped.
+int pg_scan_i32_total(pg_handle* h, const int32_t* in, int32_t* out, int32_t n, cudaStream_t s, int32_t* total_copy,
+                      const char* what, int64_t* total);
 
 static inline int pg_div_up(int64_t a, int64_t b) { return (int)((a + b - 1) / b); }
 

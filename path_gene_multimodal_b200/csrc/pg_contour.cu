@@ -272,17 +272,15 @@ int pg_instance_contours_count(pg_handle* h, int32_t height, int32_t width, cons
   h->contour_empty = false;
   PG_LAUNCH(h, s, "contour_window_kernel", contour_window_kernel<<<blocks, TPB, 0, s>>>(area, bbox, n_labels, height, width, cnt));
   PG_LAUNCH_CHECK(h);
-  if ((rc = pg_scan_i32(h, cnt, vis_off, n_labels, s, totals + 3))) return rc;
-  PG_CUDA(h, cudaMemcpyAsync(&h->pinned[10], totals + 3, sizeof(int32_t), cudaMemcpyDeviceToHost, s));
-  PG_CUDA(h, cudaStreamSynchronize(s));
-  if ((rc = pg_reserve(h, h->cell_of, (size_t)h->pinned[10] + 64))) return rc;
+  int64_t n_vis;  // visited bytes, then raw vertices: both totals are checked against the int32 offsets in 64 bits
+  if ((rc = pg_scan_i32_total(h, cnt, vis_off, n_labels, s, totals + 3, "pg_instance_contours_count (visited bits)", &n_vis))) return rc;
+  if ((rc = pg_reserve(h, h->cell_of, (size_t)n_vis + 64))) return rc;
   PG_LAUNCH(h, s, "contour_pick_kernel", contour_pick_kernel<<<blocks, TPB, 0, s>>>(inst_map, height, width, area, bbox, n_labels, vis_off,
                                                                                        (uint8_t*)h->cell_of.p, picks, cnt));
   PG_LAUNCH_CHECK(h);
-  if ((rc = pg_scan_i32(h, cnt, raw_off, n_labels, s, totals + 3))) return rc;
-  PG_CUDA(h, cudaMemcpyAsync(&h->pinned[10], totals + 3, sizeof(int32_t), cudaMemcpyDeviceToHost, s));
-  PG_CUDA(h, cudaStreamSynchronize(s));
-  const size_t n_raw = (size_t)h->pinned[10];
+  int64_t n_raw64;
+  if ((rc = pg_scan_i32_total(h, cnt, raw_off, n_labels, s, totals + 3, "pg_instance_contours_count (raw vertices)", &n_raw64))) return rc;
+  const size_t n_raw = (size_t)n_raw64;
   // raw vertices (int2) + stack (int2) in `rank`, keep flags in `cell_of` (the visited bits are done with)
   if ((rc = pg_reserve(h, h->rank, 2 * (n_raw + 8) * sizeof(int2)))) return rc;
   if ((rc = pg_reserve(h, h->cell_of, n_raw + 64))) return rc;

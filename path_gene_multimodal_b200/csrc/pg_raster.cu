@@ -120,11 +120,17 @@ raster_finish_kernel(const raster_acc* __restrict__ acc, int n_labels, pg_raster
   if (some) {
     const double n = (double)a.area;
     cr = (double)a.sr / n; cc = (double)a.sc / n;
-    // central moments from the exact integer raw moments: mu20 = sum r^2 - (sum r)^2 / n, ...
-    const double mu20 = (double)a.srr - (double)a.sr * (double)a.sr / n;
-    const double mu02 = (double)a.scc - (double)a.sc * (double)a.sc / n;
-    const double mu11 = (double)a.src - (double)a.sr * (double)a.sc / n;
-    const double ta = mu02 / n, tb = -mu11 / n, tc = mu20 / n;  // inertia tensor [[ta, tb], [tb, tc]]
+    // exact integer central moments, each rounded once: n mu20 = n sum r^2 - (sum r)^2, ... in __int128
+    // (n < 2^31, sum r^2 < 2^63: every product < 2^95), and the tensor entry mu20 / n = (n mu20) / n^2.
+    // Subtracting the raw moments in float64 instead loses digits with the square of the region's distance
+    // from the origin (1e-7 in the axis lengths at 46000 px).
+    const __int128 n_ = a.area;
+    const __int128 sr = (__int128)a.sr, sc = (__int128)a.sc;
+    const double num20 = (double)(n_ * (__int128)a.srr - sr * sr);
+    const double num02 = (double)(n_ * (__int128)a.scc - sc * sc);
+    const double num11 = (double)(n_ * (__int128)a.src - sr * sc);
+    const double n2 = n * n;
+    const double ta = num02 / n2, tb = -(num11 / n2), tc = num20 / n2;  // inertia tensor [[ta, tb], [tb, tc]]
     const double mid = 0.5 * (ta + tc), hd = 0.5 * (ta - tc);
     const double rad = sqrt(hd * hd + tb * tb);
     const double l1 = fmax(mid + rad, 0.0), l2 = fmax(mid - rad, 0.0);
@@ -288,10 +294,9 @@ extern "C" int pg_raster_solidity(pg_handle* h, int32_t height, int32_t width, c
   const int blocks = pg_div_up(n_labels, TPB);
   PG_LAUNCH(h, s, "raster_rows_kernel", raster_rows_kernel<<<blocks, TPB, 0, s>>>(area, bbox, n_labels, need));
   PG_LAUNCH_CHECK(h);
-  if ((rc = pg_scan_i32(h, need, off, n_labels, s, totals + 3))) return rc;
-  PG_CUDA(h, cudaMemcpyAsync(&h->pinned[10], totals + 3, sizeof(int32_t), cudaMemcpyDeviceToHost, s));
-  PG_CUDA(h, cudaStreamSynchronize(s));
-  if ((rc = pg_reserve(h, h->rank, ((size_t)h->pinned[10] + 16) * sizeof(int32_t)))) return rc;
+  int64_t n_scratch;
+  if ((rc = pg_scan_i32_total(h, need, off, n_labels, s, totals + 3, "pg_raster_solidity", &n_scratch))) return rc;
+  if ((rc = pg_reserve(h, h->rank, ((size_t)n_scratch + 16) * sizeof(int32_t)))) return rc;
   PG_LAUNCH(h, s, "raster_solidity_kernel", raster_solidity_kernel<<<blocks, TPB, 0, s>>>(inst_map, height, width, area, bbox, n_labels, off,
                                                                                              (int32_t*)h->rank.p, convex_area, solidity));
   PG_LAUNCH_CHECK(h);

@@ -1,6 +1,9 @@
 // K3: single-pass exclusive scan (int32) used for cell_start and CSR row pointers.
 // The look-back machinery lives in pg_scan.cuh; this file is the plain array scan: tiles of 4096 items
 // (256 threads x 16), 1M items = 245 tiles = one look-back group, i.e. no serial chain at all.
+#include <algorithm>
+#include <climits>
+#include <cstring>
 #include "pg_scan.cuh"
 
 namespace {
@@ -73,6 +76,16 @@ __global__ void scan_empty_kernel(int32_t* out, int32_t* total_copy) {
   if (total_copy) *total_copy = 0;
 }
 
+// 64-bit sum of the scan's input (two's complement, so the unsigned atomics add signed values correctly)
+__global__ void __launch_bounds__(SCAN_THREADS)
+sum_i64_kernel(const int32_t* __restrict__ in, int32_t n, unsigned long long* __restrict__ sum) {
+  long long v = 0;
+  for (int64_t i = (int64_t)blockIdx.x * SCAN_THREADS + threadIdx.x; i < n; i += (int64_t)gridDim.x * SCAN_THREADS) v += in[i];
+#pragma unroll
+  for (int o = 16; o > 0; o >>= 1) v += __shfl_down_sync(0xffffffffu, v, o);
+  if ((threadIdx.x & 31) == 0 && v != 0) atomicAdd(sum, (unsigned long long)v);
+}
+
 }  // namespace
 
 int pg_scan_prepare(pg_handle* h, int num_tiles, int group, cudaStream_t s, pg_scan_state* st) {
@@ -117,6 +130,28 @@ int pg_scan_i32(pg_handle* h, const int32_t* in, int32_t* out, int32_t n, cudaSt
   else
     PG_LAUNCH(h, s, "scan_kernel", pg_launch_pdl(1, scan_kernel<false>, num_tiles, SCAN_THREADS, s, const_cast<int32_t*>(in), out, n, st, total_copy, pub));
   PG_LAUNCH_CHECK(h);
+  return PG_OK;
+}
+
+int pg_scan_i32_total(pg_handle* h, const int32_t* in, int32_t* out, int32_t n, cudaStream_t s, int32_t* total_copy,
+                      const char* what, int64_t* total) {
+  unsigned long long* sum = (unsigned long long*)((char*)h->misc.p + PG_MISC_SUM64);
+  PG_CUDA(h, cudaMemsetAsync(sum, 0, sizeof(*sum), s));
+  if (n > 0) {
+    const int blocks = (int)std::min<int64_t>(pg_div_up(n, SCAN_THREADS), 1024);
+    PG_LAUNCH(h, s, "sum_i64_kernel", sum_i64_kernel<<<blocks, SCAN_THREADS, 0, s>>>(in, n, sum));
+    PG_LAUNCH_CHECK(h);
+  }
+  int rc = pg_scan_i32(h, in, out, n, s, total_copy);
+  if (rc) return rc;
+  PG_CUDA(h, cudaMemcpyAsync(&h->pinned[12], sum, sizeof(*sum), cudaMemcpyDeviceToHost, s));
+  PG_CUDA(h, cudaStreamSynchronize(s));
+  int64_t t;
+  memcpy(&t, &h->pinned[12], sizeof(t));
+  if (t < 0 || t > INT32_MAX)
+    return pg_set_error(h, PG_ERR_INVALID, "%s: %lld scratch entries needed, more than int32 offsets address (%d)", what,
+                        (long long)t, INT32_MAX);
+  *total = t;
   return PG_OK;
 }
 
