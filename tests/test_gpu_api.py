@@ -271,7 +271,8 @@ def test_graph_statistics_against_networkx():
         G.add_edges_from(map(tuple, g["edges"]))
         st = clustering_coefficients(g["row_ptr"], g["col"])
         want = nx.clustering(G)
-        np.testing.assert_allclose(st["clustering"], [want[i] for i in range(len(xy))], rtol=1e-12, atol=0)
+        # one correctly rounded division of the same exact integers on both sides: bit for bit
+        assert np.array_equal(st["clustering"], [want[i] for i in range(len(xy))])
         tri = nx.triangles(G)
         assert np.array_equal(st["triangles"], [tri[i] for i in range(len(xy))])
         dc = nx.degree_centrality(G)
