@@ -239,7 +239,7 @@ int pg_compose_degree(pg_handle* h, int32_t n, const int32_t* row_ptr, const int
                       const int32_t* type, int32_t n_types, int32_t* nbr_count, int32_t* degree,
                       pg_degree_stats* stats, int32_t* hist, int32_t hist_len, pg_stream stream);
 
-/* ---- K9: halo selection for strip-sharded slides (no reference counterpart; SURVEY 8e).
+/* ---- K9: halo selection for strip-sharded slides (no reference counterpart; SURVEY 8e; csrc/pg_shard.cu).
  * Packs the points with x < lo_edge or x >= hi_edge into 24-byte records {x, y, gid, type}
  * (order unspecified); count_out int32 [1] device.  capacity in records. */
 typedef struct {
@@ -249,20 +249,15 @@ typedef struct {
 int pg_halo_pack(pg_handle* h, int32_t n, const double* xy, const int32_t* type, const int32_t* gid,
                  double lo_edge, double hi_edge, pg_halo_rec* out, int32_t capacity,
                  int32_t* count_out, pg_stream stream);
-/* Appends to xy/type/gid (starting at slot n_base) the records of `recs` whose x lies in
- * [x_lo, x_hi) and whose owner rank differs (recs from `skip_begin..skip_end` are this rank's own
- * contribution and are ignored). count_out int32 [1] device = number appended. */
-int pg_halo_unpack(pg_handle* h, const pg_halo_rec* recs, int32_t n_recs, int32_t skip_begin,
-                   int32_t skip_end, double x_lo, double x_hi, double* xy, int32_t* type,
-                   int32_t* gid, int32_t n_base, int32_t capacity, int32_t* count_out,
-                   pg_stream stream);
 
-/* Device-side exchange steps of the strip sharding (csrc/pg_shard.cu).
+/* Device-side exchange steps of the strip sharding (K9, csrc/pg_shard.cu).
  * pg_strip_partition: out = the n points as 24-byte records grouped by owning strip (strip q owns x in
  *   [inner_edges[q-1], inner_edges[q]); inner_edges host f64 [n_strips-1] ascending), input order kept inside every
  *   strip; totals int32 [n_strips] device = records per strip (the send counts of the all-to-all).
- * pg_halo_unpack_multi: pg_halo_unpack for n_ranges x-ranges (host f64 [n_ranges][2], appended in that order behind
- *   slot n_base) in one enqueue; counts_out int32 [n_ranges] device.
+ * pg_halo_unpack_multi: appends to xy/type/gid, starting at slot n_base, the records of `recs` whose x lies in an
+ *   x-range [x_lo, x_hi) of ranges (host f64 [n_ranges][2], appended in that order) in one enqueue; recs
+ *   skip_begin..skip_end-1 are this rank's own contribution and are ignored. counts_out int32 [n_ranges] device =
+ *   number appended per range.
  * pg_gid_maps: id_map int32 [n_ids] = row of every global id among the first n_rows points (-1 elsewhere) and
  *   type_by_gid int32 [n_ids] = type of every id among all n points (0 elsewhere); either may be NULL. */
 int pg_strip_partition(pg_handle* h, int32_t n, const double* xy, const int32_t* type, const int32_t* gid,

@@ -93,7 +93,6 @@ SIGNATURES = {
     "pg_csr_upper_fill": (C.c_int, [vp, i32, vp, vp, vp, vp, vp, vp, vp, vp, vp, vp]),
     "pg_compose_degree": (C.c_int, [vp, i32, vp, vp, vp, i32, vp, vp, vp, vp, i32, vp]),
     "pg_halo_pack": (C.c_int, [vp, i32, vp, vp, vp, f64, f64, vp, i32, vp, vp]),
-    "pg_halo_unpack": (C.c_int, [vp, vp, i32, i32, i32, f64, f64, vp, vp, vp, i32, i32, vp, vp]),
     "pg_strip_partition": (C.c_int, [vp, i32, vp, vp, vp, i32, C.POINTER(f64), vp, vp, vp]),
     "pg_halo_unpack_multi": (C.c_int, [vp, vp, i32, i32, i32, i32, C.POINTER(f64), vp, vp, vp, i32, i32, vp, vp]),
     "pg_widen_halfpx": (C.c_int, [vp, i64, vp, vp, vp]),

@@ -628,64 +628,6 @@ interactions_kernel(const int32_t* __restrict__ type, const int32_t* __restrict_
     if (s_acc[q]) atomicAdd(&inter[q], s_acc[q]);
 }
 
-// ---- K9 halo pack / unpack ---------------------------------------------------------------------
-__global__ void __launch_bounds__(TPB)
-halo_pack_kernel(const double2* __restrict__ xy, const int32_t* __restrict__ type, const int32_t* __restrict__ gid,
-                 int n, double lo_edge, double hi_edge, pg_halo_rec* __restrict__ out, int capacity,
-                 int32_t* count, int32_t* overflow) {
-  const int i = blockIdx.x * TPB + threadIdx.x;
-  bool take = false;
-  double2 p = make_double2(0, 0);
-  if (i < n) { p = xy[i]; take = p.x < lo_edge || p.x >= hi_edge; }
-  // warp-aggregated append: one atomic per warp
-  const unsigned m = __ballot_sync(0xffffffffu, take);
-  if (m == 0) return;
-  const int lane = threadIdx.x & 31;
-  int base = 0;
-  if (lane == __ffs(m) - 1) base = atomicAdd(count, __popc(m));
-  base = __shfl_sync(0xffffffffu, base, __ffs(m) - 1);
-  if (take) {
-    const int o = base + __popc(m & ((1u << lane) - 1));
-    if (o < capacity) {
-      pg_halo_rec r;
-      r.x = p.x; r.y = p.y; r.gid = gid ? gid[i] : i; r.type = type ? type[i] : 0;
-      out[o] = r;
-    } else {
-      atomicExch(overflow, 1);
-    }
-  }
-}
-
-__global__ void __launch_bounds__(TPB)
-halo_unpack_kernel(const pg_halo_rec* __restrict__ recs, int n_recs, int skip_begin, int skip_end, double x_lo,
-                   double x_hi, double2* __restrict__ xy, int32_t* __restrict__ type, int32_t* __restrict__ gid,
-                   int n_base, int capacity, int32_t* count, int32_t* overflow) {
-  const int i = blockIdx.x * TPB + threadIdx.x;
-  bool take = false;
-  pg_halo_rec r;
-  r.x = r.y = 0; r.gid = r.type = 0;
-  if (i < n_recs && !(i >= skip_begin && i < skip_end)) {
-    r = recs[i];
-    take = r.x >= x_lo && r.x < x_hi;
-  }
-  const unsigned m = __ballot_sync(0xffffffffu, take);
-  if (m == 0) return;
-  const int lane = threadIdx.x & 31;
-  int base = 0;
-  if (lane == __ffs(m) - 1) base = atomicAdd(count, __popc(m));
-  base = __shfl_sync(0xffffffffu, base, __ffs(m) - 1);
-  if (take) {
-    const int o = n_base + base + __popc(m & ((1u << lane) - 1));
-    if (o < capacity) {
-      xy[o] = make_double2(r.x, r.y);
-      if (type) type[o] = r.type;
-      if (gid) gid[o] = r.gid;
-    } else {
-      atomicExch(overflow, 1);
-    }
-  }
-}
-
 }  // namespace
 
 extern "C" {
@@ -924,41 +866,6 @@ int pg_type_interactions(pg_handle* h, int32_t n, const int32_t* type, const int
   const int blocks = std::min(pg_div_up(n, TPB), h->sm_count * 4);
   PG_LAUNCH(h, s, "interactions_kernel", interactions_kernel<<<blocks, TPB, 0, s>>>(type, nbr_count, n, n_types, (unsigned long long*)inter));
   PG_LAUNCH_CHECK(h);
-  return PG_OK;
-}
-
-int pg_halo_pack(pg_handle* h, int32_t n, const double* xy, const int32_t* type, const int32_t* gid,
-                 double lo_edge, double hi_edge, pg_halo_rec* out, int32_t capacity, int32_t* count_out,
-                 pg_stream stream) {
-  if (!h) return PG_ERR_INVALID;
-  cudaStream_t s = (cudaStream_t)stream;
-  PG_CUDA(h, cudaSetDevice(h->device));
-  h->last_stream = s;
-  PG_REQUIRE(h, n >= 0 && capacity >= 0 && count_out && (capacity == 0 || out), "pg_halo_pack: bad argument");
-  PG_CUDA(h, cudaMemsetAsync(count_out, 0, sizeof(int32_t), s));
-  if (n > 0) {
-    PG_LAUNCH(h, s, "halo_pack_kernel", halo_pack_kernel<<<pg_div_up(n, TPB), TPB, 0, s>>>((const double2*)xy, type, gid, n, lo_edge, hi_edge, out, capacity,
-                                                      count_out, (int32_t*)((char*)h->misc.p + PG_MISC_OVERFLOW)));
-    PG_LAUNCH_CHECK(h);
-  }
-  return PG_OK;
-}
-
-int pg_halo_unpack(pg_handle* h, const pg_halo_rec* recs, int32_t n_recs, int32_t skip_begin, int32_t skip_end,
-                   double x_lo, double x_hi, double* xy, int32_t* type, int32_t* gid, int32_t n_base,
-                   int32_t capacity, int32_t* count_out, pg_stream stream) {
-  if (!h) return PG_ERR_INVALID;
-  cudaStream_t s = (cudaStream_t)stream;
-  PG_CUDA(h, cudaSetDevice(h->device));
-  h->last_stream = s;
-  PG_REQUIRE(h, n_recs >= 0 && n_base >= 0 && capacity >= n_base && count_out && xy, "pg_halo_unpack: bad argument");
-  PG_CUDA(h, cudaMemsetAsync(count_out, 0, sizeof(int32_t), s));
-  if (n_recs > 0) {
-    PG_LAUNCH(h, s, "halo_unpack_kernel", halo_unpack_kernel<<<pg_div_up(n_recs, TPB), TPB, 0, s>>>(recs, n_recs, skip_begin, skip_end, x_lo, x_hi, (double2*)xy,
-                                                             type, gid, n_base, capacity, count_out,
-                                                             (int32_t*)((char*)h->misc.p + PG_MISC_OVERFLOW)));
-    PG_LAUNCH_CHECK(h);
-  }
   return PG_OK;
 }
 

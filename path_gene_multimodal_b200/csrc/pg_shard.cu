@@ -1,11 +1,13 @@
 // Strip sharding of one giant slide (SURVEY 8e, BASELINE config 5): the device-side pieces of the exchange steps
-// that the first version left to eager torch ops (bucketize / argsort / index_put):
+// (K9), most of which the first version left to eager torch ops (bucketize / argsort / index_put):
 //   pg_strip_partition   points -> 24-byte records grouped by owning strip (the send buffer of the all-to-all),
 //                        stable and deterministic: count per (strip, CTA) -> one look-back scan -> placement by
 //                        warp match + in-CTA prefix. No atomics, no sort.
-//   pg_halo_unpack_multi several x-ranges of the gathered halo records appended behind the owned points in one
-//                        enqueue (each range starts where the previous one ended, read on the device), so the
-//                        host reads all counts with ONE synchronisation.
+//   pg_halo_pack / _push the points near the strip edges -> 24-byte records, into a local buffer (then all-gathered)
+//                        or straight into every peer's receive slab.
+//   pg_halo_unpack_multi several x-ranges of the gathered (or, _slab, the received) halo records appended behind the
+//                        owned points in one enqueue (each range starts where the previous one ended, read on the
+//                        device), so the host reads all counts with ONE synchronisation.
 //   pg_gid_maps          dense maps global id -> local row and global id -> type for the undirected union of a
 //                        strip + halo (rows address their neighbours by global id).
 // No reference counterpart: the reference runs one slide per LSF job (/root/reference/main.py:322-335).
@@ -71,39 +73,6 @@ partition_place_kernel(const double2* __restrict__ xy, const int32_t* __restrict
     totals[threadIdx.x] = base[(int64_t)(threadIdx.x + 1) * n_cta] - base[(int64_t)threadIdx.x * n_cta];
 }
 
-// appends the records of one x-range; the first free slot is n_base + the counts of the ranges before this one
-__global__ void __launch_bounds__(TPB)
-halo_unpack_range_kernel(const pg_halo_rec* __restrict__ recs, int n_recs, int skip_begin, int skip_end, double x_lo,
-                         double x_hi, double2* __restrict__ xy, int32_t* __restrict__ type, int32_t* __restrict__ gid,
-                         int n_base, int capacity, int32_t* counts, int range, int32_t* overflow) {
-  const int i = blockIdx.x * TPB + threadIdx.x;
-  int first = n_base;
-  for (int q = 0; q < range; ++q) first += counts[q];
-  bool take = false;
-  pg_halo_rec r;
-  r.x = r.y = 0; r.gid = r.type = 0;
-  if (i < n_recs && !(i >= skip_begin && i < skip_end)) {
-    r = recs[i];
-    take = r.x >= x_lo && r.x < x_hi;
-  }
-  const unsigned m = __ballot_sync(0xffffffffu, take);
-  if (m == 0) return;
-  const int lane = threadIdx.x & 31;
-  int at = 0;
-  if (lane == __ffs(m) - 1) at = atomicAdd(&counts[range], __popc(m));
-  at = __shfl_sync(0xffffffffu, at, __ffs(m) - 1);
-  if (take) {
-    const int o = first + at + __popc(m & ((1u << lane) - 1u));
-    if (o < capacity) {
-      xy[o] = make_double2(r.x, r.y);
-      if (type) type[o] = r.type;
-      if (gid) gid[o] = r.gid;
-    } else {
-      atomicExch(overflow, 1);
-    }
-  }
-}
-
 // ---- compact staging format of contour vertices: int16 half-pixels -> float32 pixels.
 // skimage.measure.find_contours(mask, 0.5) (aggregated_hovernet_run.py:185) puts every vertex on the half-pixel
 // lattice of its tile, so 2 * coordinate is a small integer: a table staged as int16 pairs carries the polygons in 4
@@ -128,34 +97,61 @@ widen_halfpx_kernel(const int16_t* __restrict__ in, float* __restrict__ out, int
   }
 }
 
-// ---- the halo exchange as ONE step over NVLink peer memory: pack + all-gather fused -----------------------------
-// Every rank owns a receive slab [world][cap] of 24-byte records followed by [world] int32 counts, mapped into all
-// ranks (symmetric memory). The pack kernel of rank r writes each selected record straight into slot [r][o] of every
-// peer's slab (P2P stores through NVSwitch); a one-warp kernel then publishes the count. No staging buffer, no padded
-// payload, no collective library call, and no host read to size anything - the receiver's unpack kernel walks
-// world x cap slots and takes the first count[src] of every source.
+// ---- K9: the halo exchange ---------------------------------------------------------------------------------------
+// A rank selects its points near the strip edges into 24-byte records; the receiver appends the records of each x-range
+// behind its owned points. Two transports share the select and the append:
+//   NCCL:        pack into a local buffer -> all-gather (sharding.py) -> unpack the flat gathered array, skipping this
+//                rank's own window.
+//   peer memory: every rank owns a receive slab [world][cap] of records followed by [world] int32 counts, mapped into
+//                all ranks (symmetric memory). The select kernel of rank r stores each record straight into slot [r][o]
+//                of every peer's slab (P2P stores through NVSwitch); a one-warp kernel then publishes the count. No
+//                staging buffer, no padded payload, no collective library call, and no host read to size anything -
+//                the receiver's unpack walks world x cap slots and takes the first count[src] of every source.
+
+// Warp-aggregated append, one atomic per warp: the lanes with `take` get consecutive slots of the list counted by
+// *count. Returns the lane's slot, -1 without `take`. Every lane of the warp calls it.
+__device__ __forceinline__ int warp_append(bool take, int32_t* count) {
+  const unsigned m = __ballot_sync(0xffffffffu, take);
+  if (m == 0) return -1;
+  const int lane = threadIdx.x & 31, leader = __ffs(m) - 1;
+  int base = 0;
+  if (lane == leader) base = atomicAdd(count, __popc(m));
+  base = __shfl_sync(0xffffffffu, base, leader);
+  return take ? base + __popc(m & ((1u << lane) - 1u)) : -1;
+}
+
+// where a selected record goes (slot o < cap)
+struct local_dst {     // pg_halo_pack: a buffer of cap records
+  pg_halo_rec* out;
+  int cap;
+  __device__ void store(int o, const pg_halo_rec& r) const { out[o] = r; }
+};
+struct peer_dst {      // pg_halo_push: slot [rank][o] of every peer's slab
+  const unsigned long long* peer_ptrs;   // read through __ldg: nvcc ignores __restrict__ on a struct member, and without
+  int world, rank, cap;                  // it every peer store would be assumed to alias the table
+  __device__ void store(int o, const pg_halo_rec& r) const {
+    PG_ASSERT(o >= 0 && o < cap && rank >= 0 && rank < world);
+    for (int q = 0; q < world; ++q)
+      if (q != rank) reinterpret_cast<pg_halo_rec*>(__ldg(&peer_ptrs[q]))[(size_t)rank * cap + o] = r;
+  }
+};
+
+// the points with x < lo_edge or x >= hi_edge (never a NaN x); *count counts all of them, slots past dst.cap raise the
+// overflow flag. Profiled as halo_pack_kernel / halo_push_kernel.
+template <class Dst>
 __global__ void __launch_bounds__(TPB)
-halo_push_kernel(const double2* __restrict__ xy, const int32_t* __restrict__ type, const int32_t* __restrict__ gid, int n,
-                 double lo_edge, double hi_edge, const unsigned long long* __restrict__ peer_ptrs, int world, int rank, int cap,
-                 int32_t* count, int32_t* overflow) {
+halo_select_kernel(const double2* __restrict__ xy, const int32_t* __restrict__ type, const int32_t* __restrict__ gid,
+                   int n, double lo_edge, double hi_edge, Dst dst, int32_t* count, int32_t* overflow) {
   const int i = blockIdx.x * TPB + threadIdx.x;
   bool take = false;
   double2 p = make_double2(0, 0);
   if (i < n) { p = xy[i]; take = p.x < lo_edge || p.x >= hi_edge; }
-  const unsigned m = __ballot_sync(0xffffffffu, take);
-  if (m == 0) return;
-  const int lane = threadIdx.x & 31;
-  int base = 0;
-  if (lane == __ffs(m) - 1) base = atomicAdd(count, __popc(m));
-  base = __shfl_sync(0xffffffffu, base, __ffs(m) - 1);
-  if (!take) return;
-  const int o = base + __popc(m & ((1u << lane) - 1u));
-  if (o >= cap) { atomicExch(overflow, 1); return; }
+  const int o = warp_append(take, count);
+  if (o < 0) return;
+  if (o >= dst.cap) { atomicExch(overflow, 1); return; }
   pg_halo_rec r;
   r.x = p.x; r.y = p.y; r.gid = gid ? gid[i] : i; r.type = type ? type[i] : 0;
-  PG_ASSERT(o >= 0 && o < cap && rank >= 0 && rank < world);
-  for (int q = 0; q < world; ++q)
-    if (q != rank) reinterpret_cast<pg_halo_rec*>(peer_ptrs[q])[(size_t)rank * cap + o] = r;
+  dst.store(o, r);
 }
 
 __global__ void halo_push_counts_kernel(const unsigned long long* __restrict__ peer_ptrs, int world, int rank, int cap,
@@ -167,44 +163,71 @@ __global__ void halo_push_counts_kernel(const unsigned long long* __restrict__ p
   __threadfence_system();
 }
 
-// the receiver's side: slot s of the slab = entry s % cap of source s / cap, valid while below that source's count
+// has(s): whether slot s of an unpack's record array holds a record. slab_src::has also raises the overflow flag
+// (once per source) when a source's published count exceeds cap.
+struct gathered_src {  // pg_halo_unpack_multi: the flat gathered records; [skip_begin, skip_end) are this rank's own
+  using index = int;
+  int n_recs, skip_begin, skip_end;
+  __device__ bool has(int s, int32_t*) const { return s < n_recs && !(s >= skip_begin && s < skip_end); }
+};
+struct slab_src {      // pg_halo_unpack_slab: slot s = entry s % cap of source s / cap, valid below that source's count
+  using index = int64_t;       // world x cap may pass 2^31
+  const int32_t* src_counts;   // [world], behind the world x cap records
+  int world, rank, cap;
+  __device__ bool has(int64_t s, int32_t* overflow) const {
+    if (s >= (int64_t)world * cap) return false;
+    const int src = (int)(s / cap), idx = (int)(s - (int64_t)src * cap);
+    const int cnt = src != rank ? __ldg(&src_counts[src]) : 0;
+    if (idx == 0 && cnt > cap) atomicExch(overflow, 1);
+    return idx < min(cnt, cap);
+  }
+};
+
+// appends the records with x in [x_lo, x_hi) (never a NaN x); the first free slot is n_base + the counts of the
+// ranges before this one. Profiled as halo_unpack_range_kernel / halo_unpack_slab_kernel.
+template <class Src>
 __global__ void __launch_bounds__(TPB)
-halo_unpack_slab_kernel(const pg_halo_rec* __restrict__ slab, int world, int rank, int cap, double x_lo, double x_hi,
-                        double2* __restrict__ xy, int32_t* __restrict__ type, int32_t* __restrict__ gid, int n_base,
-                        int capacity, int32_t* counts, int range, int32_t* overflow) {
-  const int64_t s = (int64_t)blockIdx.x * TPB + threadIdx.x;
-  const int32_t* src_counts = reinterpret_cast<const int32_t*>(reinterpret_cast<const char*>(slab) + (size_t)world * cap * sizeof(pg_halo_rec));
+halo_unpack_kernel(const pg_halo_rec* __restrict__ recs, Src src, double x_lo, double x_hi, double2* __restrict__ xy,
+                   int32_t* __restrict__ type, int32_t* __restrict__ gid, int n_base, int capacity, int32_t* counts,
+                   int range, int32_t* overflow) {
+  const typename Src::index s = (typename Src::index)blockIdx.x * TPB + threadIdx.x;
   int first = n_base;
   for (int q = 0; q < range; ++q) first += counts[q];
   bool take = false;
   pg_halo_rec r;
   r.x = r.y = 0; r.gid = r.type = 0;
-  if (s < (int64_t)world * cap) {
-    const int src = (int)(s / cap), idx = (int)(s - (int64_t)src * cap);
-    const int cnt = src != rank ? src_counts[src] : 0;
-    if (idx == 0 && cnt > cap) atomicExch(overflow, 1);
-    if (idx < min(cnt, cap)) {
-      r = slab[s];
-      take = r.x >= x_lo && r.x < x_hi;
-    }
+  if (src.has(s, overflow)) {
+    r = recs[s];
+    take = r.x >= x_lo && r.x < x_hi;
   }
-  const unsigned m = __ballot_sync(0xffffffffu, take);
-  if (m == 0) return;
-  const int lane = threadIdx.x & 31;
-  int at = 0;
-  if (lane == __ffs(m) - 1) at = atomicAdd(&counts[range], __popc(m));
-  at = __shfl_sync(0xffffffffu, at, __ffs(m) - 1);
-  if (take) {
-    const int o = first + at + __popc(m & ((1u << lane) - 1u));
-    PG_ASSERT(o >= n_base);
-    if (o < capacity) {
-      xy[o] = make_double2(r.x, r.y);
-      if (type) type[o] = r.type;
-      if (gid) gid[o] = r.gid;
-    } else {
-      atomicExch(overflow, 1);
-    }
+  const int at = warp_append(take, &counts[range]);
+  if (at < 0) return;
+  const int o = first + at;
+  PG_ASSERT(o >= n_base);
+  if (o < capacity) {
+    xy[o] = make_double2(r.x, r.y);
+    if (type) type[o] = r.type;
+    if (gid) gid[o] = r.gid;
+  } else {
+    atomicExch(overflow, 1);
   }
+}
+
+// clears counts_out [n_ranges], then one launch per non-empty range over the `slots` records of recs
+template <class Src>
+int unpack_ranges(pg_handle* h, cudaStream_t s, const char* name, const pg_halo_rec* recs, Src src, int64_t slots,
+                  int32_t n_ranges, const double* ranges, double* xy, int32_t* type, int32_t* gid, int32_t n_base,
+                  int32_t capacity, int32_t* counts_out) {
+  PG_CUDA(h, cudaMemsetAsync(counts_out, 0, (size_t)n_ranges * sizeof(int32_t), s));
+  if (slots == 0) return PG_OK;
+  int32_t* ovf = (int32_t*)((char*)h->misc.p + PG_MISC_OVERFLOW);
+  for (int r = 0; r < n_ranges; ++r) {
+    if (!(ranges[2 * r + 1] > ranges[2 * r])) continue;  // empty range
+    PG_LAUNCH(h, s, name, halo_unpack_kernel<<<pg_div_up(slots, TPB), TPB, 0, s>>>(
+        recs, src, ranges[2 * r], ranges[2 * r + 1], (double2*)xy, type, gid, n_base, capacity, counts_out, r, ovf));
+    PG_LAUNCH_CHECK(h);
+  }
+  return PG_OK;
 }
 
 __global__ void __launch_bounds__(TPB)
@@ -297,6 +320,24 @@ int pg_strip_partition(pg_handle* h, int32_t n, const double* xy, const int32_t*
   return PG_OK;
 }
 
+int pg_halo_pack(pg_handle* h, int32_t n, const double* xy, const int32_t* type, const int32_t* gid,
+                 double lo_edge, double hi_edge, pg_halo_rec* out, int32_t capacity, int32_t* count_out,
+                 pg_stream stream) {
+  if (!h) return PG_ERR_INVALID;
+  cudaStream_t s = (cudaStream_t)stream;
+  PG_CUDA(h, cudaSetDevice(h->device));
+  h->last_stream = s;
+  PG_REQUIRE(h, n >= 0 && capacity >= 0 && count_out && (capacity == 0 || out), "pg_halo_pack: bad argument");
+  PG_CUDA(h, cudaMemsetAsync(count_out, 0, sizeof(int32_t), s));
+  if (n > 0) {
+    PG_LAUNCH(h, s, "halo_pack_kernel", halo_select_kernel<<<pg_div_up(n, TPB), TPB, 0, s>>>(
+        (const double2*)xy, type, gid, n, lo_edge, hi_edge, local_dst{out, capacity}, count_out,
+        (int32_t*)((char*)h->misc.p + PG_MISC_OVERFLOW)));
+    PG_LAUNCH_CHECK(h);
+  }
+  return PG_OK;
+}
+
 int pg_halo_unpack_multi(pg_handle* h, const pg_halo_rec* recs, int32_t n_recs, int32_t skip_begin, int32_t skip_end,
                          int32_t n_ranges, const double* ranges, double* xy, int32_t* type, int32_t* gid, int32_t n_base,
                          int32_t capacity, int32_t* counts_out, pg_stream stream) {
@@ -306,16 +347,8 @@ int pg_halo_unpack_multi(pg_handle* h, const pg_halo_rec* recs, int32_t n_recs, 
   h->last_stream = s;
   PG_REQUIRE(h, n_recs >= 0 && n_base >= 0 && capacity >= n_base && n_ranges >= 1 && n_ranges <= 8 && ranges && counts_out && xy,
              "pg_halo_unpack_multi: bad argument");
-  PG_CUDA(h, cudaMemsetAsync(counts_out, 0, (size_t)n_ranges * sizeof(int32_t), s));
-  if (n_recs == 0) return PG_OK;
-  int32_t* ovf = (int32_t*)((char*)h->misc.p + PG_MISC_OVERFLOW);
-  for (int r = 0; r < n_ranges; ++r) {
-    if (!(ranges[2 * r + 1] > ranges[2 * r])) continue;  // empty range
-    PG_LAUNCH(h, s, "halo_unpack_range_kernel", halo_unpack_range_kernel<<<pg_div_up(n_recs, TPB), TPB, 0, s>>>(
-        recs, n_recs, skip_begin, skip_end, ranges[2 * r], ranges[2 * r + 1], (double2*)xy, type, gid, n_base, capacity, counts_out, r, ovf));
-    PG_LAUNCH_CHECK(h);
-  }
-  return PG_OK;
+  return unpack_ranges(h, s, "halo_unpack_range_kernel", recs, gathered_src{n_recs, skip_begin, skip_end}, n_recs, n_ranges,
+                       ranges, xy, type, gid, n_base, capacity, counts_out);
 }
 
 int pg_widen_halfpx(pg_handle* h, int64_t n_values, const int16_t* in, float* out, pg_stream stream) {
@@ -343,9 +376,9 @@ int pg_halo_push(pg_handle* h, int32_t n, const double* xy, const int32_t* type,
   int32_t* count = (int32_t*)((char*)h->misc.p + PG_MISC_HALOCNT);
   PG_CUDA(h, cudaMemsetAsync(count, 0, sizeof(int32_t), s));
   if (n > 0) {
-    PG_LAUNCH(h, s, "halo_push_kernel", halo_push_kernel<<<pg_div_up(n, TPB), TPB, 0, s>>>(
-        (const double2*)xy, type, gid, n, lo_edge, hi_edge, (const unsigned long long*)peer_ptrs_dev, world, rank, cap, count,
-        (int32_t*)((char*)h->misc.p + PG_MISC_OVERFLOW)));
+    PG_LAUNCH(h, s, "halo_push_kernel", halo_select_kernel<<<pg_div_up(n, TPB), TPB, 0, s>>>(
+        (const double2*)xy, type, gid, n, lo_edge, hi_edge, peer_dst{(const unsigned long long*)peer_ptrs_dev, world, rank, cap},
+        count, (int32_t*)((char*)h->misc.p + PG_MISC_OVERFLOW)));
     PG_LAUNCH_CHECK(h);
   }
   PG_LAUNCH(h, s, "halo_push_counts_kernel", halo_push_counts_kernel<<<1, 1024, 0, s>>>((const unsigned long long*)peer_ptrs_dev, world, rank, cap, count));
@@ -362,16 +395,10 @@ int pg_halo_unpack_slab(pg_handle* h, const void* slab, int32_t world, int32_t r
   h->last_stream = s;
   PG_REQUIRE(h, slab && world >= 1 && rank >= 0 && rank < world && cap >= 1 && n_base >= 0 && capacity >= n_base &&
                     n_ranges >= 1 && n_ranges <= 8 && ranges && counts_out && xy, "pg_halo_unpack_slab: bad argument");
-  PG_CUDA(h, cudaMemsetAsync(counts_out, 0, (size_t)n_ranges * sizeof(int32_t), s));
-  int32_t* ovf = (int32_t*)((char*)h->misc.p + PG_MISC_OVERFLOW);
+  const pg_halo_rec* recs = (const pg_halo_rec*)slab;
   const int64_t slots = (int64_t)world * cap;
-  for (int r = 0; r < n_ranges; ++r) {
-    if (!(ranges[2 * r + 1] > ranges[2 * r])) continue;
-    PG_LAUNCH(h, s, "halo_unpack_slab_kernel", halo_unpack_slab_kernel<<<pg_div_up(slots, TPB), TPB, 0, s>>>(
-        (const pg_halo_rec*)slab, world, rank, cap, ranges[2 * r], ranges[2 * r + 1], (double2*)xy, type, gid, n_base, capacity, counts_out, r, ovf));
-    PG_LAUNCH_CHECK(h);
-  }
-  return PG_OK;
+  return unpack_ranges(h, s, "halo_unpack_slab_kernel", recs, slab_src{(const int32_t*)(recs + slots), world, rank, cap}, slots,
+                       n_ranges, ranges, xy, type, gid, n_base, capacity, counts_out);
 }
 
 int pg_gid_maps(pg_handle* h, int32_t n, int32_t n_rows, const int32_t* gid, const int32_t* type, int32_t n_ids,

@@ -581,14 +581,6 @@ class Engine:
                                           self._stream()))
         return recs, count
 
-    def halo_unpack(self, recs, n_recs, skip_begin, skip_end, x_lo, x_hi, xy, types, gid, n_base):
-        count = self._empty((1,), torch.int32)
-        self._check(self.lib.pg_halo_unpack(self._h, C.c_void_p(recs.data_ptr()), int(n_recs), int(skip_begin), int(skip_end),
-                                            float(x_lo), float(x_hi), self._p(xy, torch.float64, "xy"),
-                                            self._p(types, torch.int32, "types"), self._p(gid, torch.int32, "gid"),
-                                            int(n_base), int(xy.shape[0]), self._p(count, torch.int32, "count"), self._stream()))
-        return count
-
     def strip_partition(self, xy, types, gid, inner_edges):
         """Records (24 B: x, y, gid, type) of all points grouped by owning strip + per-strip totals (pg_strip_partition)."""
         n = int(xy.shape[0])

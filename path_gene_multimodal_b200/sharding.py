@@ -19,6 +19,7 @@ from __future__ import annotations
 
 import math
 from dataclasses import dataclass
+from functools import partial
 
 import numpy as np
 import torch
@@ -140,11 +141,9 @@ def exchange_halo(eng, xy, types, gid, strip: Strip, width: float, rank: int, wo
     read per exchange: the gathered counts (they size the padded payload); the pack kernel cannot overflow, its
     capacity is the number of points."""
     n = int(xy.shape[0])
-    lo_edge = -_INF if strip.is_first else strip.lo + width
-    hi_edge = _INF if strip.is_last else strip.hi - width
     if world == 1:
         return torch.empty((0, 3), dtype=torch.float64, device=xy.device), 0
-    recs, count = eng.halo_pack(xy, types, gid, lo_edge, hi_edge, capacity=max(n, 1))
+    recs, count = eng.halo_pack(xy, types, gid, strip.x_lo + width, strip.x_hi - width, capacity=max(n, 1))
     counts = yield ("all_gather", count)                    # [world, 1] int32
     counts = counts.reshape(-1).tolist()                    # host sync: sizes the padded payload
     max_cnt = max(max(counts), 1)
@@ -154,25 +153,33 @@ def exchange_halo(eng, xy, types, gid, strip: Strip, width: float, rank: int, wo
     return all_recs.reshape(world * max_cnt, 3).contiguous(), max_cnt
 
 
-def merge_halo(eng, xy, types, gid, all_recs, max_cnt, rank, ranges):
-    """Append to the owned points the gathered records whose x lies in each [a, b) of ``ranges`` (in that
-    order), skipping this rank's own contribution. Returns (xy_all, types_all, gid_all, [count per range]).
-    One enqueue for all ranges (pg_halo_unpack_multi) and one host read of the counts."""
+def _append_ghosts(xy, types, gid, ghost_cap: int, ranges, unpack):
+    """The owned points copied to the front of arrays with room for ``ghost_cap`` ghosts, behind which
+    ``unpack(ranges, xy_all, types_all, gid_all, n_owned)`` (Engine.halo_unpack_multi / _slab with the source bound)
+    appends the ghosts of each range. Returns (xy_all, types_all, gid_all, [count per range]) trimmed to the points
+    present. One host read; none when ``unpack`` is None (nothing to append)."""
     n = int(xy.shape[0])
-    n_recs = int(all_recs.shape[0])
-    cap = n + n_recs
+    cap = n + ghost_cap
     xy_all = torch.empty((cap, 2), dtype=torch.float64, device=xy.device)
     ty_all = torch.empty((cap,), dtype=torch.int32, device=xy.device)
     gid_all = torch.empty((cap,), dtype=torch.int32, device=xy.device)
     xy_all[:n] = xy
     ty_all[:n] = types
     gid_all[:n] = gid
-    if n_recs == 0:
+    if unpack is None:
         return xy_all[:n], ty_all[:n], gid_all[:n], [0] * len(ranges)
-    counts = eng.halo_unpack_multi(all_recs, n_recs, rank * max_cnt, (rank + 1) * max_cnt, ranges, xy_all, ty_all, gid_all, n)
-    got = counts.tolist()                                   # host sync: the grid build needs the point count
+    got = unpack(ranges, xy_all, ty_all, gid_all, n).tolist()   # host sync: the grid build needs the point count
     base = n + sum(got)
     return xy_all[:base], ty_all[:base], gid_all[:base], got
+
+
+def merge_halo(eng, xy, types, gid, all_recs, max_cnt, rank, ranges):
+    """Append to the owned points the gathered records whose x lies in each [a, b) of ``ranges`` (in that
+    order), skipping this rank's own contribution. Returns (xy_all, types_all, gid_all, [count per range]).
+    One enqueue for all ranges (pg_halo_unpack_multi) and one host read of the counts."""
+    n_recs = int(all_recs.shape[0])
+    unpack = partial(eng.halo_unpack_multi, all_recs, n_recs, rank * max_cnt, (rank + 1) * max_cnt) if n_recs else None
+    return _append_ghosts(xy, types, gid, n_recs, ranges, unpack)
 
 
 class PeerHalo:
@@ -199,22 +206,12 @@ class PeerHalo:
     def exchange(self, eng, xy, types, gid, strip: "Strip", width: float, ranges, ghost_cap: int | None = None):
         """Push this rank's edge points to every peer, then append the received records of each x-range to the owned
         points. Same return as merge_halo. One host read (the unpack counts + the overflow flag)."""
-        n = int(xy.shape[0])
-        lo_edge = -_INF if strip.is_first else strip.lo + width
-        hi_edge = _INF if strip.is_last else strip.hi - width
         self.hdl.barrier(channel=0)                             # every peer is done reading the previous exchange
-        eng.halo_push(xy, types, gid, lo_edge, hi_edge, self.ptrs_dev, self.world, self.rank, self.cap)
+        eng.halo_push(xy, types, gid, strip.x_lo + width, strip.x_hi - width, self.ptrs_dev, self.world, self.rank, self.cap)
         self.hdl.barrier(channel=0)                             # all records and counts have landed
         ghost_cap = int(ghost_cap) if ghost_cap is not None else min(self.world - 1, 4) * self.cap
-        cap = n + ghost_cap
-        xy_all = torch.empty((cap, 2), dtype=torch.float64, device=xy.device)
-        ty_all = torch.empty((cap,), dtype=torch.int32, device=xy.device)
-        gid_all = torch.empty((cap,), dtype=torch.int32, device=xy.device)
-        xy_all[:n] = xy
-        ty_all[:n] = types
-        gid_all[:n] = gid
-        counts = eng.halo_unpack_slab(self.buf, self.world, self.rank, self.cap, ranges, xy_all, ty_all, gid_all, n)
-        got = counts.tolist()                                   # host sync: the grid build needs the point count
+        out = _append_ghosts(xy, types, gid, ghost_cap, ranges,
+                             partial(eng.halo_unpack_slab, self.buf, self.world, self.rank, self.cap))
         try:
             eng.check_overflow()
         except RuntimeError as exc:
@@ -222,8 +219,16 @@ class PeerHalo:
                 raise
             raise RuntimeError(f"PeerHalo: a rank packed more than cap={self.cap} halo records (or more than {ghost_cap} "
                                "ghosts arrived here); build the PeerHalo with a larger cap") from exc
-        base = n + sum(got)
-        return xy_all[:base], ty_all[:base], gid_all[:base], got
+        return out
+
+
+def _halo(eng, xy, types, gid, strip: Strip, width: float, rank: int, world: int, ranges, peer):
+    """Generator: the owned points and the ghosts of each x-range, as merge_halo returns them. The halo of ``width``
+    travels through ``peer``'s slabs when it is given and there are peers, else through exchange_halo."""
+    if peer is not None and world > 1:
+        return peer.exchange(eng, xy, types, gid, strip, width, ranges)
+    all_recs, max_cnt = yield from exchange_halo(eng, xy, types, gid, strip, width, rank, world)
+    return merge_halo(eng, xy, types, gid, all_recs, max_cnt, rank, ranges)
 
 
 def sharded_radius_graph(eng, xy, types, gid, r: float, strip: Strip, rank: int, world: int, n_types: int = 5,
@@ -234,13 +239,8 @@ def sharded_radius_graph(eng, xy, types, gid, r: float, strip: Strip, rank: int,
     over the owned rows, plus ``row_gid`` (global id of each row) and ``n_ghost``."""
     from .engine import radius_cell
 
-    lo = -_INF if strip.is_first else strip.lo - r
-    hi = _INF if strip.is_last else strip.hi + r
-    if peer is not None and world > 1:
-        xy_all, ty_all, gid_all, got = peer.exchange(eng, xy, types, gid, strip, r, [(lo, hi)])
-    else:
-        all_recs, max_cnt = yield from exchange_halo(eng, xy, types, gid, strip, r, rank, world)
-        xy_all, ty_all, gid_all, got = merge_halo(eng, xy, types, gid, all_recs, max_cnt, rank, [(lo, hi)])
+    ranges = [(strip.x_lo - r, strip.x_hi + r)]
+    xy_all, ty_all, gid_all, got = yield from _halo(eng, xy, types, gid, strip, r, rank, world, ranges, peer)
     n_own = int(xy.shape[0])
     eng.grid_build(xy_all, ty_all, gid_all, radius_cell(r), bounds, n_query=n_own)
     g = eng.radius_graph(r, upper=upper, n_types=n_types, want_dist32=True, want_dist64=True, want_edges=upper)
@@ -254,8 +254,8 @@ def _strip_bounds(strip: Strip, width: float, bounds):
     if bounds is None:
         return None
     x0, y0, x1, y1 = (float(v) for v in bounds)
-    lo = x0 if strip.is_first else max(x0, strip.lo - width)
-    hi = x1 if strip.is_last else min(x1, strip.hi + width)
+    lo = max(x0, strip.x_lo - width)
+    hi = min(x1, strip.x_hi + width)
     return (lo, y0, max(hi, lo), y1)
 
 
@@ -277,16 +277,11 @@ def sharded_knn_graph(eng, xy, types, gid, k: int, strip: Strip, rank: int, worl
     h = float(h0)
     for _ in range(max_rounds):
         width = 2.0 * h if union else h
-        lo1 = -_INF if strip.is_first else strip.lo - h
-        hi1 = _INF if strip.is_last else strip.hi + h
+        lo1, hi1 = strip.x_lo - h, strip.x_hi + h
         ranges = [(lo1, hi1)]
         if union:
-            ranges += [(-_INF if strip.is_first else strip.lo - 2 * h, lo1), (hi1, _INF if strip.is_last else strip.hi + 2 * h)]
-        if peer is not None and world > 1:
-            xy_all, ty_all, gid_all, got = peer.exchange(eng, xy, types, gid, strip, width, ranges)
-        else:
-            all_recs, max_cnt = yield from exchange_halo(eng, xy, types, gid, strip, width, rank, world)
-            xy_all, ty_all, gid_all, got = merge_halo(eng, xy, types, gid, all_recs, max_cnt, rank, ranges)
+            ranges += [(strip.x_lo - 2 * h, lo1), (hi1, strip.x_hi + 2 * h)]
+        xy_all, ty_all, gid_all, got = yield from _halo(eng, xy, types, gid, strip, width, rank, world, ranges, peer)
         n_q = n_own + (got[0] if union else 0)
         n_all = int(xy_all.shape[0])
         kn = None
@@ -302,9 +297,7 @@ def sharded_knn_graph(eng, xy, types, gid, k: int, strip: Strip, rank: int, worl
                 ext = torch.stack([xy_all.amax(0) - xy_all.amin(0)]).reshape(-1).tolist()
                 area = max(ext[0], 1e-9) * max(ext[1], 1e-9)
             eng.grid_build(xy_all, ty_all, gid_all, default_knn_cell(n_all, area, k), box, n_query=n_q)
-            x_lo = -_INF if strip.is_first else strip.lo - width
-            x_hi = _INF if strip.is_last else strip.hi + width
-            kn = eng.knn(k, dist_dtype=torch.float64, x_lo=x_lo, x_hi=x_hi, check_halo=True)
+            kn = eng.knn(k, dist_dtype=torch.float64, x_lo=strip.x_lo - width, x_hi=strip.x_hi + width, check_halo=True)
             red[0] = kn["halo_ok"][0].to(torch.float64)
             if n_own:
                 red[1] = -kn["dist"][:n_own, k - 1].max()

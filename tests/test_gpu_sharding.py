@@ -299,3 +299,96 @@ def test_peer_slab_halo_equals_allgather_path(engine):
     engine.halo_unpack_slab(tiny[0], world, 0, 16, [(-inf, inf)], buf[0], buf[1], buf[2], 0)
     with pytest.raises(RuntimeError):
         engine.check_overflow()
+
+
+def _meta(recs):
+    """(gid, type) int32 columns of 24-byte halo records held as float64 [n, 3]."""
+    m = recs[:, 2].contiguous().view(torch.int32).reshape(-1, 2)
+    return m[:, 0], m[:, 1]
+
+
+def test_halo_pack_past_capacity(engine):
+    """pg_halo_pack with fewer slots than selected points: the count still counts every selected point, the overflow
+    is reported once, and the slots that were written hold distinct selected points, intact. A NaN x is never packed."""
+    dev = torch.device("cuda", 0)
+    xy, ty, side = synth.make_points(20_000, seed=55)
+    d_xy, d_ty = torch.from_numpy(xy).to(dev), torch.from_numpy(ty).to(dev)
+    d_xy[::97, 0] = float("nan")
+    gid = torch.arange(len(xy), dtype=torch.int32, device=dev) * 3 + 1
+    lo_edge, hi_edge = side * 0.1, side * 0.9
+    sel = (d_xy[:, 0] < lo_edge) | (d_xy[:, 0] >= hi_edge)
+    n_sel, cap = int(sel.sum()), 500
+    assert n_sel > 2 * cap
+    engine.check_overflow()
+    recs, count = engine.halo_pack(d_xy, d_ty, gid, lo_edge, hi_edge, capacity=cap)
+    assert int(count.item()) == n_sel
+    with pytest.raises(RuntimeError) as exc:
+        engine.check_overflow()
+    assert exc.value.code == -4
+    engine.check_overflow()
+    g, t = _meta(recs)
+    assert torch.unique(g).numel() == cap
+    row = ((g - 1) // 3).long()
+    assert torch.equal(g, gid[row]) and bool(sel[row].all())
+    assert torch.equal(recs[:, :2], d_xy[row]) and torch.equal(t, d_ty[row])
+    # without gid / type: the gid is the row index and the type 0
+    recs, count = engine.halo_pack(d_xy, None, None, lo_edge, hi_edge, capacity=n_sel)
+    engine.check_overflow()
+    g, t = _meta(recs)
+    assert torch.equal(torch.sort(g).values, torch.nonzero(sel).reshape(-1).to(torch.int32)) and not bool(t.any())
+
+
+_INF = float("inf")
+
+
+def _gathered(engine, n_recs, seed):
+    """Records of n_recs points (gid = row) in the layout of the all-gathered payload, every 13th a NaN padding row.
+    Returns (recs, xy, types, side)."""
+    dev = torch.device("cuda", 0)
+    xy, ty, side = synth.make_points(n_recs, seed=seed)
+    d_xy, d_ty = torch.from_numpy(xy).to(dev), torch.from_numpy(ty).to(dev)
+    recs, count = engine.halo_pack(d_xy, d_ty, None, _INF, -_INF, capacity=n_recs)
+    assert int(count.item()) == n_recs
+    recs[::13] = float("nan")
+    return recs, d_xy, d_ty, side
+
+
+def test_halo_unpack_multi_skip_window(engine):
+    """The records of [skip_begin, skip_end) (this rank's own) and NaN padding never land, in any range."""
+    dev = torch.device("cuda", 0)
+    n_recs, n_base, skip = 30_000, 1000, (9_000, 17_000)
+    recs, d_xy, d_ty, side = _gathered(engine, n_recs, 56)
+    ranges = [(side * 0.2, side * 0.6), (-_INF, side * 0.2), (side * 0.6, _INF)]
+    cap = n_base + n_recs
+    a = [torch.full((cap, 2), -1.0, dtype=torch.float64, device=dev), torch.full((cap,), -1, dtype=torch.int32, device=dev),
+         torch.full((cap,), -1, dtype=torch.int32, device=dev)]
+    engine.check_overflow()
+    got = engine.halo_unpack_multi(recs, n_recs, skip[0], skip[1], ranges, a[0], a[1], a[2], n_base).tolist()
+    engine.check_overflow()
+    g_all = _meta(recs)[0]
+    keep = ~torch.isnan(recs[:, 0])
+    keep[skip[0]:skip[1]] = False
+    assert sum(got) == int(keep.sum())
+    assert bool((a[2][:n_base] == -1).all()) and bool((a[2][n_base + sum(got):] == -1).all())
+    at = n_base
+    for (lo, hi), c in zip(ranges, got):
+        want = keep & (recs[:, 0] >= lo) & (recs[:, 0] < hi)
+        assert c == int(want.sum())
+        g = a[2][at:at + c]
+        assert torch.equal(torch.sort(g).values, torch.sort(g_all[want]).values)
+        assert torch.equal(a[0][at:at + c], d_xy[g.long()]) and torch.equal(a[1][at:at + c], d_ty[g.long()])
+        at += c
+
+
+def test_halo_unpack_multi_reports_a_small_destination(engine):
+    dev = torch.device("cuda", 0)
+    n_recs, n_base = 30_000, 100
+    recs, _, _, side = _gathered(engine, n_recs, 57)
+    cap = n_base + 1000
+    a = [torch.empty((cap, 2), dtype=torch.float64, device=dev), torch.empty(cap, dtype=torch.int32, device=dev),
+         torch.empty(cap, dtype=torch.int32, device=dev)]
+    engine.check_overflow()
+    engine.halo_unpack_multi(recs, n_recs, 0, 0, [(-_INF, side * 0.5), (side * 0.5, _INF)], a[0], a[1], a[2], n_base)
+    with pytest.raises(RuntimeError) as exc:
+        engine.check_overflow()
+    assert exc.value.code == -4
