@@ -298,6 +298,45 @@ int pg_clustering(pg_handle* h, int32_t n, const int32_t* row_ptr, const int32_t
 int pg_type_interactions(pg_handle* h, int32_t n, const int32_t* type, const int32_t* nbr_count,
                          int32_t n_types, int64_t* inter, pg_stream stream);
 
+/* ---- K15: neighbourhood enrichment (csrc/pg_enrich.cu): the type-interaction matrix of an undirected edge list
+ * against the same counts under random relabelling of the nodes - the label-permutation z-score of
+ * squidpy.gr.nhood_enrichment, which makes "cell-cell interaction patterns" (README.md:133) readable when one type
+ * dominates the slide.
+ *   edges int32 [n_edges][2] rows (i, j) (build_radius_graph / build_knn_graph's i<j list; any order works); a row
+ *         with an id outside [0, n) is skipped, as pg_clustering skips foreign ids. 4-byte alignment suffices.
+ *   type  int32 [n]; labels outside 1..n_types count nowhere (but are permuted like every other label).
+ * Counting: for a labelling t every edge row (i, j) adds 1 to c[t_i - 1][t_j - 1] and 1 to c[t_j - 1][t_i - 1] (the
+ *   directed entries of the symmetric adjacency, squidpy's counting); with the original types c equals
+ *   pg_type_interactions of the same graph's composition.
+ * Permutation p (0 <= p < n_perms): node i gets the label type[pi_p(i)], pi_p a keyed bijection of [0, n):
+ *   h = the least h >= 1 with 4^h >= n; a value x < 4^h is split into L = x >> h, R = x & (2^h - 1);
+ *   8 Feistel rounds r = 0..7: (L, R) <- (R, L ^ (splitmix64(R ^ k_{p,r}) & (2^h - 1))),
+ *     k_{p,r} = splitmix64(seed ^ (64 p + r));  x <- (L << h) | R;
+ *   cycle-walk: repeat the 8 rounds until x < n.  pi_p(i) = that x.
+ *   splitmix64(x) (uint64 arithmetic mod 2^64): z = x + 0x9E3779B97F4A7C15; z = (z ^ (z >> 30)) * 0xBF58476D1CE4E5B9;
+ *     z = (z ^ (z >> 27)) * 0x94D049BB133111EB; return z ^ (z >> 31).
+ *   For h >= 2 a Feistel network only reaches even permutations of its 4^h domain, so for a handful of nodes the
+ *   family is visibly not the whole symmetric group; the count statistics match uniform permutations from n ~ 20 on.
+ * Statistics, per (a, b), from S1 = sum_p c_p (int64) and S2 = sum_p c_p^2 (128-bit), exact integers each converted
+ *   to float64 once:  perm_mean = S1 / P;  perm_std = sqrt(P S2 - S1^2) / P (ddof 0);
+ *   zscore = (P count - S1) / sqrt(P S2 - S1^2) - NaN / +-inf where the permutation variance is 0 (IEEE division).
+ * n = 0 or n_edges = 0: zero counts, mean and std 0, NaN zscore.  Only integer atomics: the outputs do not depend on
+ * the run, the chunking or the handle.  Outputs [n_types][n_types], each pointer may be NULL.  Asynchronous; no host
+ * synchronisation beyond workspace growth (labels of at most PG_ENRICH_CHUNK_BYTES / n permutations at a time, and
+ * 8 (n_perms + 1) n_types^2 bytes of counts).  PG_ERR_INVALID for n < 0, n_edges < 0, n_types outside
+ * 1..PG_MAX_TYPES, n_perms outside 1..PG_ENRICH_MAX_PERMS. */
+#define PG_ENRICH_MAX_PERMS 100000
+#define PG_ENRICH_CHUNK_BYTES (64 << 20)
+typedef struct {
+  int64_t* count;     /* observed directed counts */
+  double* zscore;
+  double* perm_mean;
+  double* perm_std;
+} pg_enrich_out;
+int pg_nhood_enrichment(pg_handle* h, int32_t n, const int32_t* type, int32_t n_types, int64_t n_edges,
+                        const int32_t* edges, int32_t n_perms, uint64_t seed, const pg_enrich_out* out,
+                        pg_stream stream);
+
 /* ---- K12: raster region properties of an instance map (SURVEY 8f-3): what skimage regionprops gives
  * aggregated_hovernet_run.py:172-181 (bbox per instance) and hovernet_tile_inference.ipynb:2415-2429 (cell 18:
  * area, perimeter, eccentricity, major / minor axis length, orientation).  inst_map int32 [height][width], labels

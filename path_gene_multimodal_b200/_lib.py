@@ -16,6 +16,7 @@ PG_RADIUS_SYMMETRIC = 0
 PG_RADIUS_UPPER = 1
 PG_MAX_TYPES = 16
 PG_MAX_K = 64
+PG_ENRICH_MAX_PERMS = 100000
 
 PG_OK, PG_ERR_INVALID, PG_ERR_CUDA, PG_ERR_STATE, PG_ERR_CAPACITY, PG_ERR_NOMEM = 0, -1, -2, -3, -4, -5
 
@@ -48,6 +49,10 @@ class PgRasterOut(C.Structure):
 
 class PgHullOut(C.Structure):
     _fields_ = [(name, vp) for name in ("convex_area", "solidity", "orientation")]
+
+
+class PgEnrichOut(C.Structure):
+    _fields_ = [(name, vp) for name in ("count", "zscore", "perm_mean", "perm_std")]
 
 
 class PathGraphError(RuntimeError):
@@ -102,6 +107,7 @@ SIGNATURES = {
     "pg_narrow_counts": (C.c_int, [vp, vp, i64, vp, i32, vp]),
     "pg_clustering": (C.c_int, [vp, i32, vp, vp, vp, vp, vp]),
     "pg_type_interactions": (C.c_int, [vp, i32, vp, vp, i32, vp, vp]),
+    "pg_nhood_enrichment": (C.c_int, [vp, i32, vp, i32, i64, vp, i32, C.c_uint64, C.POINTER(PgEnrichOut), vp]),
     "pg_raster_props": (C.c_int, [vp, i32, i32, vp, i32, C.POINTER(PgRasterOut), vp]),
     "pg_raster_solidity": (C.c_int, [vp, i32, i32, vp, i32, vp, vp, vp, vp, vp]),
     "pg_ring_hull_f32": (C.c_int, [vp, i32, i64, vp, vp, C.POINTER(PgHullOut), vp]),

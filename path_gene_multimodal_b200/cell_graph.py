@@ -267,6 +267,40 @@ def type_interaction_matrix(types, nbr_count, n_types: int = 5, device=None) -> 
         return _host.to_host(eng.type_interactions(d_t, d_c, n_types))
 
 
+def neighbourhood_enrichment(edges, types, n_types: int = 5, n_perms: int = 1000, seed: int = 0, device=None) -> dict:
+    """Neighbourhood enrichment of an undirected graph (squidpy.gr.nhood_enrichment's statistic): how much more
+    often type a+1 neighbours type b+1 than under random relabelling of the nodes.
+
+    ``edges`` int32 / int64 [E,2] rows (i, j), as ``build_radius_graph`` / ``build_knn_graph`` return them; ``types``
+    int [N] (values outside 1..n_types count nowhere).  Every edge row adds one entry (a, b) and one (b, a), so
+    ``count`` equals ``type_interaction_matrix`` of the same graph.  ``n_perms`` labellings permute ``types`` by keyed
+    bijections of [0, N) derived from ``seed`` (the exact construction is in include/pathgraph.h, K15); the same
+    seed gives the same result bit for bit.  Returns [T,T] arrays ``count`` int64, ``perm_mean`` / ``perm_std``
+    float64 (mean and ddof-0 std of the permuted counts) and ``zscore`` = (count - perm_mean) / perm_std, NaN or
+    +-inf where the permuted counts never vary.  Raises ``ValueError`` on a bad edge shape or an id outside
+    [0, N), before anything is launched."""
+    t = _host.as_int32(types, "types").reshape(-1)
+    n = t.shape[0]
+    e = np.asarray(edges)
+    if e.size == 0 and e.ndim < 2:
+        e = e.reshape(0, 2)
+    if e.ndim != 2 or e.shape[1] != 2:
+        raise ValueError("edges must have shape (E, 2)")
+    if e.size and e.dtype.kind not in "iu":
+        raise ValueError(f"edges must be integer ids, got dtype {e.dtype}")
+    if e.size and (e.min() < 0 or e.max() >= n):
+        raise ValueError(f"edge ids must lie in [0, {n})")
+    if not 1 <= n_types <= _lib.PG_MAX_TYPES:
+        raise ValueError(f"n_types must be in 1..{_lib.PG_MAX_TYPES}")
+    if not 1 <= n_perms <= _lib.PG_ENRICH_MAX_PERMS:
+        raise ValueError(f"n_perms must be in 1..{_lib.PG_ENRICH_MAX_PERMS}")
+    eng = get_engine(device)
+    with torch.cuda.device(eng.device):
+        d_e = _host.to_device(e, np.int32, eng.device)  # ids < N <= 2^31 - 1 fit int32
+        d_t = _host.to_device(t, np.int32, eng.device)
+        return _host.to_host_many(eng.nhood_enrichment(d_e, d_t, n_types, n_perms, seed))
+
+
 def knn_graph_frame(final_df, k: int = 5, centroid_col: str = "centroid", centroid_order: str = "yx",
                     type_col: str | None = None, device=None):
     """Cell 11 at DataFrame level (ipynb:1766-1951): returns ``(df, graph)``.

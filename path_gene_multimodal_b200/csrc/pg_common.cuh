@@ -79,6 +79,8 @@ struct pg_handle {
   double morph_mean_verts = 0;  // pg_map_morph_hint: expected vertices per ring (sizes K1's shared-memory slabs)
   pg_buf hull;         // K14 (pg_hull.cu): chain buffers of the rings that do not fit a warp's slab
   size_t hull_smem_set[2] = {0, 0};  // K14: dynamic shared memory opted in on this handle's device, per T
+  pg_buf enrich_lab;   // K15 (pg_enrich.cu): uint8 labels of one chunk of permutations, [rows][n]
+  pg_buf enrich_cnt;   // K15: int64 ordered type-pair counts per labelling, [P + 1][T * T]
   // launch accounting / optional per-kernel CUDA-event timing (pg_profile_*)
   int64_t launches = 0;
   bool profiling = false;

@@ -124,7 +124,8 @@ int pg_destroy(pg_handle* h) {
   cudaSetDevice(h->device);
   cudaDeviceSynchronize();
   pg_buf* bufs[] = {&h->cell_count, &h->cell_start, &h->cell_of, &h->rank,      &h->s_rec,     &h->s_pos,     &h->s_gid,     &h->knn_retry,     &h->pt_meta,   &h->tmp_ent,   &h->row_off,
-                    &h->row_count,  &h->scan_state, &h->misc,    &h->sym_extra, &h->sym_cursor, &h->sym_recip, &h->hull};
+                    &h->row_count,  &h->scan_state, &h->misc,    &h->sym_extra, &h->sym_cursor, &h->sym_recip, &h->hull,
+                    &h->enrich_lab, &h->enrich_cnt};
   for (pg_buf* b : bufs)
     if (b->p) cudaFree(b->p);
   if (h->pinned) cudaFreeHost(h->pinned);
@@ -138,7 +139,8 @@ const char* pg_last_error(pg_handle* h) { return h ? h->err.c_str() : g_create_e
 int64_t pg_workspace_bytes(pg_handle* h) {
   if (!h) return 0;
   pg_buf* bufs[] = {&h->cell_count, &h->cell_start, &h->cell_of, &h->rank,      &h->s_rec,     &h->s_pos,     &h->s_gid,     &h->knn_retry,     &h->pt_meta,   &h->tmp_ent,   &h->row_off,
-                    &h->row_count,  &h->scan_state, &h->misc,    &h->sym_extra, &h->sym_cursor, &h->sym_recip, &h->hull};
+                    &h->row_count,  &h->scan_state, &h->misc,    &h->sym_extra, &h->sym_cursor, &h->sym_recip, &h->hull,
+                    &h->enrich_lab, &h->enrich_cnt};
   int64_t t = 0;
   for (pg_buf* b : bufs) t += (int64_t)b->cap;
   return t;

@@ -554,6 +554,32 @@ class Engine:
                                                   self._p(inter, torch.int64, "inter"), self._stream()))
         return inter
 
+    # ---- K15 -----------------------------------------------------------------------------------
+    def nhood_enrichment(self, edges, types, n_types=5, n_perms=1000, seed=0):
+        """Label-permutation enrichment of the type-interaction matrix (pg_nhood_enrichment).
+
+        edges int32 [E,2] (e.g. ``radius_graph(..., want_edges32=True)["edges32"][:E]``; rows with an id outside
+        [0, N) are skipped); types int32 [N].  Returns a dict of device tensors [T,T]: count int64, zscore, perm_mean,
+        perm_std float64.  Asynchronous (no host synchronisation once the workspace has grown)."""
+        n = int(types.numel())
+        if edges.dim() != 2 or edges.shape[1] != 2:
+            raise ValueError("edges must have shape (E, 2)")
+        seed = int(seed)
+        if not 0 <= seed < 2 ** 64:
+            raise ValueError("seed must be in [0, 2**64)")
+        t = int(n_types)
+        res = {"count": self._empty((t, t), torch.int64)}
+        for name in ("zscore", "perm_mean", "perm_std"):
+            res[name] = self._empty((t, t), torch.float64)
+        eo = _lib.PgEnrichOut()
+        eo.count = self._p(res["count"], torch.int64, "count")
+        for name in ("zscore", "perm_mean", "perm_std"):
+            setattr(eo, name, self._p(res[name], torch.float64, name))
+        self._check(self.lib.pg_nhood_enrichment(self._h, n, self._p(types, torch.int32, "types"), t, int(edges.shape[0]),
+                                                 self._p(edges, torch.int32, "edges"), int(n_perms), seed,
+                                                 C.byref(eo), self._stream()))
+        return res
+
     # ---- K10 -----------------------------------------------------------------------------------
     def node_features(self, feat, types=None, onehot_values=None):
         """z-scored feature columns + type one-hot -> x float32 [N, n_onehot + n_feat] (pg_node_features).
