@@ -116,7 +116,8 @@ int pg_grid_build(pg_handle* h, int32_t n, int32_t n_query, const double* xy, co
 /* Coordinates must be finite (cKDTree raises on NaN / inf). With bounds = NULL pg_grid_build itself reports it;
  * with caller-given bounds the build is asynchronous, the histogram kernel flags the offending input and
  * PG_ERR_INVALID comes from the next call that synchronises: pg_grid_check (synchronises the stream),
- * pg_radius_total or pg_check_overflow. */
+ * pg_radius_total or pg_check_overflow. A span that overflows double (xmax - xmin or ymax - ymin = inf for finite
+ * points or bounds, e.g. -1e308 .. 1e308) is PG_ERR_INVALID from pg_grid_build itself. */
 int pg_grid_check(pg_handle* h);
 /* The points of the built grid in CELL ORDER (a spatial sort of the input, one coalesced pass over the records):
  * xy f64 [n,2], type int32 [n], gid int32 [n] = the id of each point (gid given to pg_grid_build, else its row);

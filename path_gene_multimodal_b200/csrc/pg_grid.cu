@@ -216,12 +216,19 @@ int pg_grid_build(pg_handle* h, int32_t n, int32_t n_query, const double* xy, co
       return pg_set_error(h, PG_ERR_INVALID, "pg_grid_build: coordinates must be finite");
   }
 
+  // finite points can still span more than a double holds (-1e308 .. 1e308): no cell size bins that
+  PG_REQUIRE(h, std::isfinite(b[2] - b[0]) && std::isfinite(b[3] - b[1]),
+             "pg_grid_build: the coordinate span (%g x %g) overflows double", b[2] - b[0], b[3] - b[1]);
+
   // cell count is capped; a larger-than-asked cell only makes queries visit more cells (they
   // derive their ring radius from the actual cell size), never changes results.
   const double max_cells = std::min((double)(1 << 28), std::max(8.0 * (double)n, (double)(1 << 20)));
   double cell = cell_size;
   int64_t nx, ny, nys;
   while (true) {
+    // backstop: after the span check above a finite span fits one cell long before the cell overflows, so this never
+    // fires today; it keeps the loop from spinning should that check ever change
+    PG_REQUIRE(h, std::isfinite(cell), "pg_grid_build: no finite cell size bins the span (%g x %g)", b[2] - b[0], b[3] - b[1]);
     const double fx = std::floor((b[2] - b[0]) / cell) + 1, fy = std::floor((b[3] - b[1]) / cell) + 1;
     const double fys = std::ceil(fy / PG_STRIP);
     // rows are padded to whole strips: the padded count may reach 4 x the cap for thin grids (< 2^30 either way)

@@ -342,7 +342,8 @@ extern "C" int pg_knn(pg_handle* h, int32_t k, int32_t* knn_idx, double* dist64,
   const pg_grid& gr = h->grid;
   PG_REQUIRE(h, k >= 1 && k <= PG_MAX_K, "pg_knn: k must be in 1..%d (got %d)", PG_MAX_K, k);
   PG_REQUIRE(h, k < gr.n, "pg_knn: k (%d) must be smaller than the number of points (%d)", k, gr.n);
-  PG_REQUIRE(h, knn_idx != nullptr, "pg_knn: knn_idx is NULL");
+  // no query rows (a strip that holds only halo points): the [0, k] outputs may be empty allocations
+  PG_REQUIRE(h, knn_idx != nullptr || gr.n_query == 0, "pg_knn: knn_idx is NULL");
   int32_t* retry_count = (int32_t*)((char*)h->misc.p + PG_MISC_KNN_RETRY);
   PG_LAUNCH(h, s, "knn_prepare_kernel", knn_prepare_kernel<<<1, 1, 0, s>>>(halo_ok, retry_count));
   PG_LAUNCH_CHECK(h);
