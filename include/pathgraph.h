@@ -338,6 +338,23 @@ int pg_nhood_enrichment(pg_handle* h, int32_t n, const int32_t* type, int32_t n_
                         const int32_t* edges, int32_t n_perms, uint64_t seed, const pg_enrich_out* out,
                         pg_stream stream);
 
+/* ---- K16: type-pair distance histogram over the built grid (csrc/pg_pairhist.cu): the counts behind
+ * squidpy.gr.co_occurrence and Ripley's K / L - "cell-cell interaction patterns" (README.md:133) read across distance.
+ *   thresholds host f64 [n_thr], finite, >= 0, strictly ascending; 1 <= n_thr <= PG_PAIRHIST_MAX_THR (64)
+ *   hist  int64 [n_thr][n_types][n_types]: hist[b][a-1][c-1] = ordered pairs (i, j), i a query row (< n_query),
+ *         j any grid point, id_i != id_j, type_i = a, type_j = c, with
+ *           b = 0:  d2 <= t_0^2;   b >= 1:  t_{b-1}^2 < d2 <= t_b^2   (pairs past t_{n_thr-1} count nowhere)
+ *         d2 = __dadd_rn(__dmul_rn(dx,dx), __dmul_rn(dy,dy)), t_b^2 rounded once in float64 (the radius rule).
+ *   type_count int64 [n_types] (may be NULL): query rows of each type.
+ * Types outside 1..n_types count nowhere. Integer counts only, so the result does not depend on the run.
+ * The walk covers the ball of t_{n_thr-1} on whatever cell the grid was built with (a grid built for a small radius
+ * works at a large one, only slower); work is n_query x the points of the (2R+1)^2 block, R = t_max / cell rounded up.
+ * With ids (gid) and n_query set for a strip + halo of t_max, the strips' histograms sum to the whole slide's.
+ * Asynchronous, no host synchronisation. hist / type_count 8-byte aligned. */
+#define PG_PAIRHIST_MAX_THR 64
+int pg_pair_dist_hist(pg_handle* h, int32_t n_types, int32_t n_thr, const double* thresholds,
+                      int64_t* hist, int64_t* type_count, pg_stream stream);
+
 /* ---- K12: raster region properties of an instance map (SURVEY 8f-3): what skimage regionprops gives
  * aggregated_hovernet_run.py:172-181 (bbox per instance) and hovernet_tile_inference.ipynb:2415-2429 (cell 18:
  * area, perimeter, eccentricity, major / minor axis length, orientation).  inst_map int32 [height][width], labels

@@ -6,7 +6,8 @@ Mirrors /root/reference/hovernet_tile_inference.ipynb:
 * ``build_radius_graph``   cells 23-26 (ipynb:2963-3042): ``edges`` int64 [E,2] (``i<j``), ``edge_index``,
   ``edge_attr`` float32 [2E,1];
 * ``filter_graph_by_type`` cell 12 (ipynb:1989-2002);
-* ``neighbour_type_composition`` / ``degree_stats``: named in README.md:127,136 only; defined in SURVEY A.5.
+* ``neighbour_type_composition`` / ``degree_stats``: named in README.md:127,136 only; defined in SURVEY A.5;
+* ``co_occurrence`` / ``ripley``: cell-type patterns across distance (squidpy.gr.co_occurrence / ripley's statistics).
 
 Host arrays in, host arrays out; everything in between is libpathgraph (uniform-grid binning, grid
 queries, two-pass CSR) on the GPU.  No CPU fallback.
@@ -17,7 +18,7 @@ import numpy as np
 import torch
 
 from . import _host, _lib
-from .engine import default_knn_cell, get_engine, radius_cell
+from .engine import default_knn_cell, get_engine, pair_hist_cell, radius_cell
 
 TYPE_NAMES = {1: "neoplastic", 2: "inflammatory", 3: "connective", 4: "dead", 5: "epithelial"}       # ipynb:1774-1780
 CLASS_COLORS = {1: "tab:red", 2: "tab:green", 3: "tab:blue", 4: "tab:gray", 5: "tab:orange"}           # ipynb:1782-1788
@@ -299,6 +300,125 @@ def neighbourhood_enrichment(edges, types, n_types: int = 5, n_perms: int = 1000
         d_e = _host.to_device(e, np.int32, eng.device)  # ids < N <= 2^31 - 1 fit int32
         d_t = _host.to_device(t, np.int32, eng.device)
         return _host.to_host_many(eng.nhood_enrichment(d_e, d_t, n_types, n_perms, seed))
+
+
+def _distances(values, name: str, min_len: int) -> np.ndarray:
+    """Host thresholds for K16: 1-D float64, finite, >= 0, strictly ascending, min_len..PG_PAIRHIST_MAX_THR entries."""
+    t = np.asarray(values, dtype=np.float64)
+    if t.ndim != 1 or not min_len <= t.shape[0] <= _lib.PG_PAIRHIST_MAX_THR:
+        raise ValueError(f"{name} must be a 1-D array of {min_len}..{_lib.PG_PAIRHIST_MAX_THR} distances")
+    if not np.isfinite(t).all() or (t < 0).any():
+        raise ValueError(f"{name} must be finite and >= 0")
+    if (np.diff(t) <= 0).any():
+        raise ValueError(f"{name} must be strictly ascending")
+    return t
+
+
+def _pair_hist(coords, types, thresholds, n_types: int, device) -> tuple:
+    """Validated host input -> K16 over a grid built for thresholds[-1]: (hist int64 [B,T,T], type_count int64 [T],
+    coords, the engine, the device coordinates)."""
+    c = np.asarray(coords, dtype=np.float64)
+    if c.ndim != 2 or c.shape[1] != 2:
+        raise ValueError("coords must have shape (N, 2)")
+    if c.shape[0] > _host.INT32_MAX:
+        raise OverflowError("more than 2^31 points")
+    if not np.isfinite(c).all():
+        raise ValueError("coords must be finite")
+    t = _host.as_int32(types, "types").reshape(-1)
+    if t.shape[0] != c.shape[0]:
+        raise ValueError("types must have one entry per point")
+    if not 1 <= n_types <= _lib.PG_MAX_TYPES:
+        raise ValueError(f"n_types must be in 1..{_lib.PG_MAX_TYPES}")
+    eng = get_engine(device)
+    with torch.cuda.device(eng.device):
+        d_xy = _host.to_device(c, np.float64, eng.device)
+        d_t = _host.to_device(t, np.int32, eng.device)
+        b = _bounds(c)
+        area = max(b[2] - b[0], 1e-9) * max(b[3] - b[1], 1e-9)
+        eng.grid_build(d_xy, d_t, None, pair_hist_cell(float(thresholds[-1]), c.shape[0], area), b)
+        res = _host.to_host_many(eng.pair_dist_hist(thresholds, n_types))
+    return res["hist"], res["type_count"], c, eng, d_xy
+
+
+def co_occurrence(coords, types, interval, n_types: int = 5, max_dist: float | None = None, cumulative: bool = False,
+                  device=None) -> dict:
+    """Co-occurrence of cell types across distance (the statistic squidpy.gr.co_occurrence documents): for each
+    distance interval, how much more likely a cell of type c+1 is near a cell of type a+1 than anywhere.
+
+    ``interval``: ascending distances t_0 < ... < t_B (2..64 of them, finite, >= 0), or an int together with
+    ``max_dist`` for ``np.linspace(0, max_dist, interval)``.  Interval b is the annulus t_b < d <= t_{b+1}, or the disc
+    d <= t_{b+1} with ``cumulative``.  There is no whole-slide default: squidpy's (up to half the slide's extent) makes
+    every pair of the slide a candidate, which is quadratic in N; pick the distances that matter (tens to hundreds of
+    micrometres) and the work is N x the cells within t_B.
+    ``types`` int [N]; values outside 1..n_types count nowhere.  Pairs are ordered pairs (i, j) of distinct points (a
+    duplicate point is a neighbour at distance 0), with squared distances compared exactly as ``build_radius_graph``
+    does.  Returns ``interval`` float64 [B+1], ``count`` int64 [T,T,B] (squidpy's layout: count[a, c, b] = pairs with
+    i of type a+1, j of type c+1 in interval b), ``occ`` float64 [T,T,B] = count * S / (R_a R_c) per interval, R = the
+    row sums and S = the total of that interval's counts - p(c | a) / p(c), NaN where R_a or R_c is 0 - and
+    ``type_count`` int64 [T].  This follows squidpy's documented definition, not its code: its versions differ on
+    whether an interval is an annulus or a disc.  Raises ``ValueError`` on bad shapes, non-finite coordinates or
+    distances, distances that are negative or not strictly ascending, more than 64 of them, or ``n_types`` outside
+    1..16, before anything is launched."""
+    if isinstance(interval, (int, np.integer)):
+        if max_dist is None or not (np.isfinite(max_dist) and max_dist > 0):
+            raise ValueError("an int interval needs a finite max_dist > 0")
+        thr = _distances(np.linspace(0.0, float(max_dist), int(interval)), "interval", 2)
+    else:
+        if max_dist is not None:
+            raise ValueError("max_dist only goes with an int interval")
+        thr = _distances(interval, "interval", 2)
+    hist, type_count, *_ = _pair_hist(coords, types, thr, n_types, device)
+    cnt = np.cumsum(hist, axis=0)[1:] if cumulative else hist[1:]
+    count = np.ascontiguousarray(np.moveaxis(cnt, 0, -1))
+    return {"interval": thr, "count": count, "occ": occurrence_ratio(count), "type_count": type_count}
+
+
+def occurrence_ratio(count) -> np.ndarray:
+    """occ[a, c, b] = count[a, c, b] * S_b / (R_ab R_cb) in float64, R = row sums, S = total of interval b; NaN where a
+    row sum is 0 (co_occurrence's ``occ`` from its ``count``)."""
+    cnt = np.asarray(count, dtype=np.int64)
+    row = cnt.sum(axis=1).astype(np.float64)                  # [T, B]
+    tot = cnt.sum(axis=(0, 1)).astype(np.float64)             # [B]
+    den = row[:, None, :] * row[None, :, :]
+    with np.errstate(divide="ignore", invalid="ignore"):
+        occ = cnt.astype(np.float64) * tot / den
+    occ[den == 0] = np.nan
+    return occ
+
+
+def ripley(coords, radii, types=None, n_types: int = 5, area: float | None = None, device=None) -> dict:
+    """Ripley's K and L functions at ``radii`` (ascending, 1..64 distances, finite, >= 0), without edge correction.
+
+    K_ac(r) = A C_ac(r) / (n_a n_c) and, on the diagonal, A C_aa(r) / (n_a (n_a - 1)), where C_ac(r) counts ordered
+    pairs of distinct points of types a+1 and c+1 at distance <= r (the squared-distance rule of ``build_radius_graph``)
+    and n_a the points of type a+1; L = sqrt(K / pi).  ``types=None`` gives the univariate K over all points (``K`` and
+    ``L`` of shape [len(radii)]); otherwise they are [T,T,len(radii)] (NaN where a count of points is too small).
+    ``area`` defaults to the area of the points' convex hull, as squidpy.gr.ripley uses, computed on the GPU by the
+    polygon hull kernel (K14) over one ring of all N points.  Returns ``radii``, ``K``, ``L``, ``area``, ``n`` (points
+    per type) and ``count`` (C, int64, same layout as ``K``).  Raises ``ValueError`` on the inputs ``co_occurrence``
+    rejects and on an ``area`` that is not finite and > 0."""
+    r = _distances(radii, "radii", 1)
+    univariate = types is None
+    c = np.asarray(coords, dtype=np.float64)
+    if univariate:
+        n_types = 1
+        types = np.ones(c.shape[0] if c.ndim == 2 else 0, dtype=np.int32)
+    if area is not None and not (np.isfinite(area) and area > 0):
+        raise ValueError("area must be finite and > 0")
+    hist, n_t, c, eng, d_xy = _pair_hist(c, types, r, n_types, device)
+    if area is None:
+        with torch.cuda.device(eng.device):
+            off = _host.to_device(np.array([0, c.shape[0]], dtype=np.int32), np.int32, eng.device)
+            area = float(_host.to_host(eng.ring_hull(off, d_xy)["convex_area"])[0])
+    count = np.ascontiguousarray(np.moveaxis(np.cumsum(hist, axis=0), 0, -1))   # [T, T, len(radii)]
+    den = n_t[:, None] * n_t[None, :] - np.diag(n_t)                              # n_a n_c, n_a (n_a - 1)
+    with np.errstate(divide="ignore", invalid="ignore"):
+        k = float(area) * count.astype(np.float64) / den[:, :, None].astype(np.float64)
+    k[np.broadcast_to(den[:, :, None] <= 0, k.shape)] = np.nan
+    lf = np.sqrt(k / np.pi)
+    if univariate:
+        k, lf, count = k[0, 0], lf[0, 0], count[0, 0]
+    return {"radii": r, "K": k, "L": lf, "area": float(area), "n": n_t, "count": count}
 
 
 def knn_graph_frame(final_df, k: int = 5, centroid_col: str = "centroid", centroid_order: str = "yx",

@@ -118,6 +118,7 @@ struct pg_kernel_scope {
 #define PG_MISC_TOTALS 128    // int32 x 8 totals copied to pinned memory: [0] radius [1] union [2] upper [3] contour scans; [4..5] uint64 overflow-region entries the last count pass needed
 #define PG_MISC_TMPCUR 192    // uint64 allocation cursor of tmp_ent's overflow region (zero between count passes: the row pass moves it to TOTALS[4..5])
 #define PG_MISC_SUM64 200     // int64: 64-bit total of the last pg_scan_i32_total (copied to pinned[12..13])
+#define PG_MISC_PAIRHIST_TICKET 208  // uint64: point cursor of pair_hist_kernel's CTAs (zeroed before each launch)
 #define PG_MISC_FEAT_TICKET 4608  // uint32 [PG_FEAT_MAX_COLS] CTA tickets of feature_stats_kernel, one per column (zero between launches)
 #define PG_FEAT_MAX_COLS 256
 #define PG_MISC_ACC 256       // pg_stats_acc: degree-statistics accumulators kept in their reset state

@@ -1,5 +1,8 @@
 // Shared device-side pieces of the grid queries (K5 kNN, K6 radius).
 #pragma once
+#include <algorithm>
+#include <cfloat>
+#include <cmath>
 #include "pg_common.cuh"
 
 // One point of the cell-ordered array = one 32-byte DRAM sector: the counting-sort scatter writes it
@@ -31,6 +34,22 @@ static inline pg_grid_view pg_make_view(const pg_handle* h) {
   v.n = h->grid.n; v.n_query = h->grid.n_query; v.nx = h->grid.nx; v.ny = h->grid.ny; v.nys = h->grid.nys;
   v.x0 = h->grid.x0; v.y0 = h->grid.y0; v.cell = h->grid.cell; v.inv_cell = h->grid.inv_cell;
   return v;
+}
+
+// Block radius of a query of radius r over the grid gr (K6's radius walk, K16's pair histogram).
+static inline int pg_ring_radius(double r, const pg_grid& gr) {
+  // every point within r lies at most R cells away along each axis. The binning t = fl(fl(v - x0) * inv_cell) rounds
+  // twice (each within t eps / 2), so two points r apart can land r * inv_cell + 2 t eps apart; the t that matters is
+  // below max(nx, ny) + R + 1 (a pair clamped on the same side shares its border cell), so 4 max(nx, ny) eps covers it
+  // with room to spare. A fixed slack does not cover it: at t just below 2^26, r = 13/64 and cell = r (1 + 3e-9),
+  // two points exactly r apart bin two rows apart. radius_cell's 2^-20 margin keeps R = 1 up to the 2^28-cell cap.
+  // Capped in double before the conversion: a block of radius max(nx, ny) already covers the grid, and a ball far
+  // larger than the grid (r / cell past INT_MAX, or cx + R past INT_MAX in the block walk) would not convert or add
+  // safely.
+  const double cover = (double)std::max(gr.nx, gr.ny);
+  const double R = std::ceil(r * gr.inv_cell * (1.0 + 1e-9) + 1e-9 + 4.0 * cover * DBL_EPSILON);
+  if (!(R < cover)) return std::max((int)cover, 1);
+  return R < 1.0 ? 1 : (int)R;
 }
 
 #ifdef __CUDACC__

@@ -562,21 +562,6 @@ radius_gather_kernel(int n_query, const int32_t* row_ptr, const int32_t* row_off
   gather_rows32(rp, end, off, id, (lane == 31 ? end : rp_next) - rp, tmp, o, capacity, overflow);
 }
 
-static inline int ring_radius(double r, const pg_grid& gr) {
-  // every point within r lies at most R cells away along each axis. The binning t = fl(fl(v - x0) * inv_cell) rounds
-  // twice (each within t eps / 2), so two points r apart can land r * inv_cell + 2 t eps apart; the t that matters is
-  // below max(nx, ny) + R + 1 (a pair clamped on the same side shares its border cell), so 4 max(nx, ny) eps covers it
-  // with room to spare. A fixed slack does not cover it: at t just below 2^26, r = 13/64 and cell = r (1 + 3e-9),
-  // two points exactly r apart bin two rows apart. radius_cell's 2^-20 margin keeps R = 1 up to the 2^28-cell cap.
-  // Capped in double before the conversion: a block of radius max(nx, ny) already covers the grid, and a ball far
-  // larger than the grid (r / cell past INT_MAX, or cx + R past INT_MAX in the block walk) would not convert or add
-  // safely.
-  const double cover = (double)std::max(gr.nx, gr.ny);
-  const double R = std::ceil(r * gr.inv_cell * (1.0 + 1e-9) + 1e-9 + 4.0 * cover * DBL_EPSILON);
-  if (!(R < cover)) return std::max((int)cover, 1);
-  return R < 1.0 ? 1 : (int)R;
-}
-
 // sizes tmp_ent for the pass described by h->last_count: one region per walk CTA + the overflow region
 int size_tmp(pg_handle* h) {
   const pg_grid& gr = h->grid;
@@ -611,7 +596,7 @@ int launch_count_pass(pg_handle* h, cudaStream_t s) {
     return PG_OK;
   }
   pg_grid_view v = pg_make_view(h);
-  const int R = ring_radius(a.r, gr);
+  const int R = pg_ring_radius(a.r, gr);
   const bool upper = a.flags == PG_RADIUS_UPPER;
   const bool wide = a.nbr_count && a.n_types > PG_PACKED_TYPES;
   walk_out w;

@@ -31,6 +31,13 @@ def radius_cell(r: float) -> float:
     return r * (1.0 + 2.0 ** -20) if r > 0 else 1.0
 
 
+def pair_hist_cell(t_max: float, n: int, area: float) -> float:
+    """Cell size for the pair histogram (K16): t_max / 4, so the 9x9 block is 1.6x the ball's area instead of the 3x3
+    block's 2.9x, but no smaller than one point per cell on average (smaller cells only add runs to the walk)."""
+    floor = math.sqrt(area / n) if n > 0 and area > 0 else 0.0
+    return max(t_max / 4.0, floor, 1e-12)
+
+
 class Engine:
     """One libpathgraph handle (= one workspace) on one CUDA device. Not thread-safe."""
 
@@ -578,6 +585,22 @@ class Engine:
         self._check(self.lib.pg_nhood_enrichment(self._h, n, self._p(types, torch.int32, "types"), t, int(edges.shape[0]),
                                                  self._p(edges, torch.int32, "edges"), int(n_perms), seed,
                                                  C.byref(eo), self._stream()))
+        return res
+
+    # ---- K16 -----------------------------------------------------------------------------------
+    def pair_dist_hist(self, thresholds, n_types=5):
+        """Type-pair distance histogram over the built grid (pg_pair_dist_hist).
+
+        ``thresholds``: ascending distances t_0 < ... < t_{B-1} (host, at most ``PG_PAIRHIST_MAX_THR``).  Returns a dict
+        of int64 device tensors: ``hist`` [B,T,T], hist[b, a-1, c-1] = ordered pairs (query row i of type a, grid point j
+        of type c, i != j) with t_{b-1} < d <= t_b (b = 0: d <= t_0), and ``type_count`` [T] (query rows per type).
+        Asynchronous (no host synchronisation once the workspace has grown)."""
+        t = np.asarray(thresholds, dtype=np.float64).reshape(-1)
+        nt, k = int(n_types), int(t.shape[0])
+        res = {"hist": self._empty((k, nt, nt), torch.int64), "type_count": self._empty((nt,), torch.int64)}
+        thr = (C.c_double * max(k, 1))(*t.tolist())
+        self._check(self.lib.pg_pair_dist_hist(self._h, nt, k, thr, self._p(res["hist"], torch.int64, "hist"),
+                                               self._p(res["type_count"], torch.int64, "type_count"), self._stream()))
         return res
 
     # ---- K10 -----------------------------------------------------------------------------------
