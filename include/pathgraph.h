@@ -355,6 +355,51 @@ int pg_nhood_enrichment(pg_handle* h, int32_t n, const int32_t* type, int32_t n_
 int pg_pair_dist_hist(pg_handle* h, int32_t n_types, int32_t n_thr, const double* thresholds,
                       int64_t* hist, int64_t* type_count, pg_stream stream);
 
+/* ---- K17: spatial autocorrelation of per-nucleus features over a cell graph (csrc/pg_autocorr.cu): Moran's I or
+ * Geary's C of every feature column with permutation statistics - squidpy.gr.spatial_autocorr's statistic - which asks
+ * whether a measurement (area, eccentricity, neighbour composition...) is spatially clustered on the slide.
+ *   row_ptr int32 [n+1], col int32 [row_ptr[n]]: a symmetric CSR without duplicate entries (build_radius_graph's
+ *           symmetric_csr / build_knn_graph's union); entries with col outside [0, n) are skipped, as pg_clustering
+ *           skips them, and do not count in any degree.
+ *   feat    float64 [n_feat][n] (K10's layout), 1 <= n_feat <= PG_AUTOCORR_MAX_FEAT.
+ * Weights: d_i = the in-range entries of row i; w_ij = 1 per entry (binary) or 1 / d_i (PG_AUTOCORR_ROW_STD).
+ *   S0 = sum w_ij, S1 = 1/2 sum (w_ij + w_ji)^2, S2 = sum_i (w_i. + w_.i)^2. Binary: S0 = sum d_i, S1 = 2 S0,
+ *   S2 = 4 sum d_i^2, exact int64 sums each converted to float64 once. Row-standardised: S0 = the non-isolated nodes,
+ *   S1 = 1/2 sum over entries (1/d_i + 1/d_j)^2, S2 = sum over non-isolated i of (1 + sum_{j in N(i)} 1/d_j)^2, float64.
+ * Statistic of a column x: z = x - mean(x) over all n nodes, m2 = sum z_i^2;
+ *   Moran  I = n sum_ij w_ij z_i z_j / (S0 m2);   Geary  C = (n - 1) sum_ij w_ij (z_i - z_j)^2 / (2 S0 m2)
+ *   (Geary's sum is taken per entry, never through its cancelling expansion). m2 = 0 or S0 = 0 gives NaN.
+ *   Analytic moments under normality, for the caller: Moran E = -1/(n-1), V = (n^2 S1 - n S2 + 3 S0^2) / ((n^2 - 1)
+ *   S0^2) - E^2; Geary E = 1, V = ((2 S1 + S2)(n - 1) - 4 S0^2) / (2 (n + 1) S0^2).
+ * Permutations: in labelling p (0 <= p < n_perms) node i takes the values x[pi_p(i)] of ALL columns at once (one
+ *   shuffle per permutation shared by the features, squidpy's procedure); pi_p is K15's, bit for bit, for the same seed.
+ *   The observed statistic is labelling "identity" and goes through the same arithmetic.
+ * Outputs (each pointer may be NULL), per column f:
+ *   stat [n_feat] float64; perm_mean, perm_var (ddof 0) [n_feat] float64 (NaN when n_perms = 0);
+ *   n_ge [n_feat] int64 = #{p : stat_p >= stat} (0 for a NaN stat); sims [n_perms][n_feat] float64 = stat_p;
+ *   s012 float64 [3] = S0, S1, S2.
+ * Every float sum has a fixed order (a thread's share, a shuffle tree, the warps in index order, the CTA partials in
+ * index order), so the outputs do not depend on the run, the chunking or the handle; no float atomics. A non-finite
+ * value in a column makes that column's outputs NaN (n_ge 0) and touches no other column. Asynchronous: no host
+ * synchronisation beyond workspace growth (32 n_feat/4 n bytes of centred values, int32 indices of at most
+ * PG_AUTOCORR_CHUNK_BYTES / 4n permutations at a time, 8 (n_perms + 1) n_feat bytes of statistics). PG_ERR_INVALID for
+ * n < 0, n_feat outside 1..PG_AUTOCORR_MAX_FEAT, n_perms outside 0..PG_ENRICH_MAX_PERMS, unknown flags, NULL inputs. */
+#define PG_AUTOCORR_GEARY 1    /* Geary's C instead of Moran's I */
+#define PG_AUTOCORR_ROW_STD 2  /* row-standardised weights w_ij = 1 / d_i instead of binary */
+#define PG_AUTOCORR_MAX_FEAT 256
+#define PG_AUTOCORR_CHUNK_BYTES (32 << 20)
+typedef struct {
+  double* stat;
+  double* perm_mean;
+  double* perm_var;
+  int64_t* n_ge;
+  double* sims;
+  double* s012;
+} pg_autocorr_out;
+int pg_spatial_autocorr(pg_handle* h, int32_t n, const int32_t* row_ptr, const int32_t* col, int32_t n_feat,
+                        const double* feat, int32_t flags, int32_t n_perms, uint64_t seed, const pg_autocorr_out* out,
+                        pg_stream stream);
+
 /* ---- K12: raster region properties of an instance map (SURVEY 8f-3): what skimage regionprops gives
  * aggregated_hovernet_run.py:172-181 (bbox per instance) and hovernet_tile_inference.ipynb:2415-2429 (cell 18:
  * area, perimeter, eccentricity, major / minor axis length, orientation).  inst_map int32 [height][width], labels

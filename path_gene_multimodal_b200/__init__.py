@@ -10,7 +10,8 @@ Public surface (reference-style module-level functions; see DESIGN.md / INTEGRAT
     neighbour_type_composition, degree_stats,
     filter_graph_by_type, clustering_coefficients,
     type_interaction_matrix, neighbourhood_enrichment,
-    co_occurrence, ripley, knn_graph_frame                (cell_graph)
+    co_occurrence, ripley, spatial_autocorr,
+    knn_graph_frame                                       (cell_graph)
     to_networkx                                           (interop: nx.Graph keyed by nuc_id, cell 11)
     read_nuclei_table, write_nuclei_table, table_to_soa,
     add_wsi_coords_to_table, process_nuclei_file          (nuclei_io: Parquet / CSV <-> SoA / CSR)
@@ -32,7 +33,7 @@ _EXPORTS = {
     "neighbour_type_composition": "cell_graph", "degree_stats": "cell_graph",
     "filter_graph_by_type": "cell_graph", "clustering_coefficients": "cell_graph",
     "type_interaction_matrix": "cell_graph", "neighbourhood_enrichment": "cell_graph",
-    "co_occurrence": "cell_graph", "ripley": "cell_graph",
+    "co_occurrence": "cell_graph", "ripley": "cell_graph", "spatial_autocorr": "cell_graph",
     "knn_graph_frame": "cell_graph", "to_networkx": "interop",
     "edge_index_from_edges": "graph_features",
     "read_nuclei_table": "nuclei_io", "write_nuclei_table": "nuclei_io", "table_to_soa": "nuclei_io",

@@ -11,7 +11,7 @@ PKG_DIR = Path(__file__).resolve().parent
 CSRC = PKG_DIR / "csrc"
 INCLUDE = PKG_DIR.parent / "include"
 LIB_PATH = PKG_DIR / "libpathgraph.so"
-SOURCES = ["pg_handle.cu", "pg_scan.cu", "pg_grid.cu", "pg_radius.cu", "pg_knn.cu", "pg_graph.cu", "pg_shard.cu", "pg_morph.cu", "pg_features.cu", "pg_raster.cu", "pg_contour.cu", "pg_hull.cu", "pg_enrich.cu", "pg_pairhist.cu"]
+SOURCES = ["pg_handle.cu", "pg_scan.cu", "pg_grid.cu", "pg_radius.cu", "pg_knn.cu", "pg_graph.cu", "pg_shard.cu", "pg_morph.cu", "pg_features.cu", "pg_raster.cu", "pg_contour.cu", "pg_hull.cu", "pg_enrich.cu", "pg_pairhist.cu", "pg_autocorr.cu"]
 
 NVCC_FLAGS = [
     "-gencode", "arch=compute_100a,code=sm_100a",

@@ -7,12 +7,15 @@ Mirrors /root/reference/hovernet_tile_inference.ipynb:
   ``edge_attr`` float32 [2E,1];
 * ``filter_graph_by_type`` cell 12 (ipynb:1989-2002);
 * ``neighbour_type_composition`` / ``degree_stats``: named in README.md:127,136 only; defined in SURVEY A.5;
-* ``co_occurrence`` / ``ripley``: cell-type patterns across distance (squidpy.gr.co_occurrence / ripley's statistics).
+* ``co_occurrence`` / ``ripley``: cell-type patterns across distance (squidpy.gr.co_occurrence / ripley's statistics);
+* ``spatial_autocorr``: Moran's I / Geary's C of per-nucleus features over the graph (squidpy.gr.spatial_autocorr).
 
 Host arrays in, host arrays out; everything in between is libpathgraph (uniform-grid binning, grid
 queries, two-pass CSR) on the GPU.  No CPU fallback.
 """
 from __future__ import annotations
+
+import math
 
 import numpy as np
 import torch
@@ -419,6 +422,149 @@ def ripley(coords, radii, types=None, n_types: int = 5, area: float | None = Non
     if univariate:
         k, lf, count = k[0, 0], lf[0, 0], count[0, 0]
     return {"radii": r, "K": k, "L": lf, "area": float(area), "n": n_t, "count": count}
+
+
+def _normal_tail(z) -> np.ndarray:
+    """P(Z > |z|) of a standard normal, elementwise (NaN stays NaN)."""
+    z = np.asarray(z, dtype=np.float64)
+    out = np.full(z.shape, np.nan)
+    ok = ~np.isnan(z)
+    out[ok] = [0.5 * math.erfc(abs(v) / math.sqrt(2.0)) for v in z[ok]]
+    return out
+
+
+def fdr_bh(pvals) -> np.ndarray:
+    """Benjamini-Hochberg adjusted p-values (statsmodels' ``multipletests(method="fdr_bh")``): p_(k) n / k with the
+    running minimum taken from the largest p down, clipped at 1. NaN p-values are left out and stay NaN."""
+    p = np.asarray(pvals, dtype=np.float64)
+    out = np.full(p.shape, np.nan)
+    ok = np.flatnonzero(~np.isnan(p))
+    if ok.size:
+        order = ok[np.argsort(p[ok], kind="stable")]
+        adj = p[order] * ok.size / np.arange(1, ok.size + 1)
+        out[order] = np.minimum(np.minimum.accumulate(adj[::-1])[::-1], 1.0)
+    return out
+
+
+def autocorr_moments(mode: str, n: int, s0: float, s1: float, s2: float) -> tuple[float, float]:
+    """Expectation and variance of Moran's I / Geary's C under the normality assumption, from the weight sums."""
+    with np.errstate(divide="ignore", invalid="ignore"):
+        n, s0, s1, s2 = (np.float64(v) for v in (n, s0, s1, s2))
+        if mode == "moran":
+            e = -1.0 / (n - 1.0)
+            v = (n * n * s1 - n * s2 + 3.0 * s0 * s0) / ((n * n - 1.0) * s0 * s0) - e * e
+        else:
+            e = np.float64(1.0)
+            v = ((2.0 * s1 + s2) * (n - 1.0) - 4.0 * s0 * s0) / (2.0 * (n + 1.0) * s0 * s0)
+    return float(e), float(v)
+
+
+def _csr_host(row_ptr, col) -> tuple[np.ndarray, np.ndarray]:
+    """Validated symmetric-CSR arrays as int32: row_ptr [N+1] starting at 0, non-decreasing, ending at len(col), and
+    col ids in [0, N)."""
+    rp, c = np.asarray(row_ptr), np.asarray(col)
+    if rp.ndim != 1 or rp.shape[0] < 1 or (rp.size and rp.dtype.kind not in "iu"):
+        raise ValueError("row_ptr must be a 1-D integer array of N + 1 offsets")
+    if c.ndim != 1 or (c.size and c.dtype.kind not in "iu"):
+        raise ValueError("col must be a 1-D integer array")
+    rp, c = rp.astype(np.int64), c.astype(np.int64)
+    n = rp.shape[0] - 1
+    if n > _host.INT32_MAX or c.shape[0] > _host.INT32_MAX:
+        raise ValueError("the graph must have fewer than 2^31 nodes and entries")
+    if rp[0] != 0 or rp[-1] != c.shape[0] or (np.diff(rp) < 0).any():
+        raise ValueError("row_ptr must start at 0, never decrease and end at len(col)")
+    if c.size and (c.min() < 0 or c.max() >= n):
+        raise ValueError(f"col ids must lie in [0, {n})")
+    return rp.astype(np.int32), c.astype(np.int32)
+
+
+def spatial_autocorr(row_ptr, col, features, mode: str = "moran", transformation: bool = True, n_perms=None,
+                     seed: int = 0, two_tailed: bool = False, corr_method: str | None = "fdr_bh", device=None):
+    """Spatial autocorrelation of per-nucleus features over a cell graph (squidpy.gr.spatial_autocorr's statistic):
+    Moran's I (``mode="moran"``) or Geary's C (``"geary"``) of every column, with its analytic and permutation p-values.
+
+    ``row_ptr`` / ``col``: a symmetric CSR without duplicate entries over N nodes (``build_radius_graph(...,
+    symmetric_csr=True)`` or ``build_knn_graph``).  ``features``: [N, F] array or DataFrame (for example
+    ``nuclei_morphology_table(...)[CONT_COLS]``), 1 <= F <= 256; column names become the index, rows keep the column
+    order.  ``transformation``: row-standardised weights 1 / degree (squidpy's default) instead of binary ones.
+    ``n_perms``: None for the analytic test only, else 1..100 000 permutations of the nodes, all columns shuffled
+    together (squidpy's procedure), drawn from ``seed`` by K15's keyed bijections (include/pathgraph.h) - the same
+    seed gives the same result bit for bit.
+
+    Returns a DataFrame with squidpy's columns: ``I`` or ``C``, ``pval_norm`` (the normal tail of (stat - E) / sqrt(V)
+    under the normality assumption) and ``var_norm`` (V); with permutations also ``pval_z_sim`` (the normal tail of
+    (stat - perm mean) / perm std), ``pval_sim`` = (min(n_ge, P - n_ge) + 1) / (P + 1), n_ge = permutations at or above
+    the observed value, and ``var_sim`` (ddof 0).  ``two_tailed`` doubles the three p-values, as squidpy does.
+    ``corr_method="fdr_bh"`` adds Benjamini-Hochberg ``<pval>_fdr_bh`` columns across the features (None: no
+    correction).  A constant column, or a graph without edges, gives a NaN statistic and NaN p-values (left out of the
+    adjustment).  Raises ``ValueError`` before anything is launched on a malformed CSR,
+    a feature table of the wrong length or width, a non-finite feature value (naming its column: a nucleus without a
+    polygon has NaN morphology and must be dropped or filled first), an unknown ``mode`` or ``corr_method``, or
+    ``n_perms`` out of range."""
+    import pandas as pd
+
+    if mode not in ("moran", "geary"):
+        raise ValueError(f"mode must be 'moran' or 'geary', got {mode!r}")
+    if corr_method not in (None, "fdr_bh"):
+        raise ValueError(f"corr_method must be 'fdr_bh' or None, got {corr_method!r}")
+    if n_perms is not None and not (isinstance(n_perms, (int, np.integer)) and 1 <= n_perms <= _lib.PG_ENRICH_MAX_PERMS):
+        raise ValueError(f"n_perms must be None or an int in 1..{_lib.PG_ENRICH_MAX_PERMS}")
+    rp, c = _csr_host(row_ptr, col)
+    n = rp.shape[0] - 1
+    if isinstance(features, pd.DataFrame):
+        names = list(features.columns)
+        x = features.to_numpy(dtype=np.float64)
+    else:
+        x = np.asarray(features, dtype=np.float64)
+        if x.ndim == 1:
+            x = x[:, None]
+        names = list(range(x.shape[1])) if x.ndim == 2 else []
+    if x.ndim != 2 or x.shape[0] != n:
+        raise ValueError(f"features must have shape (N, F) with N = {n} graph nodes")
+    if not 1 <= x.shape[1] <= _lib.PG_AUTOCORR_MAX_FEAT:
+        raise ValueError(f"features must have 1..{_lib.PG_AUTOCORR_MAX_FEAT} columns, got {x.shape[1]}")
+    bad = np.flatnonzero(~np.isfinite(x).all(axis=0))
+    if bad.size:
+        raise ValueError(f"feature column {names[bad[0]]!r} has non-finite values")
+    p = int(n_perms or 0)
+    eng = get_engine(device)
+    with torch.cuda.device(eng.device):
+        d_rp = _host.to_device(rp, np.int32, eng.device)
+        d_c = _host.to_device(c, np.int32, eng.device)
+        d_x = _host.to_device(np.ascontiguousarray(x.T), np.float64, eng.device)
+        res = _host.to_host_many(eng.spatial_autocorr(d_rp, d_c, d_x, mode, transformation, p, seed))
+    return autocorr_frame(res, names, mode, n, p, two_tailed, corr_method)
+
+
+def autocorr_frame(res: dict, names, mode: str, n: int, n_perms: int, two_tailed: bool = False,
+                   corr_method: str | None = "fdr_bh"):
+    """spatial_autocorr's DataFrame from the host copies of pg_spatial_autocorr's outputs (``stat``, ``perm_mean``,
+    ``perm_var``, ``n_ge``, ``s012``) over n nodes and ``n_perms`` permutations. Where the statistic is undefined (NaN:
+    a constant column, or a graph without edges) every p-value is NaN too, so it never reads as significant and the
+    Benjamini-Hochberg adjustment leaves it out."""
+    import pandas as pd
+
+    stat = np.asarray(res["stat"], dtype=np.float64)
+    undefined = np.isnan(stat)
+    e, v = autocorr_moments(mode, n, *res["s012"])
+    with np.errstate(divide="ignore", invalid="ignore"):
+        cols = {"I" if mode == "moran" else "C": stat, "pval_norm": _normal_tail((stat - e) / np.sqrt(v)),
+                "var_norm": np.full(stat.shape, v)}
+        if n_perms:
+            cols["pval_z_sim"] = _normal_tail((stat - res["perm_mean"]) / np.sqrt(res["perm_var"]))
+            n_ge = np.asarray(res["n_ge"])
+            cols["pval_sim"] = np.where(undefined, np.nan, (np.minimum(n_ge, n_perms - n_ge) + 1.0) / (n_perms + 1.0))
+            cols["var_sim"] = np.where(undefined, np.nan, res["perm_var"])
+    if two_tailed:
+        for k in ("pval_norm", "pval_z_sim", "pval_sim"):
+            if k in cols:
+                cols[k] = cols[k] * 2.0
+    df = pd.DataFrame(cols, index=pd.Index(names))
+    if corr_method is not None:
+        for k in ("pval_norm", "pval_z_sim", "pval_sim"):
+            if k in df.columns:
+                df[f"{k}_{corr_method}"] = fdr_bh(df[k].to_numpy())
+    return df
 
 
 def knn_graph_frame(final_df, k: int = 5, centroid_col: str = "centroid", centroid_order: str = "yx",

@@ -81,6 +81,12 @@ struct pg_handle {
   size_t hull_smem_set[2] = {0, 0};  // K14: dynamic shared memory opted in on this handle's device, per T
   pg_buf enrich_lab;   // K15 (pg_enrich.cu): uint8 labels of one chunk of permutations, [rows][n]
   pg_buf enrich_cnt;   // K15: int64 ordered type-pair counts per labelling, [P + 1][T * T]
+  pg_buf ac_z;         // K17 (pg_autocorr.cu): centred feature values, node-major groups of 4 columns, [G][n] double4
+  pg_buf ac_idx;       // K17: int32 pi_p(i) of one chunk of labellings, [rows][n]
+  pg_buf ac_deg;       // K17: int32 in-range entries per row
+  pg_buf ac_sims;      // K17: float64 statistic per labelling and column, [P + 1][n_feat] (row 0 = observed)
+  pg_buf ac_part;      // K17: float64 CTA partials of the fixed-order reductions
+  pg_buf ac_misc;      // K17: pg_ac_misc (column means / m2, S0-S2, integer degree sums) + CTA tickets
   // launch accounting / optional per-kernel CUDA-event timing (pg_profile_*)
   int64_t launches = 0;
   bool profiling = false;

@@ -7,8 +7,8 @@
 // labels, so its rows stay in L2 between the two kernels of the chunk and a 20 M-nucleus slide needs a bounded
 // workspace.
 //   perm_labels_kernel  lab[row][i] = type[pi_p(i)] as uint8 (0 = outside 1..T). One keyed Feistel evaluation per node
-//                       and permutation (x cycle-walks); each lane walks its own queue of nodes, so a lane whose walk
-//                       is long does not hold the other 31 lanes back.
+//                       and permutation (x cycle-walks; pg_perm.cuh, shared with K17); each lane walks its own queue
+//                       of nodes, so a lane whose walk is long does not hold the other 31 lanes back.
 //   perm_count_kernel   grid-stride over the edge rows of one labelling; every (t_i, t_j) pair is counted once in a
 //                       lane-private shared-memory column ([T*T][32] uint32: a warp's 32 increments always hit 32
 //                       different banks, so the dominant pair - type 1 x type 1 is a quarter of all entries on C2 -
@@ -18,20 +18,13 @@
 // Only integer atomics: the outputs do not depend on the order in which they arrive.
 #include <algorithm>
 #include "pg_common.cuh"
+#include "pg_perm.cuh"
 
 namespace {
 
 constexpr int TPB = 256;
-constexpr int ROUNDS = 8;
 constexpr int LAB_PER_THREAD = 16;     // nodes a labels thread walks (amortises its 8 round keys)
 constexpr int EDGES_PER_THREAD = 16;   // edge rows a count thread takes per labelling (amortises the counter flush)
-
-__device__ __forceinline__ uint64_t splitmix64(uint64_t x) {
-  uint64_t z = x + 0x9E3779B97F4A7C15ull;
-  z = (z ^ (z >> 30)) * 0xBF58476D1CE4E5B9ull;
-  z = (z ^ (z >> 27)) * 0x94D049BB133111EBull;
-  return z ^ (z >> 31);
-}
 
 __device__ __forceinline__ uint8_t label_of(int t, int n_types) {
   return (t >= 1 && t <= n_types) ? (uint8_t)t : (uint8_t)0;
@@ -49,29 +42,9 @@ perm_labels_kernel(const int32_t* __restrict__ type, int n, int n_types, int hbi
     for (; i < n; i += stride) out[i] = label_of(__ldg(&type[i]), n_types);
     return;
   }
-  const uint64_t p = (uint64_t)(row - 1);
-  uint64_t k[ROUNDS];
-#pragma unroll
-  for (int r = 0; r < ROUNDS; ++r) k[r] = splitmix64(seed ^ (64ull * p + (uint64_t)r));
-  const uint32_t mask = (1u << hbits) - 1u;
-  // one Feistel evaluation per iteration; a lane moves to its next node as soon as its walk lands inside [0, n)
-  uint32_t x = (uint32_t)i;
-  while (i < n) {
-    uint32_t L = x >> hbits, R = x & mask;
-#pragma unroll
-    for (int r = 0; r < ROUNDS; ++r) {
-      const uint32_t f = (uint32_t)splitmix64((uint64_t)R ^ k[r]) & mask;
-      const uint32_t nr = L ^ f;
-      L = R;
-      R = nr;
-    }
-    x = (L << hbits) | R;
-    if (x < (uint32_t)n) {
-      out[i] = label_of(__ldg(&type[x]), n_types);
-      i += stride;
-      x = (uint32_t)i;
-    }
-  }
+  uint64_t k[PG_PERM_ROUNDS];
+  pg_perm_keys(seed, (uint64_t)(row - 1), k);
+  pg_perm_walk(i, stride, n, hbits, k, [&](int64_t v, uint32_t x) { out[v] = label_of(__ldg(&type[x]), n_types); });
 }
 
 // cnt[blockIdx.y][(a-1) T + (b-1)] += number of edge rows (i, j) with labels (a, b) in labelling blockIdx.y
@@ -158,8 +131,7 @@ int pg_nhood_enrichment(pg_handle* h, int32_t n, const int32_t* type, int32_t n_
   unsigned long long* cnt = (unsigned long long*)h->enrich_cnt.p;
   PG_CUDA(h, cudaMemsetAsync(cnt, 0, (size_t)rows_total * nk * sizeof(int64_t), s));
   if (n > 0 && n_edges > 0) {
-    int hbits = 1;  // least h >= 1 with 4^h >= n
-    while (((int64_t)1 << (2 * hbits)) < (int64_t)n) ++hbits;
+    const int hbits = pg_perm_half_bits(n);
     const int64_t chunk = std::min<int64_t>({std::max<int64_t>(1, (int64_t)PG_ENRICH_CHUNK_BYTES / n), rows_total, 65535});
     if ((rc = pg_reserve(h, h->enrich_lab, (size_t)chunk * (size_t)n))) return rc;
     uint8_t* lab = (uint8_t*)h->enrich_lab.p;

@@ -125,7 +125,8 @@ int pg_destroy(pg_handle* h) {
   cudaDeviceSynchronize();
   pg_buf* bufs[] = {&h->cell_count, &h->cell_start, &h->cell_of, &h->rank,      &h->s_rec,     &h->s_pos,     &h->s_gid,     &h->knn_retry,     &h->pt_meta,   &h->tmp_ent,   &h->row_off,
                     &h->row_count,  &h->scan_state, &h->misc,    &h->sym_extra, &h->sym_cursor, &h->sym_recip, &h->hull,
-                    &h->enrich_lab, &h->enrich_cnt};
+                    &h->enrich_lab, &h->enrich_cnt, &h->ac_z,    &h->ac_idx,    &h->ac_deg,     &h->ac_sims,    &h->ac_part,
+                    &h->ac_misc};
   for (pg_buf* b : bufs)
     if (b->p) cudaFree(b->p);
   if (h->pinned) cudaFreeHost(h->pinned);
@@ -140,7 +141,8 @@ int64_t pg_workspace_bytes(pg_handle* h) {
   if (!h) return 0;
   pg_buf* bufs[] = {&h->cell_count, &h->cell_start, &h->cell_of, &h->rank,      &h->s_rec,     &h->s_pos,     &h->s_gid,     &h->knn_retry,     &h->pt_meta,   &h->tmp_ent,   &h->row_off,
                     &h->row_count,  &h->scan_state, &h->misc,    &h->sym_extra, &h->sym_cursor, &h->sym_recip, &h->hull,
-                    &h->enrich_lab, &h->enrich_cnt};
+                    &h->enrich_lab, &h->enrich_cnt, &h->ac_z,    &h->ac_idx,    &h->ac_deg,     &h->ac_sims,    &h->ac_part,
+                    &h->ac_misc};
   int64_t t = 0;
   for (pg_buf* b : bufs) t += (int64_t)b->cap;
   return t;

@@ -587,6 +587,45 @@ class Engine:
                                                  C.byref(eo), self._stream()))
         return res
 
+    # ---- K17 -----------------------------------------------------------------------------------
+    def spatial_autocorr(self, row_ptr, col, feat, mode="moran", transformation=True, n_perms=0, seed=0,
+                         want_sims=False):
+        """Moran's I / Geary's C of every feature column over a symmetric CSR, with permutation statistics
+        (pg_spatial_autocorr).
+
+        row_ptr int32 [N+1], col int32 [E] (entries outside [0, N) are skipped); feat float64 [F, N] (one row per
+        column); ``transformation``: row-standardised weights 1 / d_i instead of binary ones.  Returns a dict of device
+        tensors: stat, perm_mean, perm_var float64 [F], n_ge int64 [F], s012 float64 [3] (S0, S1, S2) and, with
+        ``want_sims``, sims float64 [n_perms, F].  Asynchronous (no host synchronisation once the workspace has grown)."""
+        if mode not in ("moran", "geary"):
+            raise ValueError(f"mode must be 'moran' or 'geary', got {mode!r}")
+        if feat.dim() != 2:
+            raise ValueError("feat must have shape (F, N)")
+        n = int(row_ptr.numel()) - 1
+        n_feat = int(feat.shape[0])
+        if n < 0 or int(feat.shape[1]) != n:
+            raise ValueError("feat must have one value per CSR row")
+        seed = int(seed)
+        if not 0 <= seed < 2 ** 64:
+            raise ValueError("seed must be in [0, 2**64)")
+        p = int(n_perms)
+        flags = (_lib.PG_AUTOCORR_GEARY if mode == "geary" else 0) | (_lib.PG_AUTOCORR_ROW_STD if transformation else 0)
+        res = {name: self._empty((n_feat,), torch.float64) for name in ("stat", "perm_mean", "perm_var")}
+        res["n_ge"] = self._empty((n_feat,), torch.int64)
+        res["s012"] = self._empty((3,), torch.float64)
+        if want_sims:
+            res["sims"] = self._empty((p, n_feat), torch.float64)
+        ao = _lib.PgAutocorrOut()
+        for name, t in res.items():
+            setattr(ao, name, self._p(t, torch.int64 if name == "n_ge" else torch.float64, name))
+        if col is None or col.numel() == 0:  # no entries: the C entry still wants a col array it will not read
+            col = self._empty((1,), torch.int32)
+        self._check(self.lib.pg_spatial_autocorr(self._h, n, self._p(row_ptr, torch.int32, "row_ptr"),
+                                                 self._p(col, torch.int32, "col"), n_feat,
+                                                 self._p(feat, torch.float64, "feat"), flags, p, seed, C.byref(ao),
+                                                 self._stream()))
+        return res
+
     # ---- K16 -----------------------------------------------------------------------------------
     def pair_dist_hist(self, thresholds, n_types=5):
         """Type-pair distance histogram over the built grid (pg_pair_dist_hist).
