@@ -400,6 +400,62 @@ int pg_spatial_autocorr(pg_handle* h, int32_t n, const int32_t* row_ptr, const i
                         const double* feat, int32_t flags, int32_t n_perms, uint64_t seed, const pg_autocorr_out* out,
                         pg_stream stream);
 
+/* ---- K18: local indicators of spatial association (csrc/pg_lisa.cu): one value per node and feature column, which
+ * says WHERE a feature clusters (immune hot spots, regions of large nuclei, the cold margin around them) where K17 says
+ * whether. Local Moran's I_i (Anselin 1995; PySAL esda Moran_Local) or Getis-Ord Gi / Gi* z-scores (Ord & Getis 1995;
+ * esda G_Local), with conditional permutation tests.
+ *   row_ptr / col: a symmetric CSR as for K17. Entries with col outside [0, n) and self entries (col == i) are skipped:
+ *           conditional randomisation keeps node i fixed (esda separates self weights for the same reason).
+ *           d_i = the remaining entries of row i.
+ *   feat    float64 [n_feat][n] (K10's layout), 1 <= n_feat <= PG_AUTOCORR_MAX_FEAT.
+ * Weights: w = 1 (binary) or w = 1 / d_i (PG_AUTOCORR_ROW_STD). Per column, z = x - mean over all n nodes (K17's
+ * centring, bit for bit), m2 = sum z^2.
+ *   lag     S_i = sum_{j in N(i)} z_j in CSR entry order; L_i = S_i (binary) or S_i / d_i (row-standardised; 0 when
+ *           d_i = 0).
+ *   Moran   I_i = c z_i L_i, c = (n - 1) / m2 (esda's n_1 z lz / den).
+ *   Gi*     (PG_LOCAL_GETIS_ORD | PG_LOCAL_STAR): the self term belongs to the neighbourhood. Binary: W_i = S1_i = d_i + 1,
+ *           w_ii = w = 1; row-standardised: W_i = 1, S1_i = w_ii = w = 1 / (d_i + 1).
+ *           Z_i = (w_ii z_i + w S_i) / (sqrt(m2 / n) sqrt((n S1_i - W_i^2) / (n - 1))).
+ *   Gi      (PG_LOCAL_GETIS_ORD): binary W_i = S1_i = d_i; row-standardised W_i = 1, S1_i = 1 / d_i.
+ *           N_i = L_i + W_i z_i / (n - 1), s_i^2 = (m2 - z_i^2 n / (n - 1)) / (n - 1),
+ *           Z_i = N_i / (s_i sqrt(((n - 1) S1_i - W_i^2) / (n - 2)))
+ *           (Ord & Getis's x(i) mean and S(i) over the other n - 1 values, rewritten on z so that nothing cancels).
+ *   A quantity <= 0 under a square root, m2 = 0 or n too small for the formula (Gi*: n < 2, Gi: n < 3) gives NaN.
+ * Draws: K = max d_i. Permutation p draws r_p[j] = pi'_p(j), j < K, pi'_p K15's keyed bijection (same round keys
+ *   k_{p,r}) on [0, n - 1): a uniform K-subset in random order, the role of esda's permutation(n - 1)[:max_card]. Node i's
+ *   j-th neighbour in permutation p is s = r_p[j] + (r_p[j] >= i) (never i itself); S_ip = sum_{j < d_i} z_s in ascending
+ *   j, and stat_ip follows from S_ip through the same arithmetic as stat_i from S_i. All nodes and columns share the
+ *   draws of a permutation.
+ * Outputs, each pointer may be NULL, [n_feat][n] unless stated:
+ *   stat, lag float64: I_i or Z_i, and L_i;
+ *   n_ge int32 = #{p : stat_ip >= stat_i} (0 for a NaN stat or d_i = 0);
+ *   perm_mean, perm_var float64 (ddof 0) from d1 = sum_p delta_p and d2 = sum_p delta_p^2, delta_p = stat_ip - stat_i,
+ *     both in ascending p: perm_mean = stat_i + d1 / P, perm_var = max(0, d2 / P - (d1 / P)^2); NaN when n_perms = 0 or
+ *     d_i = 0;
+ *   sims float64 [n_perms][n_feat][n] = stat_ip (NaN where d_i = 0), for tests on small graphs;
+ *   mean, m2 float64 [n_feat].
+ * Isolated nodes (d_i = 0) keep the formula's statistic and get no permutation outputs. A non-finite value in a column
+ * makes that column NaN (n_ge 0) and touches no other column. Every float sum has a fixed order and every node's
+ * permutation sums live in one thread, so the outputs do not depend on the run or the handle; no float atomics.
+ * Asynchronous: no host synchronisation beyond workspace growth (K17's 32 n_feat/4 n bytes of centred values, 12 n
+ * bytes of degrees and degree order). PG_ERR_INVALID on K17's conditions, and PG_LOCAL_STAR without
+ * PG_LOCAL_GETIS_ORD. */
+#define PG_LOCAL_GETIS_ORD 4  /* Getis-Ord Gi instead of local Moran */
+#define PG_LOCAL_STAR 8       /* Gi*: node i counts in its own neighbourhood */
+typedef struct {
+  double* stat;
+  double* lag;
+  int32_t* n_ge;
+  double* perm_mean;
+  double* perm_var;
+  double* sims;
+  double* mean;
+  double* m2;
+} pg_local_out;
+int pg_local_autocorr(pg_handle* h, int32_t n, const int32_t* row_ptr, const int32_t* col, int32_t n_feat,
+                      const double* feat, int32_t flags, int32_t n_perms, uint64_t seed, const pg_local_out* out,
+                      pg_stream stream);
+
 /* ---- K12: raster region properties of an instance map (SURVEY 8f-3): what skimage regionprops gives
  * aggregated_hovernet_run.py:172-181 (bbox per instance) and hovernet_tile_inference.ipynb:2415-2429 (cell 18:
  * area, perimeter, eccentricity, major / minor axis length, orientation).  inst_map int32 [height][width], labels

@@ -21,6 +21,8 @@ PG_PAIRHIST_MAX_THR = 64
 PG_AUTOCORR_GEARY = 1
 PG_AUTOCORR_ROW_STD = 2
 PG_AUTOCORR_MAX_FEAT = 256
+PG_LOCAL_GETIS_ORD = 4
+PG_LOCAL_STAR = 8
 
 PG_OK, PG_ERR_INVALID, PG_ERR_CUDA, PG_ERR_STATE, PG_ERR_CAPACITY, PG_ERR_NOMEM = 0, -1, -2, -3, -4, -5
 
@@ -61,6 +63,10 @@ class PgEnrichOut(C.Structure):
 
 class PgAutocorrOut(C.Structure):
     _fields_ = [(name, vp) for name in ("stat", "perm_mean", "perm_var", "n_ge", "sims", "s012")]
+
+
+class PgLocalOut(C.Structure):
+    _fields_ = [(name, vp) for name in ("stat", "lag", "n_ge", "perm_mean", "perm_var", "sims", "mean", "m2")]
 
 
 class PathGraphError(RuntimeError):
@@ -117,6 +123,7 @@ SIGNATURES = {
     "pg_type_interactions": (C.c_int, [vp, i32, vp, vp, i32, vp, vp]),
     "pg_nhood_enrichment": (C.c_int, [vp, i32, vp, i32, i64, vp, i32, C.c_uint64, C.POINTER(PgEnrichOut), vp]),
     "pg_spatial_autocorr": (C.c_int, [vp, i32, vp, vp, i32, vp, i32, i32, C.c_uint64, C.POINTER(PgAutocorrOut), vp]),
+    "pg_local_autocorr": (C.c_int, [vp, i32, vp, vp, i32, vp, i32, i32, C.c_uint64, C.POINTER(PgLocalOut), vp]),
     "pg_pair_dist_hist": (C.c_int, [vp, i32, i32, C.POINTER(f64), vp, vp, vp]),
     "pg_raster_props": (C.c_int, [vp, i32, i32, vp, i32, C.POINTER(PgRasterOut), vp]),
     "pg_raster_solidity": (C.c_int, [vp, i32, i32, vp, i32, vp, vp, vp, vp, vp]),

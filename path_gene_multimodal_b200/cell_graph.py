@@ -8,7 +8,9 @@ Mirrors /root/reference/hovernet_tile_inference.ipynb:
 * ``filter_graph_by_type`` cell 12 (ipynb:1989-2002);
 * ``neighbour_type_composition`` / ``degree_stats``: named in README.md:127,136 only; defined in SURVEY A.5;
 * ``co_occurrence`` / ``ripley``: cell-type patterns across distance (squidpy.gr.co_occurrence / ripley's statistics);
-* ``spatial_autocorr``: Moran's I / Geary's C of per-nucleus features over the graph (squidpy.gr.spatial_autocorr).
+* ``spatial_autocorr``: Moran's I / Geary's C of per-nucleus features over the graph (squidpy.gr.spatial_autocorr);
+* ``local_autocorr``: local Moran's I_i / Getis-Ord Gi(*) per nucleus, where a feature clusters (esda Moran_Local /
+  G_Local).
 
 Host arrays in, host arrays out; everything in between is libpathgraph (uniform-grid binning, grid
 queries, two-pass CSR) on the GPU.  No CPU fallback.
@@ -478,6 +480,28 @@ def _csr_host(row_ptr, col) -> tuple[np.ndarray, np.ndarray]:
     return rp.astype(np.int32), c.astype(np.int32)
 
 
+def _feature_matrix(features, n: int) -> tuple[np.ndarray, list]:
+    """Validated float64 [n, F] feature values and the column names, from an [N, F] / [N] array or a DataFrame."""
+    import pandas as pd
+
+    if isinstance(features, pd.DataFrame):
+        names = list(features.columns)
+        x = features.to_numpy(dtype=np.float64)
+    else:
+        x = np.asarray(features, dtype=np.float64)
+        if x.ndim == 1:
+            x = x[:, None]
+        names = list(range(x.shape[1])) if x.ndim == 2 else []
+    if x.ndim != 2 or x.shape[0] != n:
+        raise ValueError(f"features must have shape (N, F) with N = {n} graph nodes")
+    if not 1 <= x.shape[1] <= _lib.PG_AUTOCORR_MAX_FEAT:
+        raise ValueError(f"features must have 1..{_lib.PG_AUTOCORR_MAX_FEAT} columns, got {x.shape[1]}")
+    bad = np.flatnonzero(~np.isfinite(x).all(axis=0))
+    if bad.size:
+        raise ValueError(f"feature column {names[bad[0]]!r} has non-finite values")
+    return x, names
+
+
 def spatial_autocorr(row_ptr, col, features, mode: str = "moran", transformation: bool = True, n_perms=None,
                      seed: int = 0, two_tailed: bool = False, corr_method: str | None = "fdr_bh", device=None):
     """Spatial autocorrelation of per-nucleus features over a cell graph (squidpy.gr.spatial_autocorr's statistic):
@@ -501,8 +525,6 @@ def spatial_autocorr(row_ptr, col, features, mode: str = "moran", transformation
     a feature table of the wrong length or width, a non-finite feature value (naming its column: a nucleus without a
     polygon has NaN morphology and must be dropped or filled first), an unknown ``mode`` or ``corr_method``, or
     ``n_perms`` out of range."""
-    import pandas as pd
-
     if mode not in ("moran", "geary"):
         raise ValueError(f"mode must be 'moran' or 'geary', got {mode!r}")
     if corr_method not in (None, "fdr_bh"):
@@ -511,21 +533,7 @@ def spatial_autocorr(row_ptr, col, features, mode: str = "moran", transformation
         raise ValueError(f"n_perms must be None or an int in 1..{_lib.PG_ENRICH_MAX_PERMS}")
     rp, c = _csr_host(row_ptr, col)
     n = rp.shape[0] - 1
-    if isinstance(features, pd.DataFrame):
-        names = list(features.columns)
-        x = features.to_numpy(dtype=np.float64)
-    else:
-        x = np.asarray(features, dtype=np.float64)
-        if x.ndim == 1:
-            x = x[:, None]
-        names = list(range(x.shape[1])) if x.ndim == 2 else []
-    if x.ndim != 2 or x.shape[0] != n:
-        raise ValueError(f"features must have shape (N, F) with N = {n} graph nodes")
-    if not 1 <= x.shape[1] <= _lib.PG_AUTOCORR_MAX_FEAT:
-        raise ValueError(f"features must have 1..{_lib.PG_AUTOCORR_MAX_FEAT} columns, got {x.shape[1]}")
-    bad = np.flatnonzero(~np.isfinite(x).all(axis=0))
-    if bad.size:
-        raise ValueError(f"feature column {names[bad[0]]!r} has non-finite values")
+    x, names = _feature_matrix(features, n)
     p = int(n_perms or 0)
     eng = get_engine(device)
     with torch.cuda.device(eng.device):
@@ -565,6 +573,106 @@ def autocorr_frame(res: dict, names, mode: str, n: int, n_perms: int, two_tailed
             if k in df.columns:
                 df[f"{k}_{corr_method}"] = fdr_bh(df[k].to_numpy())
     return df
+
+
+def local_autocorr(row_ptr, col, features, mode: str = "moran", transformation: bool = True, star: bool = True,
+                   n_perms: int = 999, seed: int = 0, alpha: float = 0.05, corr_method: str | None = "fdr_bh",
+                   device=None):
+    """Local indicators of spatial association of per-nucleus features over a cell graph: where on the slide a feature
+    clusters. Local Moran's I_i with its quadrant (``mode="moran"``; PySAL esda ``Moran_Local``) or Getis-Ord Gi* / Gi
+    hot-spot z-scores (``"getis_ord"``; esda ``G_Local``), per node and column, with conditional permutation tests:
+    node i keeps its value and its d_i neighbours are replaced by d_i values drawn from the other N - 1 nodes.
+
+    ``row_ptr`` / ``col``: a symmetric CSR over N nodes (``build_radius_graph(..., symmetric_csr=True)`` or
+    ``build_knn_graph``); self entries are skipped.  ``features``: [N, F] array or DataFrame, 1 <= F <= 256.
+    ``transformation``: row-standardised weights 1 / degree instead of binary ones.  ``star``: Gi* (the node counts in
+    its own neighbourhood) rather than Gi; Getis-Ord only.  ``n_perms``: 1..100 000 permutations drawn from ``seed`` by
+    K15's keyed bijections (include/pathgraph.h; the same seed gives the same result bit for bit); every node and
+    column shares the draws of one permutation, as esda does.
+
+    Returns a DataFrame indexed by node with columns ``(feature, field)``.  Moran fields: ``I``, ``q`` (1 HH, 2 LH,
+    3 LL, 4 HL from x - mean > 0 and lag > 0), ``lag``, ``EI_sim``, ``VI_sim`` (mean and ddof-0 variance of the
+    permuted I), ``z_sim``, ``p_z_sim`` (its normal tail), ``p_sim`` = (min(n_ge, P - n_ge) + 1) / (P + 1) with n_ge the
+    permutations at or above the observed value (esda's folding).  Getis-Ord fields: ``Z``, ``G`` (esda's ratio
+    sum_j w_ij x_j / sum_{j != i} x_j, with i in both sums for Gi*), ``p_norm`` (normal tail of Z), ``EZ_sim``,
+    ``VZ_sim`` and the same ``z_sim`` / ``p_z_sim`` / ``p_sim``.  ``corr_method="fdr_bh"`` adds ``p_sim_fdr_bh``,
+    Benjamini-Hochberg across the nodes of each feature.  ``cluster``: Moran q where the (adjusted) ``p_sim`` <=
+    ``alpha``, else 0; Getis-Ord +1 (hot) / -1 (cold) / 0.  Isolated nodes and undefined statistics (a constant column,
+    a Gi node without neighbours) have NaN p-values and cluster 0, and are left out of the adjustment.
+
+    Raises ``ValueError`` before anything is launched on a malformed CSR, a feature table of the wrong length or width,
+    a non-finite feature value (naming its column), an unknown ``mode`` or ``corr_method``, ``n_perms`` out of range or
+    ``alpha`` outside (0, 1)."""
+    if mode not in ("moran", "getis_ord"):
+        raise ValueError(f"mode must be 'moran' or 'getis_ord', got {mode!r}")
+    if corr_method not in (None, "fdr_bh"):
+        raise ValueError(f"corr_method must be 'fdr_bh' or None, got {corr_method!r}")
+    if not (isinstance(n_perms, (int, np.integer)) and 1 <= n_perms <= _lib.PG_ENRICH_MAX_PERMS):
+        raise ValueError(f"n_perms must be an int in 1..{_lib.PG_ENRICH_MAX_PERMS}")
+    if not (isinstance(alpha, (int, float, np.floating)) and 0.0 < alpha < 1.0):
+        raise ValueError(f"alpha must lie in (0, 1), got {alpha!r}")
+    rp, c = _csr_host(row_ptr, col)
+    n = rp.shape[0] - 1
+    x, names = _feature_matrix(features, n)
+    eng = get_engine(device)
+    with torch.cuda.device(eng.device):
+        d_rp = _host.to_device(rp, np.int32, eng.device)
+        d_c = _host.to_device(c, np.int32, eng.device)
+        d_x = _host.to_device(np.ascontiguousarray(x.T), np.float64, eng.device)
+        res = _host.to_host_many(eng.local_autocorr(d_rp, d_c, d_x, mode, transformation, star, int(n_perms), seed))
+    rows = np.repeat(np.arange(n, dtype=np.int64), np.diff(rp.astype(np.int64)))
+    deg = np.bincount(rows[c != rows], minlength=n)
+    return local_frame(res, x, names, deg, mode, transformation, star, int(n_perms), alpha, corr_method)
+
+
+def local_frame(res: dict, x, names, deg, mode: str, transformation: bool, star: bool, n_perms: int,
+                alpha: float = 0.05, corr_method: str | None = "fdr_bh"):
+    """local_autocorr's DataFrame from the host copies of pg_local_autocorr's outputs (``stat``, ``lag``, ``n_ge``,
+    ``perm_mean``, ``perm_var`` [F, N], ``mean`` [F]), the feature values x [N, F] and the degrees d_i (entries other
+    than i) of the N nodes."""
+    import pandas as pd
+
+    x = np.asarray(x, dtype=np.float64)
+    deg = np.asarray(deg, dtype=np.int64)
+    n = x.shape[0]
+    cols = {}
+    for f, name in enumerate(names):
+        stat, lag = res["stat"][f], res["lag"][f]
+        undefined = np.isnan(stat) | (deg == 0)
+        n_ge = np.asarray(res["n_ge"][f], dtype=np.int64)
+        p_sim = np.where(undefined, np.nan, (np.minimum(n_ge, n_perms - n_ge) + 1.0) / (n_perms + 1.0))
+        with np.errstate(divide="ignore", invalid="ignore"):
+            z_sim = (stat - res["perm_mean"][f]) / np.sqrt(res["perm_var"][f])
+        z_sim[undefined] = np.nan
+        p_adj = fdr_bh(p_sim) if corr_method is not None else p_sim
+        sig = p_adj <= alpha
+        if mode == "moran":
+            hi_x, hi_lag = x[:, f] - res["mean"][f] > 0, lag > 0
+            q = np.where(hi_x, np.where(hi_lag, 1, 4), np.where(hi_lag, 2, 3))
+            fields = {"I": stat, "q": q, "lag": lag, "EI_sim": res["perm_mean"][f], "VI_sim": res["perm_var"][f]}
+            cluster = np.where(sig, q, 0)
+        else:
+            mean = res["mean"][f]
+            if star:
+                w = 1.0 / (deg + 1.0) if transformation else 1.0
+                num = w * (x[:, f] + deg * (lag + mean) if transformation else x[:, f] + lag + deg * mean)
+                den = n * mean
+            else:
+                wsum = (deg > 0).astype(np.float64) if transformation else deg.astype(np.float64)
+                num = lag + wsum * mean
+                den = n * mean - x[:, f]
+            with np.errstate(divide="ignore", invalid="ignore"):
+                g = num / den
+            fields = {"Z": stat, "G": g, "p_norm": _normal_tail(stat), "EZ_sim": res["perm_mean"][f],
+                      "VZ_sim": res["perm_var"][f]}
+            cluster = np.where(sig, np.sign(np.nan_to_num(stat)).astype(np.int64), 0)
+        fields.update({"z_sim": z_sim, "p_z_sim": _normal_tail(z_sim), "p_sim": p_sim})
+        if corr_method is not None:
+            fields[f"p_sim_{corr_method}"] = p_adj
+        fields["cluster"] = cluster.astype(np.int64)
+        for k, v in fields.items():
+            cols[(name, k)] = v
+    return pd.DataFrame(cols, index=pd.RangeIndex(n, name="node"))
 
 
 def knn_graph_frame(final_df, k: int = 5, centroid_col: str = "centroid", centroid_order: str = "yx",

@@ -87,6 +87,10 @@ struct pg_handle {
   pg_buf ac_sims;      // K17: float64 statistic per labelling and column, [P + 1][n_feat] (row 0 = observed)
   pg_buf ac_part;      // K17: float64 CTA partials of the fixed-order reductions
   pg_buf ac_misc;      // K17: pg_ac_misc (column means / m2, S0-S2, integer degree sums) + CTA tickets
+                       // K18 (pg_lisa.cu) uses ac_z / ac_deg / ac_part / ac_misc for the same prep and degree passes
+  pg_buf lk_cnt;       // K18: int32 nodes per degree [n + 1]; the scan clears it and it becomes the scatter cursor
+  pg_buf lk_off;       // K18: int32 exclusive scan of lk_cnt [n + 1]
+  pg_buf lk_ord;       // K18: int32 nodes in ascending degree [n]
   // launch accounting / optional per-kernel CUDA-event timing (pg_profile_*)
   int64_t launches = 0;
   bool profiling = false;

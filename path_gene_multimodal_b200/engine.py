@@ -626,6 +626,49 @@ class Engine:
                                                  self._stream()))
         return res
 
+    # ---- K18 -----------------------------------------------------------------------------------
+    def local_autocorr(self, row_ptr, col, feat, mode="moran", transformation=True, star=True, n_perms=0, seed=0,
+                       want_sims=False):
+        """Local Moran's I_i or Getis-Ord Gi / Gi* of every node and feature column over a symmetric CSR, with
+        conditional permutation statistics (pg_local_autocorr).
+
+        row_ptr int32 [N+1], col int32 [E] (entries outside [0, N) and self entries are skipped); feat float64 [F, N]
+        (one row per column); ``mode`` "moran" or "getis_ord"; ``transformation``: row-standardised weights 1 / d_i;
+        ``star``: Gi* (node i in its own neighbourhood; Getis-Ord only).  Returns a dict of device tensors: stat, lag,
+        perm_mean, perm_var float64 [F, N], n_ge int32 [F, N], mean, m2 float64 [F] and, with ``want_sims``, sims
+        float64 [n_perms, F, N].  Asynchronous (no host synchronisation once the workspace has grown)."""
+        if mode not in ("moran", "getis_ord"):
+            raise ValueError(f"mode must be 'moran' or 'getis_ord', got {mode!r}")
+        if feat.dim() != 2:
+            raise ValueError("feat must have shape (F, N)")
+        n = int(row_ptr.numel()) - 1
+        n_feat = int(feat.shape[0])
+        if n < 0 or int(feat.shape[1]) != n:
+            raise ValueError("feat must have one value per CSR row")
+        seed = int(seed)
+        if not 0 <= seed < 2 ** 64:
+            raise ValueError("seed must be in [0, 2**64)")
+        p = int(n_perms)
+        flags = _lib.PG_AUTOCORR_ROW_STD if transformation else 0
+        if mode == "getis_ord":
+            flags |= _lib.PG_LOCAL_GETIS_ORD | (_lib.PG_LOCAL_STAR if star else 0)
+        res = {name: self._empty((n_feat, n), torch.float64) for name in ("stat", "lag", "perm_mean", "perm_var")}
+        res["n_ge"] = self._empty((n_feat, n), torch.int32)
+        res["mean"] = self._empty((n_feat,), torch.float64)
+        res["m2"] = self._empty((n_feat,), torch.float64)
+        if want_sims:
+            res["sims"] = self._empty((p, n_feat, n), torch.float64)
+        lo = _lib.PgLocalOut()
+        for name, t in res.items():
+            setattr(lo, name, self._p(t, torch.int32 if name == "n_ge" else torch.float64, name))
+        if col is None or col.numel() == 0:  # no entries: the C entry still wants a col array it will not read
+            col = self._empty((1,), torch.int32)
+        self._check(self.lib.pg_local_autocorr(self._h, n, self._p(row_ptr, torch.int32, "row_ptr"),
+                                               self._p(col, torch.int32, "col"), n_feat,
+                                               self._p(feat, torch.float64, "feat"), flags, p, seed, C.byref(lo),
+                                               self._stream()))
+        return res
+
     # ---- K16 -----------------------------------------------------------------------------------
     def pair_dist_hist(self, thresholds, n_types=5):
         """Type-pair distance histogram over the built grid (pg_pair_dist_hist).
