@@ -84,7 +84,8 @@ int64_t pg_workspace_bytes(pg_handle* h);
  *   tile_x/y  int32 [n_tiles]
  *   centroid  f64   [N,2]   tile-local centroid (NULL = skip)   -> wsi_centroid f64 [N,2]
  *   bbox      int32 [N,4]   tile-local bbox     (NULL = skip)   -> wsi_bbox int32 [N,4]
- *   wsi_poly_xy T   [M,2]   shifted vertices (NULL = skip)
+ *   wsi_poly_xy T   [M,2]   shifted vertices (NULL = skip); a separate array: it must not overlap poly_xy
+ *                           (the shift is not in place; wsi_poly_xy == poly_xy gives PG_ERR_INVALID)
  * Rows with < 3 vertices give NaN features. */
 /* Optional: tell the library how long the rings of the coming pg_map_morph_* calls are (n rings, total_vertices
  * vertices), so that a warp's 32 rings fit its shared-memory staging slab; without it slabs are sized for rings of

@@ -18,6 +18,7 @@
 // closed-form epilogue and all per-polygon loads / stores run one polygon per lane, fully coalesced.
 #include <algorithm>
 #include <cmath>
+#include <string>
 #include "pg_common.cuh"
 #include "pg_ring.cuh"
 
@@ -269,6 +270,15 @@ map_morph_kernel(int n, const int32_t* __restrict__ poly_off, const typename vec
   }
 }
 
+// launch-record name of one instantiation, e.g. "map_morph_kernel<f32, plain, 7>": the profile records say which
+// variant the launcher picked (tests/test_gpu_morph_variants.py relies on it)
+template <typename T, bool EXTRA, int MINB>
+const char* map_morph_name() {
+  static const std::string name = std::string("map_morph_kernel<") + (sizeof(T) == 4 ? "f32" : "f64") +
+                                  (EXTRA ? ", extra, " : ", plain, ") + std::to_string(MINB) + ">";
+  return name.c_str();
+}
+
 template <typename T>
 int launch_map_morph(pg_handle* h, int32_t n, const int32_t* poly_off, const T* poly_xy, const int32_t* nuc_tile,
                      const int32_t* tile_x, const int32_t* tile_y, const double* centroid, const int32_t* bbox,
@@ -286,6 +296,9 @@ int launch_map_morph(pg_handle* h, int32_t n, const int32_t* poly_off, const T* 
   PG_REQUIRE(h, (((uintptr_t)poly_xy | (uintptr_t)wsi_poly_xy) & (sizeof(V2) - 1)) == 0 &&
                     (((uintptr_t)centroid | (uintptr_t)wsi_centroid | (uintptr_t)bbox | (uintptr_t)wsi_bbox) & 15) == 0,
              "pg_map_morph: vertex / centroid / bbox arrays must be aligned to their vector width");
+  // the 8-lanes-per-ring path reads vertex 0 of a ring again for its closing edge after another lane has shifted it,
+  // and both pointers are __restrict__: an in-place shift would give wrong features, so it is refused
+  PG_REQUIRE(h, !wsi_poly_xy || wsi_poly_xy != poly_xy, "pg_map_morph: wsi_poly_xy must not alias poly_xy");
   if (n == 0) return PG_OK;
   pg_morph_out o{};
   if (out) o = *out;
@@ -316,7 +329,9 @@ int launch_map_morph(pg_handle* h, int32_t n, const int32_t* poly_off, const T* 
     PG_CUDA(h, cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)SLAB_BYTES_MAX));
     granted = SLAB_BYTES_MAX;
   }
-  PG_LAUNCH(h, s, extra ? "map_morph_kernel<T, true>" : "map_morph_kernel<T, false>",
+  const char* name = extra ? map_morph_name<T, true, MINB0X>()
+                           : (dense ? map_morph_name<T, false, PG_MORPH_DENSE>() : map_morph_name<T, false, MINB0>());
+  PG_LAUNCH(h, s, name,
             kern<<<blocks, TPB, smem, s>>>(n, poly_off, (const V2*)poly_xy, nuc_tile, tile_x, tile_y,
                                            (const double2*)centroid, (const int4*)bbox, (V2*)wsi_poly_xy,
                                            (double2*)wsi_centroid, (int4*)wsi_bbox, o, slab_verts));

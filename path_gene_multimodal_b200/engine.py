@@ -165,7 +165,8 @@ class Engine:
         centroid float64 [N,2]; bbox int32 [N,4].  Returns a dict of device tensors:
         wsi_poly_xy, wsi_centroid, wsi_bbox, area, perimeter, eccentricity, circularity and, with
         ``extra``, major_axis, minor_axis, centroid_x, centroid_y, poly_bbox.  ``out`` may carry
-        preallocated tensors of the same names (reused, not reallocated).
+        preallocated tensors of the same names (reused, not reallocated); ``out["wsi_poly_xy"]`` must not overlap
+        ``poly_xy`` (ValueError).
         """
         n = int(poly_off.numel()) - 1
         vt = poly_xy.dtype
@@ -182,6 +183,11 @@ class Engine:
             return t
 
         wsi_poly = get("wsi_poly_xy", (m, 2), vt) if write_polygons else None
+        if wsi_poly is not None:
+            lo, hi = poly_xy.data_ptr(), poly_xy.data_ptr() + 2 * m * poly_xy.element_size()
+            w_lo = wsi_poly.data_ptr()
+            if w_lo < hi and lo < w_lo + wsi_poly.numel() * wsi_poly.element_size():
+                raise ValueError("out['wsi_poly_xy'] overlaps poly_xy: the vertex shift is not in place")
         wsi_c = get("wsi_centroid", (n, 2), torch.float64) if centroid is not None else None
         wsi_b = get("wsi_bbox", (n, 4), torch.int32) if bbox is not None else None
         mo = PgMorphOut()
