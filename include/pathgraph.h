@@ -457,6 +457,57 @@ int pg_local_autocorr(pg_handle* h, int32_t n, const int32_t* row_ptr, const int
                       const double* feat, int32_t flags, int32_t n_perms, uint64_t seed, const pg_local_out* out,
                       pg_stream stream);
 
+/* ---- K19: cell clusters (csrc/pg_cluster.cu): connected components and DBSCAN over a cell graph, and a table with
+ * one row per cluster - the lymphocyte aggregates, tumour nests and stroma islands a pathologist counts.
+ * pg_connected_components: any CSR, row_ptr int32 [n+1], col int32. Every entry (i, j) with j in [0, n) and j != i
+ *   joins i and j; other entries are skipped, as pg_clustering skips them. A CSR that is not symmetric gives the weak
+ *   components (scipy.sparse.csgraph.connected_components with directed=False).
+ *   label int32 [n] = the rank of the node's component in the order of the components' smallest member (scipy's
+ *   numbering); n_labels int32 [1] (device) = the components.
+ * pg_dbscan: row_ptr / col the symmetric radius CSR of the points (K6 with flags 0: d2 <= eps^2, no self entries).
+ *   d_i = the entries of row i with j in [0, n) and j != i; core_i = (d_i + 1 >= min_samples) (the point counts itself,
+ *   as in sklearn). Only entries between two core nodes join. Clusters are numbered in the order of their smallest core
+ *   node; label int32 [n] = the cluster of a core node; a non-core node takes the smallest label among its core
+ *   neighbours, -1 (noise) when it has none. core uint8 [n] = core_i. n_labels int32 [1] (device) = the clusters.
+ *   This is sklearn.cluster.DBSCAN's result exactly: its dbscan_inner visits the points in index order, starts a new
+ *   cluster at each unlabelled core point and finishes that cluster (labelling every neighbour of its core points that
+ *   has no label yet) before it starts the next. So the clusters get their labels in the order of their smallest core
+ *   point, and a border point reachable from several clusters keeps the label of the first of them to reach it: the
+ *   smallest label among its core neighbours.
+ * Both: union-find (links only ever hang a root under a smaller root, so each root ends as its component's smallest
+ *   member) and a scan of the roots; the labels do not depend on the run or the handle. Asynchronous, no host
+ *   synchronisation beyond workspace growth (12 n bytes). PG_ERR_INVALID for n < 0, min_samples < 1, NULL pointers.
+ * pg_cluster_props: the clusters 0..n_clusters-1 of label int32 [n] (n_labels of the calls above; a label outside
+ *   [0, n_clusters) belongs to no cluster); xy float64 [n][2] (16-byte aligned); type int32 [n] (types outside
+ *   1..n_types count nowhere); core uint8 [n]. Outputs per cluster c, each may be NULL:
+ *     n_members int32 [K]; n_core int32 [K] (needs core); type_count int32 [K][n_types] (needs type);
+ *     centroid float64 [K][2] = the coordinate sums / n_members, each sum taken in one fixed order over the members in
+ *       ascending node index (lane l of a warp adds members l, l + 32, ... in turn, then a shuffle tree adds the lanes);
+ *     bbox float64 [K][4] = xmin, ymin, xmax, ymax (NaN centroid and bbox for a cluster without members);
+ *     member_off int32 [K+1], member_xy float64 [M][2] (16-byte aligned, M = member_off[K] = the members): the members'
+ *       coordinates grouped by cluster in ascending node index - a polygon CSR that pg_ring_hull_f64 takes as it is.
+ *   The grouping is a stable LSD counting sort on 8-bit digits of the label; every output position follows from counts
+ *   and scans, none from the order of atomics, so the outputs do not depend on the run or the handle. Asynchronous, no
+ *   host synchronisation beyond workspace growth (8 n + 4 K bytes and 8 max(K, 256 ceil(n / 2048)) bytes); the caller knows K
+ *   from n_labels (one read-back, as pg_radius_total). PG_ERR_INVALID for n < 0, n_clusters < 0, n_types outside
+ *   1..PG_MAX_TYPES, NULL required pointers. */
+typedef struct {
+  int32_t* n_members;
+  int32_t* n_core;
+  int32_t* type_count;
+  double* centroid;
+  double* bbox;
+  int32_t* member_off;
+  double* member_xy;
+} pg_cluster_out;
+int pg_connected_components(pg_handle* h, int32_t n, const int32_t* row_ptr, const int32_t* col, int32_t* label,
+                            int32_t* n_labels, pg_stream stream);
+int pg_dbscan(pg_handle* h, int32_t n, const int32_t* row_ptr, const int32_t* col, int32_t min_samples,
+              int32_t* label, uint8_t* core, int32_t* n_labels, pg_stream stream);
+int pg_cluster_props(pg_handle* h, int32_t n, const int32_t* label, int32_t n_clusters, const double* xy,
+                     const int32_t* type, int32_t n_types, const uint8_t* core, const pg_cluster_out* out,
+                     pg_stream stream);
+
 /* ---- K12: raster region properties of an instance map (SURVEY 8f-3): what skimage regionprops gives
  * aggregated_hovernet_run.py:172-181 (bbox per instance) and hovernet_tile_inference.ipynb:2415-2429 (cell 18:
  * area, perimeter, eccentricity, major / minor axis length, orientation).  inst_map int32 [height][width], labels

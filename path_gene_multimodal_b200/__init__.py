@@ -11,7 +11,7 @@ Public surface (reference-style module-level functions; see DESIGN.md / INTEGRAT
     filter_graph_by_type, clustering_coefficients,
     type_interaction_matrix, neighbourhood_enrichment,
     co_occurrence, ripley, spatial_autocorr,
-    local_autocorr,
+    local_autocorr, connected_components, cell_clusters,
     knn_graph_frame                                       (cell_graph)
     to_networkx                                           (interop: nx.Graph keyed by nuc_id, cell 11)
     read_nuclei_table, write_nuclei_table, table_to_soa,
@@ -35,7 +35,7 @@ _EXPORTS = {
     "filter_graph_by_type": "cell_graph", "clustering_coefficients": "cell_graph",
     "type_interaction_matrix": "cell_graph", "neighbourhood_enrichment": "cell_graph",
     "co_occurrence": "cell_graph", "ripley": "cell_graph", "spatial_autocorr": "cell_graph",
-    "local_autocorr": "cell_graph",
+    "local_autocorr": "cell_graph", "connected_components": "cell_graph", "cell_clusters": "cell_graph",
     "knn_graph_frame": "cell_graph", "to_networkx": "interop",
     "edge_index_from_edges": "graph_features",
     "read_nuclei_table": "nuclei_io", "write_nuclei_table": "nuclei_io", "table_to_soa": "nuclei_io",

@@ -69,6 +69,11 @@ class PgLocalOut(C.Structure):
     _fields_ = [(name, vp) for name in ("stat", "lag", "n_ge", "perm_mean", "perm_var", "sims", "mean", "m2")]
 
 
+class PgClusterOut(C.Structure):
+    _fields_ = [(name, vp) for name in ("n_members", "n_core", "type_count", "centroid", "bbox", "member_off",
+                                        "member_xy")]
+
+
 class PathGraphError(RuntimeError):
     def __init__(self, code: int, msg: str):
         super().__init__(f"libpathgraph error {code}: {msg}")
@@ -124,6 +129,9 @@ SIGNATURES = {
     "pg_nhood_enrichment": (C.c_int, [vp, i32, vp, i32, i64, vp, i32, C.c_uint64, C.POINTER(PgEnrichOut), vp]),
     "pg_spatial_autocorr": (C.c_int, [vp, i32, vp, vp, i32, vp, i32, i32, C.c_uint64, C.POINTER(PgAutocorrOut), vp]),
     "pg_local_autocorr": (C.c_int, [vp, i32, vp, vp, i32, vp, i32, i32, C.c_uint64, C.POINTER(PgLocalOut), vp]),
+    "pg_connected_components": (C.c_int, [vp, i32, vp, vp, vp, vp, vp]),
+    "pg_dbscan": (C.c_int, [vp, i32, vp, vp, i32, vp, vp, vp, vp]),
+    "pg_cluster_props": (C.c_int, [vp, i32, vp, i32, vp, vp, i32, vp, C.POINTER(PgClusterOut), vp]),
     "pg_pair_dist_hist": (C.c_int, [vp, i32, i32, C.POINTER(f64), vp, vp, vp]),
     "pg_raster_props": (C.c_int, [vp, i32, i32, vp, i32, C.POINTER(PgRasterOut), vp]),
     "pg_raster_solidity": (C.c_int, [vp, i32, i32, vp, i32, vp, vp, vp, vp, vp]),

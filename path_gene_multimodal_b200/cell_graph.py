@@ -11,6 +11,8 @@ Mirrors /root/reference/hovernet_tile_inference.ipynb:
 * ``spatial_autocorr``: Moran's I / Geary's C of per-nucleus features over the graph (squidpy.gr.spatial_autocorr);
 * ``local_autocorr``: local Moran's I_i / Getis-Ord Gi(*) per nucleus, where a feature clusters (esda Moran_Local /
   G_Local).
+* ``connected_components`` / ``cell_clusters``: components of a cell graph (scipy.sparse.csgraph) and DBSCAN clusters of
+  nuclei of chosen types (sklearn.cluster.DBSCAN) with a per-cluster table - aggregates, nests, islands.
 
 Host arrays in, host arrays out; everything in between is libpathgraph (uniform-grid binning, grid
 queries, two-pass CSR) on the GPU.  No CPU fallback.
@@ -673,6 +675,125 @@ def local_frame(res: dict, x, names, deg, mode: str, transformation: bool, star:
         for k, v in fields.items():
             cols[(name, k)] = v
     return pd.DataFrame(cols, index=pd.RangeIndex(n, name="node"))
+
+
+def connected_components(row_ptr, col, device=None) -> tuple[int, np.ndarray]:
+    """Connected components of a cell graph (scipy.sparse.csgraph.connected_components with ``directed=False``):
+    ``(n_components, labels)``, labels int32 [N] numbering the components in the order of their smallest node.
+
+    ``row_ptr`` / ``col``: a CSR over N nodes, for example ``build_radius_graph(..., symmetric_csr=True)`` or
+    ``build_knn_graph``; it need not be symmetric (an entry in either direction joins two nodes) and self entries are
+    ignored. Union-find on the GPU (K19), so a slide-wide chain costs no more than scattered clumps. Raises
+    ``ValueError`` on a malformed CSR before anything is launched."""
+    rp, c = _csr_host(row_ptr, col)
+    eng = get_engine(device)
+    with torch.cuda.device(eng.device):
+        d_rp = _host.to_device(rp, np.int32, eng.device)
+        d_c = _host.to_device(c, np.int32, eng.device)
+        host = _host.to_host_many(eng.connected_components(d_rp, d_c))
+    return int(host["n_labels"][0]), host["labels"]
+
+
+def cell_clusters(coords, eps: float, min_samples: int = 5, types=None, keep_types=None, n_types: int = 5,
+                  mpp: float | None = None, hull: bool = True, device=None) -> dict:
+    """DBSCAN clusters of nuclei (sklearn.cluster.DBSCAN's labels, exactly) with one table row per cluster: lymphocyte
+    aggregates, tumour nests, islands of stroma.
+
+    ``coords`` float [N,2] centroids; ``mpp`` scales them to micrometres first (``x_um = x_px * mpp``), and ``eps``,
+    the centroids, boxes and areas of the result are then in micrometres. ``keep_types``: cluster only the nuclei whose
+    ``types`` value is in it (all nuclei when None). Two kept nuclei are neighbours when d <= eps (the squared-distance
+    rule of ``build_radius_graph``); a nucleus is core when it has at least ``min_samples`` kept nuclei within eps,
+    itself included; clusters are the core nuclei joined through core neighbours, numbered in the order of their
+    smallest core index, and a non-core nucleus joins the lowest-numbered cluster among its core neighbours - sklearn's
+    order of work, so a border nucleus between two clusters takes the lower label.
+
+    Returns ``labels`` int64 [N] (-1 for noise and for nuclei of types not kept), ``core`` bool [N], ``n_clusters`` and
+    ``clusters``, a DataFrame indexed by cluster with ``n_nuclei``, ``n_core``, ``centroid_x`` / ``centroid_y`` (mean of
+    the members), ``bbox_xmin``, ``bbox_ymin``, ``bbox_xmax``, ``bbox_ymax``, with ``types`` ``n_type_1`` ..
+    ``n_type_T`` (members of each type, T = ``n_types``) and with ``hull`` ``hull_area`` (area of the members' convex
+    hull: NaN below 3 members, 0 for collinear members) and ``density`` = n_nuclei / hull_area (NaN where hull_area is
+    not positive). Everything runs on the GPU: the radius CSR (K6), DBSCAN and the table (K19), the hulls (K14).
+    Raises ``ValueError`` before anything is launched on bad shapes, an ``eps`` that is negative or not finite,
+    ``min_samples`` < 1, an empty ``keep_types`` or one without ``types``, ``n_types`` outside 1..16 or an ``mpp`` that
+    is not finite and > 0; non-finite coordinates raise ``ValueError`` from the grid build."""
+    import pandas as pd
+
+    c = np.asarray(coords, dtype=np.float64)
+    if c.ndim != 2 or c.shape[1] != 2:
+        raise ValueError("coords must have shape (N, 2)")
+    n = c.shape[0]
+    if n > _host.INT32_MAX:
+        raise ValueError("more than 2^31 - 1 nuclei")
+    eps = float(eps)
+    if not (np.isfinite(eps) and eps >= 0):
+        raise ValueError("eps must be finite and >= 0")
+    if not (isinstance(min_samples, (int, np.integer)) and min_samples >= 1):
+        raise ValueError("min_samples must be an int >= 1")
+    if not 1 <= n_types <= _lib.PG_MAX_TYPES:
+        raise ValueError(f"n_types must be in 1..{_lib.PG_MAX_TYPES}")
+    if mpp is not None:
+        if not (np.isfinite(mpp) and mpp > 0):
+            raise ValueError("mpp must be finite and > 0")
+        c = c * float(mpp)
+    t = None
+    if types is not None:
+        t = _host.as_int32(types, "types").reshape(-1)
+        if t.shape[0] != n:
+            raise ValueError("types must have one entry per point")
+    sel = None
+    if keep_types is not None:
+        kt = np.asarray(list(keep_types)).reshape(-1)
+        if kt.size == 0:
+            raise ValueError("keep_types must not be empty")
+        if t is None:
+            raise ValueError("keep_types needs types")
+        sel = np.flatnonzero(np.isin(t, kt))
+        c = c[sel]
+        t = t[sel]
+    m = c.shape[0]
+    labels = np.full(n, -1, dtype=np.int64)
+    core = np.zeros(n, dtype=bool)
+    k = 0
+    props = {}
+    if m > 0:
+        eng = get_engine(device)
+        with torch.cuda.device(eng.device):
+            d_xy = _host.to_device(c, np.float64, eng.device)
+            d_t = _host.to_device(t, np.int32, eng.device) if t is not None else None
+            eng.grid_build(d_xy, None, None, radius_cell(eps), None)
+            g = eng.radius_graph(eps, upper=False, compose=False, stats=False, want_dist32=False)
+            db = eng.dbscan(g["row_ptr"], g["col"], int(min_samples))
+            host = _host.to_host_many({"labels": db["labels"], "core": db["core"], "n_labels": db["n_labels"]})
+            k = int(host["n_labels"][0])
+            sub = host["labels"]
+            pr = eng.cluster_props(db["labels"], k, d_xy, d_t, n_types, db["core"],
+                                   n_members_total=int((sub >= 0).sum()))
+            if hull:
+                pr["hull_area"] = eng.ring_hull(pr["member_off"], pr["member_xy"])["convex_area"]
+            props = _host.to_host_many({name: v for name, v in pr.items() if name not in ("member_off", "member_xy")})
+        if sel is None:
+            labels[:] = sub
+            core[:] = host["core"] != 0
+        else:
+            labels[sel] = sub
+            core[sel] = host["core"] != 0
+    cols = {"n_nuclei": props.get("n_members", np.zeros(0, np.int32)),
+            "n_core": props.get("n_core", np.zeros(0, np.int32))}
+    cen = props.get("centroid", np.zeros((0, 2)))
+    box = props.get("bbox", np.zeros((0, 4)))
+    cols.update({"centroid_x": cen[:, 0], "centroid_y": cen[:, 1], "bbox_xmin": box[:, 0], "bbox_ymin": box[:, 1],
+                 "bbox_xmax": box[:, 2], "bbox_ymax": box[:, 3]})
+    if t is not None:
+        tc = props.get("type_count", np.zeros((0, n_types), np.int32))
+        for a in range(n_types):
+            cols[f"n_type_{a + 1}"] = tc[:, a]
+    if hull:
+        area = props.get("hull_area", np.zeros(0))
+        cols["hull_area"] = area
+        with np.errstate(divide="ignore", invalid="ignore"):
+            cols["density"] = np.where(area > 0, cols["n_nuclei"] / area, np.nan)
+    df = pd.DataFrame(cols, index=pd.RangeIndex(k, name="cluster"))
+    return {"labels": labels, "core": core, "n_clusters": k, "clusters": df}
 
 
 def knn_graph_frame(final_df, k: int = 5, centroid_col: str = "centroid", centroid_order: str = "yx",

@@ -91,6 +91,11 @@ struct pg_handle {
   pg_buf lk_cnt;       // K18: int32 nodes per degree [n + 1]; the scan clears it and it becomes the scatter cursor
   pg_buf lk_off;       // K18: int32 exclusive scan of lk_cnt [n + 1]
   pg_buf lk_ord;       // K18: int32 nodes in ascending degree [n]
+  pg_buf cl_parent;    // K19 (pg_cluster.cu): int32 union-find parents [n]; the table's first LSD order buffer
+  pg_buf cl_count;     // K19: int32 is_root [n]; the table's members per cluster, then per (digit, tile)
+  pg_buf cl_scan;      // K19: int32 exclusive scans of cl_count
+  pg_buf cl_order;     // K19: int32 [n] the table's second LSD order buffer
+  pg_buf cl_off;       // K19: int32 [K + 1] first member slot of each cluster
   // launch accounting / optional per-kernel CUDA-event timing (pg_profile_*)
   int64_t launches = 0;
   bool profiling = false;

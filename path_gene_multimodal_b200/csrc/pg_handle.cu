@@ -126,7 +126,8 @@ int pg_destroy(pg_handle* h) {
   pg_buf* bufs[] = {&h->cell_count, &h->cell_start, &h->cell_of, &h->rank,      &h->s_rec,     &h->s_pos,     &h->s_gid,     &h->knn_retry,     &h->pt_meta,   &h->tmp_ent,   &h->row_off,
                     &h->row_count,  &h->scan_state, &h->misc,    &h->sym_extra, &h->sym_cursor, &h->sym_recip, &h->hull,
                     &h->enrich_lab, &h->enrich_cnt, &h->ac_z,    &h->ac_idx,    &h->ac_deg,     &h->ac_sims,    &h->ac_part,
-                    &h->ac_misc,    &h->lk_cnt,     &h->lk_off,  &h->lk_ord};
+                    &h->ac_misc,    &h->lk_cnt,     &h->lk_off,  &h->lk_ord,
+                    &h->cl_parent,  &h->cl_count,   &h->cl_scan, &h->cl_order,  &h->cl_off};
   for (pg_buf* b : bufs)
     if (b->p) cudaFree(b->p);
   if (h->pinned) cudaFreeHost(h->pinned);
@@ -142,7 +143,8 @@ int64_t pg_workspace_bytes(pg_handle* h) {
   pg_buf* bufs[] = {&h->cell_count, &h->cell_start, &h->cell_of, &h->rank,      &h->s_rec,     &h->s_pos,     &h->s_gid,     &h->knn_retry,     &h->pt_meta,   &h->tmp_ent,   &h->row_off,
                     &h->row_count,  &h->scan_state, &h->misc,    &h->sym_extra, &h->sym_cursor, &h->sym_recip, &h->hull,
                     &h->enrich_lab, &h->enrich_cnt, &h->ac_z,    &h->ac_idx,    &h->ac_deg,     &h->ac_sims,    &h->ac_part,
-                    &h->ac_misc,    &h->lk_cnt,     &h->lk_off,  &h->lk_ord};
+                    &h->ac_misc,    &h->lk_cnt,     &h->lk_off,  &h->lk_ord,
+                    &h->cl_parent,  &h->cl_count,   &h->cl_scan, &h->cl_order,  &h->cl_off};
   int64_t t = 0;
   for (pg_buf* b : bufs) t += (int64_t)b->cap;
   return t;

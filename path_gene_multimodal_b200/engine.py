@@ -675,6 +675,63 @@ class Engine:
                                                self._stream()))
         return res
 
+    # ---- K19 -----------------------------------------------------------------------------------
+    def connected_components(self, row_ptr, col):
+        """Weak connected components of a CSR (pg_connected_components): entries outside [0, N) and self entries are
+        skipped. Returns ``labels`` int32 [N] (components ranked by their smallest member, scipy's numbering) and
+        ``n_labels`` int32 [1], device tensors. Asynchronous (no host synchronisation once the workspace has grown)."""
+        n = int(row_ptr.numel()) - 1
+        res = {"labels": self._empty((n,), torch.int32), "n_labels": self._empty((1,), torch.int32)}
+        if col is None or col.numel() == 0:  # no entries: the C entry still wants a col array it will not read
+            col = self._empty((1,), torch.int32)
+        self._check(self.lib.pg_connected_components(self._h, n, self._p(row_ptr, torch.int32, "row_ptr"),
+                                                     self._p(col, torch.int32, "col"),
+                                                     self._p(res["labels"], torch.int32, "labels"),
+                                                     self._p(res["n_labels"], torch.int32, "n_labels"), self._stream()))
+        return res
+
+    def dbscan(self, row_ptr, col, min_samples=5):
+        """DBSCAN over a symmetric radius CSR (pg_dbscan): a node is core when its neighbours + 1 >= ``min_samples``.
+        Returns ``labels`` int32 [N] (-1 noise; sklearn.cluster.DBSCAN's labels), ``core`` uint8 [N] and ``n_labels``
+        int32 [1], device tensors. Asynchronous (no host synchronisation once the workspace has grown)."""
+        n = int(row_ptr.numel()) - 1
+        res = {"labels": self._empty((n,), torch.int32), "core": self._empty((n,), torch.uint8),
+               "n_labels": self._empty((1,), torch.int32)}
+        if col is None or col.numel() == 0:
+            col = self._empty((1,), torch.int32)
+        self._check(self.lib.pg_dbscan(self._h, n, self._p(row_ptr, torch.int32, "row_ptr"),
+                                       self._p(col, torch.int32, "col"), int(min_samples),
+                                       self._p(res["labels"], torch.int32, "labels"),
+                                       self._p(res["core"], torch.uint8, "core"),
+                                       self._p(res["n_labels"], torch.int32, "n_labels"), self._stream()))
+        return res
+
+    def cluster_props(self, labels, n_clusters, xy, types=None, n_types=5, core=None, n_members_total=None):
+        """Per-cluster table of clusters 0..n_clusters-1 of ``labels`` int32 [N] (pg_cluster_props); xy float64 [N,2],
+        types int32 [N], core uint8 [N]. Returns device tensors n_members int32 [K], n_core int32 [K] (with ``core``),
+        type_count int32 [K,T] (with ``types``), centroid float64 [K,2], bbox float64 [K,4] (xmin, ymin, xmax, ymax),
+        member_off int32 [K+1] and member_xy float64 [M,2], the members' coordinates grouped by cluster in ascending
+        node index (a polygon CSR for ``ring_hull``). ``n_members_total``: M, the nodes with a label in [0, K), when
+        the caller knows it; else member_xy has N rows and only the first member_off[K] are written."""
+        n = int(labels.numel())
+        k = int(n_clusters)
+        m = n if n_members_total is None else int(n_members_total)
+        res = {"n_members": self._empty((k,), torch.int32), "centroid": self._empty((k, 2), torch.float64),
+               "bbox": self._empty((k, 4), torch.float64), "member_off": self._empty((k + 1,), torch.int32),
+               "member_xy": self._empty((m, 2), torch.float64)}
+        if core is not None:
+            res["n_core"] = self._empty((k,), torch.int32)
+        if types is not None:
+            res["type_count"] = self._empty((k, int(n_types)), torch.int32)
+        co = _lib.PgClusterOut()
+        for name, t in res.items():
+            setattr(co, name, self._p(t, t.dtype, name))
+        self._check(self.lib.pg_cluster_props(self._h, n, self._p(labels, torch.int32, "labels"), k,
+                                              self._p(xy, torch.float64, "xy"), self._p(types, torch.int32, "types"),
+                                              int(n_types), self._p(core, torch.uint8, "core"), C.byref(co),
+                                              self._stream()))
+        return res
+
     # ---- K16 -----------------------------------------------------------------------------------
     def pair_dist_hist(self, thresholds, n_types=5):
         """Type-pair distance histogram over the built grid (pg_pair_dist_hist).
