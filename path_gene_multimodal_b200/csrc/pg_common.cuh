@@ -134,21 +134,12 @@ struct pg_kernel_scope {
 #define PG_MISC_TMPCUR 192    // uint64 allocation cursor of tmp_ent's overflow region (zero between count passes: the row pass moves it to TOTALS[4..5])
 #define PG_MISC_SUM64 200     // int64: 64-bit total of the last pg_scan_i32_total (copied to pinned[12..13])
 #define PG_MISC_PAIRHIST_TICKET 208  // uint64: point cursor of pair_hist_kernel's CTAs (zeroed before each launch)
-#define PG_MISC_FEAT_TICKET 4608  // uint32 [PG_FEAT_MAX_COLS] CTA tickets of feature_stats_kernel, one per column (zero between launches)
+#define PG_MISC_FEAT_TICKET 8704  // uint32 [PG_FEAT_MAX_COLS] CTA tickets of feature_stats_kernel, one per column (zero between launches)
 #define PG_FEAT_MAX_COLS 256
-#define PG_MISC_ACC 256       // pg_stats_acc: degree-statistics accumulators kept in their reset state
+#define PG_MISC_ACC 256       // pg_stats_acc: degree-statistics accumulators (all zero between launches; pg_degree.cuh)
 #define PG_MISC_ACC_HIST 512  // int32 [PG_ACC_HIST_MAX] histogram accumulators (all zero between launches)
-#define PG_ACC_HIST_MAX 1024
+#define PG_ACC_HIST_MAX 2048
 #define PG_MISC_BYTES (PG_MISC_FEAT_TICKET + 4 * PG_FEAT_MAX_COLS)
-
-// accumulators behind the fused degree statistics: every CTA adds its share, the last CTA to finish
-// copies them to the caller's pg_degree_stats / hist and puts them back into the reset state, so no
-// separate init / finish launches are needed.
-struct pg_stats_acc {
-  int32_t min_degree, max_degree;
-  unsigned long long sum_degree, sumsq_degree, n_nodes;
-  unsigned int done;  // CTAs finished
-};
 
 int pg_set_error(pg_handle* h, int code, const char* fmt, ...);
 // after a stream synchronisation that followed the copy of PG_MISC_BADINPUT into h->pinned[8]
@@ -188,16 +179,8 @@ static inline cudaError_t pg_launch_pdl(int tag, void (*kernel)(KArgs...), int g
 // internal scan entry (pg_scan.cu): out[0..n] exclusive prefix of in[0..n), out[n] = total
 // total_copy (optional): a second device location that also receives the total
 // clear_in: zero in[0..n) while reading it (the buffer must then be writable)
-// publish: degree statistics to hand to the caller from the scan's first CTA (see pg_radius.cu)
-struct pg_scan_publish {
-  pg_stats_acc* acc = nullptr;   // NULL: no statistics to publish
-  int32_t* acc_hist = nullptr;
-  pg_degree_stats* stats = nullptr;
-  int32_t* hist = nullptr;  // NULL: no histogram to publish
-  int32_t hist_len = 0;
-};
 int pg_scan_i32(pg_handle* h, const int32_t* in, int32_t* out, int32_t n, cudaStream_t s, int32_t* total_copy = nullptr,
-                bool clear_in = false, const pg_scan_publish* publish = nullptr);
+                bool clear_in = false);
 // pg_scan_i32 of non-negative counts whose total the host needs: the total is also summed in 64 bits and read back
 // into *total (synchronises the stream). PG_ERR_INVALID, naming `what`, when it is past INT32_MAX: the int32
 // offsets would have wrapped.

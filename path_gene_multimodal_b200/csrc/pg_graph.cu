@@ -4,6 +4,7 @@
 // :2969-2975 (i<j edge list); composition / degree per SURVEY A.5 (README.md:127,136).
 #include <algorithm>
 #include <cstring>
+#include "pg_degree.cuh"
 #include "pg_query.cuh"
 
 namespace {
@@ -210,8 +211,7 @@ struct rank_extra {
   int n_types;
   int32_t* nbr_count;      // [n][n_types]
   int32_t* degree;
-  pg_degree_stats* stats; int32_t* hist; int hist_len;
-  pg_stats_acc* acc; int32_t* acc_hist;
+  pg_degree_out deg;
   bool sym_dist;           // the lists' distances are symmetric bit for bit: no reverse read for the min
 };
 
@@ -222,15 +222,11 @@ sym_rank_kernel(const int32_t* __restrict__ knn_idx, const DT* __restrict__ dist
                 const int32_t* __restrict__ row_ptr, const int32_t* __restrict__ tmp_col,
                 const DT* __restrict__ tmp_w, int32_t* __restrict__ col, double* __restrict__ w64,
                 float* __restrict__ w32, rank_extra x) {
+  using DG = pg_degree_cta<TPB>;
   __shared__ int s_cnt[TPB / 32][32 * PG_MAX_TYPES];
-  __shared__ int s_hist[PG_ACC_HIST_MAX];
-  __shared__ int s_mn, s_mx, s_last;
-  __shared__ unsigned long long s_sum, s_sq;
-  const bool want_stats = x.stats != nullptr || x.hist != nullptr;
-  if (want_stats) {  // CTA-wide state: before any warp may leave
-    if (x.hist && x.hist_len <= PG_ACC_HIST_MAX)
-      for (int i = threadIdx.x; i < x.hist_len; i += TPB) s_hist[i] = 0;
-    if (threadIdx.x == 0) { s_mn = 0x7fffffff; s_mx = -1; s_sum = 0; s_sq = 0; }
+  __shared__ DG::smem_t s_deg;
+  if (DG::on(x.deg)) {  // CTA-wide state: before any warp may leave
+    DG::arm(s_deg, x.deg);
     __syncthreads();
   }
   constexpr int KK = K ? K : 4;
@@ -361,58 +357,12 @@ sym_rank_kernel(const int32_t* __restrict__ knn_idx, const DT* __restrict__ dist
     for (int i = lane; i < rows_here * x.n_types; i += 32) x.nbr_count[(int64_t)r0 * x.n_types + i] = wcnt[i];
   }
   if (x.degree && r0 + lane < n) x.degree[r0 + lane] = my_cnt;
-  if (!want_stats) return;
-  // ---- degree statistics: thread -> warp -> CTA -> accumulators; the last CTA publishes them and re-arms
-  {
-    const bool have = r0 + lane < n;
-    const int d = have ? my_cnt : 0;
-    int mn = have ? d : 0x7fffffff, mx = have ? d : -1;
-    long long sum = d, sq = (long long)d * d;
-    if (x.hist) {
-      const int bin = have ? min(d, x.hist_len - 1) : -1;
-      const unsigned peers = __match_any_sync(0xffffffffu, bin);
-      if (bin >= 0 && lane == __ffs(peers) - 1) {
-        if (x.hist_len <= PG_ACC_HIST_MAX) atomicAdd(&s_hist[bin], __popc(peers));
-        else atomicAdd(&x.hist[bin], __popc(peers));
-      }
-    }
-    mn = __reduce_min_sync(0xffffffffu, mn);
-    mx = __reduce_max_sync(0xffffffffu, mx);
-#pragma unroll
-    for (int dd = 16; dd > 0; dd >>= 1) { sum += __shfl_xor_sync(0xffffffffu, sum, dd); sq += __shfl_xor_sync(0xffffffffu, sq, dd); }
-    if (lane == 0) {
-      atomicMin(&s_mn, mn); atomicMax(&s_mx, mx);
-      atomicAdd(&s_sum, (unsigned long long)sum); atomicAdd(&s_sq, (unsigned long long)sq);
-    }
-  }
+  if (!DG::on(x.deg)) return;
+  DG dg(s_deg, x.deg);
+  dg.add(my_cnt, r0 + lane < n);
+  dg.commit();
   __syncthreads();
-  if (threadIdx.x == 0) {
-    atomicMin(&x.acc->min_degree, s_mn); atomicMax(&x.acc->max_degree, s_mx);
-    atomicAdd(&x.acc->sum_degree, s_sum); atomicAdd(&x.acc->sumsq_degree, s_sq);
-  }
-  if (x.hist && x.hist_len <= PG_ACC_HIST_MAX)
-    for (int i = threadIdx.x; i < x.hist_len; i += TPB)
-      if (s_hist[i]) atomicAdd(&x.acc_hist[i], s_hist[i]);
-  __threadfence();
-  __syncthreads();
-  if (threadIdx.x == 0) s_last = atomicAdd(&x.acc->done, 1u) == gridDim.x - 1;
-  __syncthreads();
-  if (!s_last) return;
-  __threadfence();
-  if (x.hist && x.hist_len <= PG_ACC_HIST_MAX)
-    for (int i = threadIdx.x; i < x.hist_len; i += TPB) {
-      x.hist[i] = *(volatile int32_t*)&x.acc_hist[i];
-      x.acc_hist[i] = 0;
-    }
-  if (threadIdx.x == 0) {
-    volatile pg_stats_acc* a = x.acc;
-    if (x.stats) {
-      x.stats->min_degree = n > 0 ? a->min_degree : 0; x.stats->max_degree = n > 0 ? a->max_degree : 0;
-      x.stats->sum_degree = (long long)a->sum_degree; x.stats->sumsq_degree = (long long)a->sumsq_degree;
-      x.stats->n_nodes = n;
-    }
-    a->min_degree = 0x7fffffff; a->max_degree = -1; a->sum_degree = 0; a->sumsq_degree = 0; a->n_nodes = 0; a->done = 0;
-  }
+  dg.finish(n);
 }
 
 // rows are ascending by column: entries above the row's own id start at the first col > id
@@ -473,19 +423,15 @@ upper_fill_kernel(const int32_t* __restrict__ row_ptr, const int32_t* __restrict
 }
 
 // ---- K8 over a CSR ------------------------------------------------------------------------
-constexpr int HIST_SMEM_MAX = 2048;
-
 template <int TMAX>
 __global__ void __launch_bounds__(TPB)
 compose_kernel(const int32_t* __restrict__ row_ptr, const int32_t* __restrict__ col,
                const int32_t* __restrict__ type, int n, int n_types, int32_t* __restrict__ nbr_count,
-               int32_t* __restrict__ degree, pg_degree_stats* stats, int32_t* hist, int hist_len) {
-  extern __shared__ int s_hist[];
-  __shared__ int s_mn[TPB / 32], s_mx[TPB / 32], s_cnt[TPB / 32];
-  __shared__ long long s_sum[TPB / 32], s_sq[TPB / 32];
-  const bool use_smem_hist = hist != nullptr && hist_len <= HIST_SMEM_MAX;
-  if (use_smem_hist) {
-    for (int i = threadIdx.x; i < hist_len; i += TPB) s_hist[i] = 0;
+               int32_t* __restrict__ degree, pg_degree_out dout) {
+  using DG = pg_degree_cta<TPB>;
+  __shared__ DG::smem_t s_deg;
+  if (DG::on(dout)) {
+    DG::arm(s_deg, dout);
     __syncthreads();
   }
   const int i = blockIdx.x * TPB + threadIdx.x;
@@ -508,53 +454,13 @@ compose_kernel(const int32_t* __restrict__ row_ptr, const int32_t* __restrict__ 
         if (t < n_types) nbr_count[(int64_t)i * n_types + t] = tc[t];
     }
     if (degree) degree[i] = deg;
-    if (hist) {
-      const int bin = min(deg, hist_len - 1);
-      if (use_smem_hist) atomicAdd(&s_hist[bin], 1); else atomicAdd(&hist[bin], 1);
-    }
   }
-  if (stats) {
-    int mn = valid ? deg : 0x7fffffff, mx = valid ? deg : -1, cnt = valid ? 1 : 0;
-    long long sum = valid ? deg : 0, sq = valid ? (long long)deg * deg : 0;
-#pragma unroll
-    for (int d = 16; d > 0; d >>= 1) {
-      mn = min(mn, __shfl_xor_sync(0xffffffffu, mn, d));
-      mx = max(mx, __shfl_xor_sync(0xffffffffu, mx, d));
-      sum += __shfl_xor_sync(0xffffffffu, sum, d);
-      sq += __shfl_xor_sync(0xffffffffu, sq, d);
-      cnt += __shfl_xor_sync(0xffffffffu, cnt, d);
-    }
-    const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
-    if (lane == 0) { s_mn[warp] = mn; s_mx[warp] = mx; s_sum[warp] = sum; s_sq[warp] = sq; s_cnt[warp] = cnt; }
-    __syncthreads();
-    if (threadIdx.x == 0) {
-      for (int w = 1; w < TPB / 32; ++w) {
-        mn = min(mn, s_mn[w]); mx = max(mx, s_mx[w]); sum += s_sum[w]; sq += s_sq[w]; cnt += s_cnt[w];
-      }
-      if (cnt > 0) {
-        atomicMin(&stats->min_degree, mn);
-        atomicMax(&stats->max_degree, mx);
-        atomicAdd((unsigned long long*)&stats->sum_degree, (unsigned long long)sum);
-        atomicAdd((unsigned long long*)&stats->sumsq_degree, (unsigned long long)sq);
-        atomicAdd((unsigned long long*)&stats->n_nodes, (unsigned long long)cnt);
-      }
-    }
-  }
-  if (use_smem_hist) {
-    __syncthreads();
-    for (int b = threadIdx.x; b < hist_len; b += TPB) {
-      const int c = s_hist[b];
-      if (c) atomicAdd(&hist[b], c);
-    }
-  }
-}
-
-__global__ void init_stats_kernel(pg_degree_stats* stats) {
-  stats->min_degree = 0x7fffffff; stats->max_degree = -1;
-  stats->sum_degree = 0; stats->sumsq_degree = 0; stats->n_nodes = 0;
-}
-__global__ void finish_stats_kernel(pg_degree_stats* stats) {
-  if (stats->n_nodes == 0) { stats->min_degree = 0; stats->max_degree = 0; }
+  if (!DG::on(dout)) return;
+  DG dg(s_deg, dout);
+  dg.add(deg, valid);
+  dg.commit();
+  __syncthreads();
+  dg.finish(n);
 }
 
 // ---- K11 graph statistics named by the reference (README.md:136 "degree, clustering, centrality"; SURVEY 8f-4)
@@ -700,15 +606,12 @@ int pg_knn_union_fill(pg_handle* h, int32_t n, int32_t k, const int32_t* knn_idx
              "pg_knn_union_fill: nbr_count needs type and 1 <= n_types <= %d", PG_MAX_TYPES);
   PG_REQUIRE(h, !x.hist || x.hist_len >= 1, "pg_knn_union_fill: hist_len must be >= 1");
   PG_REQUIRE(h, ((uintptr_t)x.edges & 15) == 0, "pg_knn_union_fill: edges must be 16-byte aligned");
-  if (x.hist && (n == 0 || x.hist_len > PG_ACC_HIST_MAX)) PG_CUDA(h, cudaMemsetAsync(x.hist, 0, (size_t)x.hist_len * sizeof(int32_t), s));
-  if (n == 0) {
-    if (x.stats) PG_CUDA(h, cudaMemsetAsync(x.stats, 0, sizeof(pg_degree_stats), s));
-    return PG_OK;
-  }
+  rank_extra rx{};
+  int rc = pg_degree_prepare(h, x.stats, x.hist, x.hist_len, n, s, &rx.deg);
+  if (rc || n == 0) return rc;
   // the total of the matching count pass sizes the staging rows - or, for a caller that has sized its own outputs by
   // their bound and wants no host synchronisation at all, the bound does (every list entry yields at most two entries)
   int64_t total = 0;
-  int rc;
   if (x.presized) {
     total = 2 * (int64_t)n * k;
   } else if ((rc = pg_knn_union_total(h, &total, nullptr))) {
@@ -721,15 +624,12 @@ int pg_knn_union_fill(pg_handle* h, int32_t n, int32_t k, const int32_t* knn_idx
   if ((rc = pg_reserve(h, tw, ((size_t)total + 4) * sizeof(double)))) return rc;
   int32_t* cursor = (int32_t*)h->sym_extra.p;  // all zero since the count pass's scan
   const uint8_t* recip = (const uint8_t*)h->sym_recip.p;
-  rank_extra rx{};
   rx.row_id = row_id;
   rx.up_ptr = (x.edges || x.edge_w64 || x.edge_w32) ? up_row_ptr : nullptr;
   rx.edges = (long long*)x.edges; rx.ew64 = x.edge_w64; rx.ew32 = x.edge_w32;
   rx.type = x.type; rx.n_types = x.nbr_count ? x.n_types : 1; rx.nbr_count = x.nbr_count;
-  rx.degree = x.degree; rx.stats = x.stats; rx.hist = x.hist; rx.hist_len = x.hist_len;
+  rx.degree = x.degree;
   rx.sym_dist = x.symmetric_dist != 0;
-  rx.acc = (pg_stats_acc*)((char*)h->misc.p + PG_MISC_ACC);
-  rx.acc_hist = (int32_t*)((char*)h->misc.p + PG_MISC_ACC_HIST);
   const int blocks = pg_div_up(n, TPB);
   const bool vec = (((uintptr_t)knn_idx | (uintptr_t)dist64 | (uintptr_t)dist32) & 15) == 0;
 #define PG_PUSH(DT, D, K) PG_LAUNCH(h, s, "sym_push_kernel", sym_push_kernel<DT, K><<<blocks, TPB, 0, s>>>(knn_idx, D, n, k, row_id, id_map, recip, und_row_ptr, cursor, (int32_t*)tcol.p, (DT*)tw.p))
@@ -819,17 +719,13 @@ int pg_compose_degree(pg_handle* h, int32_t n, const int32_t* row_ptr, const int
   PG_REQUIRE(h, !nbr_count || (type && col && n_types >= 1 && n_types <= PG_MAX_TYPES),
              "pg_compose_degree: nbr_count needs type, col and 1 <= n_types <= %d", PG_MAX_TYPES);
   PG_REQUIRE(h, !hist || hist_len >= 1, "pg_compose_degree: hist_len must be >= 1");
-  if (stats) PG_LAUNCH(h, s, "init_stats_kernel", init_stats_kernel<<<1, 1, 0, s>>>(stats));
-  if (hist) PG_CUDA(h, cudaMemsetAsync(hist, 0, (size_t)hist_len * sizeof(int32_t), s));
-  if (n > 0) {
-    const size_t smem = (hist && hist_len <= HIST_SMEM_MAX) ? (size_t)hist_len * sizeof(int) : 0;
-    if (!nbr_count || n_types <= 8)
-      PG_LAUNCH(h, s, "compose_kernel<8>", compose_kernel<8><<<pg_div_up(n, TPB), TPB, smem, s>>>(row_ptr, col, type, n, n_types, nbr_count, degree, stats, hist, hist_len));
-    else
-      PG_LAUNCH(h, s, "compose_kernel<16>", compose_kernel<16><<<pg_div_up(n, TPB), TPB, smem, s>>>(row_ptr, col, type, n, n_types, nbr_count, degree, stats, hist, hist_len));
-    PG_LAUNCH_CHECK(h);
-  }
-  if (stats) PG_LAUNCH(h, s, "finish_stats_kernel", finish_stats_kernel<<<1, 1, 0, s>>>(stats));
+  pg_degree_out dout;
+  int rc = pg_degree_prepare(h, stats, hist, hist_len, n, s, &dout);
+  if (rc || n == 0) return rc;
+  if (!nbr_count || n_types <= 8)
+    PG_LAUNCH(h, s, "compose_kernel<8>", compose_kernel<8><<<pg_div_up(n, TPB), TPB, 0, s>>>(row_ptr, col, type, n, n_types, nbr_count, degree, dout));
+  else
+    PG_LAUNCH(h, s, "compose_kernel<16>", compose_kernel<16><<<pg_div_up(n, TPB), TPB, 0, s>>>(row_ptr, col, type, n, n_types, nbr_count, degree, dout));
   PG_LAUNCH_CHECK(h);
   return PG_OK;
 }

@@ -100,12 +100,6 @@ int pg_create(int device, pg_handle** out) {
   int rc = pg_reserve(h, h->misc, PG_MISC_BYTES);
   if (rc == PG_OK) {
     e = cudaMemset(h->misc.p, 0, PG_MISC_BYTES);
-    if (e == cudaSuccess) {  // reset state of the statistics accumulators: min = INT_MAX, max = -1, sums 0
-      pg_stats_acc acc{};
-      acc.min_degree = 0x7fffffff;
-      acc.max_degree = -1;
-      e = cudaMemcpy((char*)h->misc.p + PG_MISC_ACC, &acc, sizeof(acc), cudaMemcpyHostToDevice);
-    }
     if (e != cudaSuccess) rc = pg_set_error(nullptr, PG_ERR_CUDA, "cudaMemset: %s", cudaGetErrorString(e));
   } else {
     g_create_error = h->err;

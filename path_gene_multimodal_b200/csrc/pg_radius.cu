@@ -19,7 +19,7 @@
 //   rows   (pg_radius_count, kernel 2) one thread per 4 ROWS: reads their meta records (contiguous 256-bit loads)
 //          and writes row_ptr (decoupled look-back scan of the entry
 //          counts), degree, nbr_count and row_off coalesced; the degree statistics / histogram are reduced
-//          here too (CTA -> accumulators; the last CTA publishes them and re-arms the accumulators).
+//          here too (pg_degree.cuh: the last CTA publishes them).
 //   gather (pg_radius_fill) warp-flattened over 32 rows: lane p of the warp's contiguous output range finds its
 //          row by a 5-step shuffle search, reads one parked entry, ranks it among the row's entries by counting
 //          smaller ids (rows are short; ids are distinct) and writes col / dist / edges fully coalesced.
@@ -27,6 +27,7 @@
 #include <cmath>
 #include <cstring>
 #include <algorithm>
+#include "pg_degree.cuh"
 #include "pg_query.cuh"
 #include "pg_scan.cuh"
 
@@ -341,11 +342,7 @@ struct rows_out {
   int32_t* __restrict__ nbr_count;   // NULL when not wanted or when the walk wrote it (wide types)
   int32_t* __restrict__ row_off;
   int n_types;
-  pg_degree_stats* stats;
-  int32_t* hist;
-  int hist_len, hist_mode;           // 0 none, 1 shared-memory bins -> accumulators, 2 straight into hist (pre-zeroed)
-  pg_stats_acc* acc;
-  int32_t* acc_hist;
+  pg_degree_out deg;
   int32_t* total_copy;
   unsigned long long* ovf_cursor;    // retired here: *ovf_needed = *ovf_cursor; *ovf_cursor = 0
   unsigned long long* ovf_needed;
@@ -367,14 +364,12 @@ template <bool GATHER>
 __global__ void __launch_bounds__(TPB_ROWS)
 radius_rows_kernel(int n_query, const pg_pt_meta* meta, pg_scan_state st, rows_out o, rows_gather gx) {
   using TS = pg_tile_scan<TPB_ROWS>;
+  using DG = pg_degree_cta<TPB_ROWS>;
   __shared__ typename TS::smem_t sm;
   __shared__ int s_rp[GATHER ? ROWS_TILE + 1 : 1];
   __shared__ int s_off[GATHER ? ROWS_TILE : 1];
-  __shared__ int s_hist[PG_ACC_HIST_MAX];
-  __shared__ int s_mn, s_mx, s_last;
-  __shared__ unsigned long long s_sum, s_sq;
+  __shared__ typename DG::smem_t s_deg;
   const int tid = threadIdx.x;
-  const bool want_stats = o.stats != nullptr || o.hist_mode != 0;
   pg_pdl_launch();
   pg_pdl_wait();
   const int tile = TS::take_tile(sm, st);  // a ticket, not blockIdx.x: a tile then only waits on tiles that are already running
@@ -382,9 +377,7 @@ radius_rows_kernel(int n_query, const pg_pt_meta* meta, pg_scan_state st, rows_o
   const bool full = row0 + ROWS_ITEMS <= n_query;
 
   pg_pt_meta m[ROWS_ITEMS];
-  if (o.hist_mode == 1)
-    for (int i = tid; i < o.hist_len; i += TPB_ROWS) s_hist[i] = 0;
-  if (tid == 0) { s_mn = 0x7fffffff; s_mx = -1; s_sum = 0; s_sq = 0; }
+  DG::arm(s_deg, o.deg);
 #pragma unroll
   for (int i = 0; i < ROWS_ITEMS; ++i) {
     if (row0 + i < n_query) m[i] = ld_meta(meta + row0 + i);
@@ -394,7 +387,8 @@ radius_rows_kernel(int n_query, const pg_pt_meta* meta, pg_scan_state st, rows_o
 #pragma unroll
   for (int i = 0; i < ROWS_ITEMS; ++i) { v[i] = tsum; tsum += m[i].cnt; }
   int tile_sum;
-  const int thread_off = TS::local_scan(sm, st, tile, tsum, &tile_sum);  // barrier inside: the shared accumulators are ready
+  const int thread_off = TS::local_scan(sm, st, tile, tsum, &tile_sum);  // barrier inside: the shared statistics are armed
+  DG dg(s_deg, o.deg);
 
   // ---- everything that does not need the tile's prefix: row_off, degree, type counts, statistics
   if (full) {
@@ -430,37 +424,9 @@ radius_rows_kernel(int n_query, const pg_pt_meta* meta, pg_scan_state st, rows_o
       }
     }
   }
-  if (want_stats) {  // thread -> warp -> CTA
-    int mn = 0x7fffffff, mx = -1;
-    long long sum = 0, sq = 0;
 #pragma unroll
-    for (int i = 0; i < ROWS_ITEMS; ++i) {
-      if (row0 + i < n_query) {
-        const int d = m[i].deg;
-        mn = min(mn, d); mx = max(mx, d); sum += d; sq += (long long)d * d;
-      }
-    }
-    if (o.hist_mode != 0) {
-      // degrees cluster on a few bins: one atomic per distinct bin of the warp instead of one per lane
-#pragma unroll
-      for (int i = 0; i < ROWS_ITEMS; ++i) {
-        const int bin = row0 + i < n_query ? min(m[i].deg, o.hist_len - 1) : -1;
-        const unsigned int peers = __match_any_sync(0xffffffffu, bin);
-        if (bin >= 0 && (tid & 31) == __ffs(peers) - 1) {
-          if (o.hist_mode == 1) atomicAdd(&s_hist[bin], __popc(peers));
-          else atomicAdd(&o.hist[bin], __popc(peers));
-        }
-      }
-    }
-    mn = __reduce_min_sync(0xffffffffu, mn);
-    mx = __reduce_max_sync(0xffffffffu, mx);
-#pragma unroll
-    for (int d = 16; d > 0; d >>= 1) { sum += __shfl_xor_sync(0xffffffffu, sum, d); sq += __shfl_xor_sync(0xffffffffu, sq, d); }
-    if ((tid & 31) == 0) {
-      atomicMin(&s_mn, mn); atomicMax(&s_mx, mx);
-      atomicAdd(&s_sum, (unsigned long long)sum); atomicAdd(&s_sq, (unsigned long long)sq);
-    }
-  }
+  for (int i = 0; i < ROWS_ITEMS; ++i) dg.add(m[i].deg, row0 + i < n_query);
+  dg.commit();
 
   // ---- the prefix of the tile (barrier inside: the CTA's statistics are complete after it)
   bool last;
@@ -496,50 +462,18 @@ radius_rows_kernel(int n_query, const pg_pt_meta* meta, pg_scan_state st, rows_o
     }
   }
 
-  // ---- CTA -> accumulators; the last CTA to get here publishes them and re-arms the accumulators
-  if (want_stats) {
-    if (tid == 0) {
-      atomicMin(&o.acc->min_degree, s_mn); atomicMax(&o.acc->max_degree, s_mx);
-      atomicAdd(&o.acc->sum_degree, s_sum); atomicAdd(&o.acc->sumsq_degree, s_sq);
-    }
-    if (o.hist_mode == 1)
-      for (int i = tid; i < o.hist_len; i += TPB_ROWS)
-        if (s_hist[i]) atomicAdd(&o.acc_hist[i], s_hist[i]);
-  }
-  __threadfence();
-  __syncthreads();
-  if (tid == 0) s_last = atomicAdd(&o.acc->done, 1u) == (unsigned int)st.num_tiles - 1;
-  __syncthreads();
-  if (!s_last) return;
-  __threadfence();
-  if (o.hist_mode == 1)
-    for (int i = tid; i < o.hist_len; i += TPB_ROWS) {
-      o.hist[i] = *(volatile int32_t*)&o.acc_hist[i];
-      o.acc_hist[i] = 0;
-    }
-  if (tid == 0) {
-    volatile pg_stats_acc* a = o.acc;
-    if (o.stats) {
-      o.stats->min_degree = a->min_degree; o.stats->max_degree = a->max_degree;
-      o.stats->sum_degree = (long long)a->sum_degree; o.stats->sumsq_degree = (long long)a->sumsq_degree;
-      o.stats->n_nodes = n_query;
-    }
-    a->min_degree = 0x7fffffff; a->max_degree = -1; a->sum_degree = 0; a->sumsq_degree = 0; a->n_nodes = 0; a->done = 0;
-    if (o.ovf_cursor) { *o.ovf_needed = *(volatile unsigned long long*)o.ovf_cursor; *o.ovf_cursor = 0ull; }
+  // ---- CTA -> accumulators; the last CTA to get here publishes the statistics and retires the overflow cursor
+  if (dg.finish(n_query) && tid == 0 && o.ovf_cursor) {
+    *o.ovf_needed = *(volatile unsigned long long*)o.ovf_cursor;
+    *o.ovf_cursor = 0ull;
   }
 }
 
-// nothing to query: empty row_ptr and the statistics of an empty graph
-__global__ void empty_graph_kernel(int32_t* row_ptr, int32_t* total_copy, pg_degree_stats* stats, int32_t* hist, int hist_len,
-                                   unsigned long long* ovf_needed) {
-  if (threadIdx.x == 0) {
-    row_ptr[0] = 0;
-    *total_copy = 0;
-    *ovf_needed = 0;
-    if (stats) { stats->min_degree = 0; stats->max_degree = 0; stats->sum_degree = 0; stats->sumsq_degree = 0; stats->n_nodes = 0; }
-  }
-  if (hist)
-    for (int i = threadIdx.x; i < hist_len; i += blockDim.x) hist[i] = 0;
+// nothing to query: empty row_ptr (the statistics of the empty graph come from pg_degree_prepare)
+__global__ void empty_graph_kernel(int32_t* row_ptr, int32_t* total_copy, unsigned long long* ovf_needed) {
+  row_ptr[0] = 0;
+  *total_copy = 0;
+  *ovf_needed = 0;
 }
 
 // The stand-alone gather (pg_radius_fill): one warp per 32 consecutive rows.
@@ -590,8 +524,11 @@ int launch_count_pass(pg_handle* h, cudaStream_t s) {
   unsigned long long* cursor = (unsigned long long*)((char*)h->misc.p + PG_MISC_TMPCUR);
   int32_t* totals = (int32_t*)((char*)h->misc.p + PG_MISC_TOTALS);
   unsigned long long* needed = (unsigned long long*)(totals + 4);
+  rows_out o;
+  int rc = pg_degree_prepare(h, a.stats, a.hist, a.hist_len, nq, s, &o.deg);
+  if (rc) return rc;
   if (gr.n == 0 || nq == 0) {
-    PG_LAUNCH(h, s, "empty_graph_kernel", empty_graph_kernel<<<1, 256, 0, s>>>(a.row_ptr, totals, a.stats, a.hist, a.hist ? a.hist_len : 0, needed));
+    PG_LAUNCH(h, s, "empty_graph_kernel", empty_graph_kernel<<<1, 1, 0, s>>>(a.row_ptr, totals, needed));
     PG_LAUNCH_CHECK(h);
     return PG_OK;
   }
@@ -621,21 +558,14 @@ int launch_count_pass(pg_handle* h, cudaStream_t s) {
 #undef PG_WALK_LAUNCH
   PG_LAUNCH_CHECK(h);
 
-  rows_out o;
   o.row_ptr = a.row_ptr; o.degree = a.degree; o.nbr_count = wide ? nullptr : a.nbr_count;
   o.row_off = (int32_t*)h->row_off.p;
   o.n_types = a.nbr_count ? a.n_types : 1;
-  o.stats = a.stats; o.hist = a.hist; o.hist_len = a.hist_len;
-  o.hist_mode = a.hist ? (a.hist_len <= PG_ACC_HIST_MAX ? 1 : 2) : 0;
-  if (o.hist_mode == 2) PG_CUDA(h, cudaMemsetAsync(a.hist, 0, (size_t)a.hist_len * sizeof(int32_t), s));
-  o.acc = (pg_stats_acc*)((char*)h->misc.p + PG_MISC_ACC);
-  o.acc_hist = (int32_t*)((char*)h->misc.p + PG_MISC_ACC_HIST);
   o.total_copy = totals;
   o.ovf_cursor = cursor; o.ovf_needed = needed;
   const int tiles = pg_div_up(nq, ROWS_TILE);
   pg_scan_state st;
-  int rc = pg_scan_prepare(h, tiles, TPB_ROWS, s, &st);
-  if (rc) return rc;
+  if ((rc = pg_scan_prepare(h, tiles, TPB_ROWS, s, &st))) return rc;
   rows_gather gx{};
   if (a.fused) {
     gx.tmp = (const pg_tmp_ent*)h->tmp_ent.p;

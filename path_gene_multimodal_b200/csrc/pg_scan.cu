@@ -17,16 +17,13 @@ constexpr int SCAN_TILE = SCAN_THREADS * SCAN_ITEMS;
 
 // CLEAR: the input is zeroed as it is read (the cell histogram is handed back clean for the next build,
 // which saves a memset node per build).
-// pub.acc != NULL: the first CTA also publishes the degree statistics accumulated by the kernel before
-// this one on the stream and resets the accumulators.
 template <bool CLEAR>
 __global__ void __launch_bounds__(SCAN_THREADS)
-scan_kernel(int32_t* in, int32_t* out, int32_t n, pg_scan_state st, int32_t* total_copy, pg_scan_publish pub) {
+scan_kernel(int32_t* in, int32_t* out, int32_t n, pg_scan_state st, int32_t* total_copy) {
   using TS = pg_tile_scan<SCAN_THREADS>;
   __shared__ typename TS::smem_t sm;
   pg_pdl_launch();
   pg_pdl_wait();
-  if (pub.acc && blockIdx.x == 0) pg_publish_stats(pub, SCAN_THREADS);
   const int tile = TS::take_tile(sm, st);
   const int64_t base = (int64_t)tile * SCAN_TILE + (int64_t)threadIdx.x * SCAN_ITEMS;
 
@@ -110,9 +107,7 @@ int pg_scan_prepare(pg_handle* h, int num_tiles, int group, cudaStream_t s, pg_s
 }
 
 int pg_scan_i32(pg_handle* h, const int32_t* in, int32_t* out, int32_t n, cudaStream_t s, int32_t* total_copy,
-                bool clear_in, const pg_scan_publish* publish) {
-  pg_scan_publish pub{};
-  if (publish) pub = *publish;
+                bool clear_in) {
   if (n < 0) return pg_set_error(h, PG_ERR_INVALID, "scan: n < 0");
   if (n == 0) {
     PG_LAUNCH(h, s, "scan_empty_kernel", scan_empty_kernel<<<1, 1, 0, s>>>(out, total_copy));
@@ -126,9 +121,9 @@ int pg_scan_i32(pg_handle* h, const int32_t* in, int32_t* out, int32_t n, cudaSt
   int rc = pg_scan_prepare(h, num_tiles, SCAN_THREADS, s, &st);
   if (rc) return rc;
   if (clear_in)
-    PG_LAUNCH(h, s, "scan_kernel", pg_launch_pdl(1, scan_kernel<true>, num_tiles, SCAN_THREADS, s, const_cast<int32_t*>(in), out, n, st, total_copy, pub));
+    PG_LAUNCH(h, s, "scan_kernel", pg_launch_pdl(1, scan_kernel<true>, num_tiles, SCAN_THREADS, s, const_cast<int32_t*>(in), out, n, st, total_copy));
   else
-    PG_LAUNCH(h, s, "scan_kernel", pg_launch_pdl(1, scan_kernel<false>, num_tiles, SCAN_THREADS, s, const_cast<int32_t*>(in), out, n, st, total_copy, pub));
+    PG_LAUNCH(h, s, "scan_kernel", pg_launch_pdl(1, scan_kernel<false>, num_tiles, SCAN_THREADS, s, const_cast<int32_t*>(in), out, n, st, total_copy));
   PG_LAUNCH_CHECK(h);
   return PG_OK;
 }

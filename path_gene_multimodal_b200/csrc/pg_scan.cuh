@@ -114,21 +114,4 @@ struct pg_tile_scan {
     return prefix;
   }
 };
-
-// first CTA of a scan that follows the radius count pass: hand the degree statistics to the caller and put
-// the accumulators back into their reset state (see pg_radius.cu)
-__device__ __forceinline__ void pg_publish_stats(const pg_scan_publish& pub, int threads) {
-  if (pub.hist)
-    for (int i = threadIdx.x; i < pub.hist_len; i += threads) { pub.hist[i] = pub.acc_hist[i]; pub.acc_hist[i] = 0; }
-  if (threadIdx.x == 0) {
-    pg_stats_acc a = *pub.acc;
-    if (pub.stats) {
-      pub.stats->min_degree = a.n_nodes ? a.min_degree : 0; pub.stats->max_degree = a.n_nodes ? a.max_degree : 0;
-      pub.stats->sum_degree = (long long)a.sum_degree; pub.stats->sumsq_degree = (long long)a.sumsq_degree;
-      pub.stats->n_nodes = (long long)a.n_nodes;
-    }
-    a.min_degree = 0x7fffffff; a.max_degree = -1; a.sum_degree = 0; a.sumsq_degree = 0; a.n_nodes = 0; a.done = 0;
-    *pub.acc = a;
-  }
-}
 #endif

@@ -9,8 +9,8 @@ passes the defaults (5 nucleus types, k <= 16, 64 histogram bins). Covered here:
   memory); the select pass hands a point to the ring pass when its 3x3 block holds 65536 candidates or more (its
   histogram counters are 16-bit).
 * K7 union: mark / push / rank kernels specialised for 16-byte aligned lists (k = 4, 8, 16), generic otherwise.
-* K8: compose_kernel<8> / <16>; degree histograms in shared bins up to 1024 (radius rows, union rank) or 2048
-  (compose_degree) bins, global atomics above; the accumulators the last CTA publishes are re-armed for the next call.
+* K8: compose_kernel<8> / <16>; degree histograms in shared bins up to 2048 bins (radius rows, union rank and
+  compose_degree alike), global atomics above; the accumulators the last CTA publishes are re-armed for the next call.
 * K11 clustering on adversarial CSRs (cliques, a 20 000-leaf hub, rows straddling the 32-row warp ranges).
 * K10 node features on both sides of the tile kernel's 40-column limit, up to PG_FEAT_MAX_COLS feature columns.
 
@@ -691,8 +691,8 @@ def test_union_on_misaligned_lists(engine, k, dt):
 @pytest.mark.gpu
 @pytest.mark.parametrize("hist_len", HIST_LENS)
 def test_degree_histogram_lengths(engine, clump, hist_len):
-    # shared bins up to 1024 (radius rows, union rank) / 2048 (compose_degree), global atomics above; each call twice on
-    # one handle, since the accumulators the last CTA publishes must be re-armed for the next call
+    # shared bins up to 2048 for every producer, global atomics above; each call twice on one handle, since the
+    # accumulators the last CTA publishes must be re-armed for the next call
     xy, types, r, ref = clump["xy"], clump["types"], clump["r"], clump["ref"]
     deg = clump["deg"]
     assert deg.max() > max(HIST_LENS)

@@ -511,6 +511,25 @@ def test_knn_union_small_and_empty(engine):
     assert e0["row_ptr"].tolist() == [0] and e0["edges"].shape == (0, 2) and e0["hist"].tolist() == [0, 0, 0, 0]
 
 
+def test_degree_statistics_of_the_empty_graph(engine, monkeypatch):
+    # n = 0 through compose_degree, degree_stats and the kNN union: the statistics block (min, max, sum, sumsq, n) and
+    # the histogram are all zero, with shared bins and past them. Outputs start at -1, so one left unwritten shows.
+    from path_gene_multimodal_b200 import degree_stats
+
+    monkeypatch.setattr(engine, "_empty", lambda shape, dtype: torch.full(shape, -1, dtype=dtype, device=engine.device))
+    none = torch.empty(0, dtype=torch.int32, device="cuda")
+    for hist_len in (4, 2049):
+        cd = engine.compose_degree(torch.zeros(1, dtype=torch.int32, device="cuda"), none, none, 5, hist_len=hist_len)
+        un = engine.knn_union(torch.empty((0, 3), dtype=torch.int32, device="cuda"),
+                              torch.empty((0, 3), dtype=torch.float64, device="cuda"), types=none, hist_len=hist_len)
+        for name, res in (("compose", cd), ("union", un)):
+            assert res["stats"].tolist() == [0, 0, 0, 0], (name, hist_len)
+            assert res["hist"].tolist() == [0] * hist_len, (name, hist_len)
+        st = degree_stats(np.zeros(1, dtype=np.int64), hist_len=hist_len, device=0)
+        assert (st["min"], st["max"], st["sum"], st["sumsq"], st["n"]) == (0, 0, 0, 0, 0), hist_len
+        assert st["hist"].tolist() == [0] * hist_len and st["degree"].shape == (0,), hist_len
+
+
 # ---------------------------------------------------------------- seeded fuzz against the brute-force oracles
 def _fuzz_points(rng, n, kind):
     if kind == "uniform":
